@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the matrix-factorization hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2|c1|c4|c4mini]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2|c1|c4|c4mini] [--dump-outputs DIR]
 
 Primary line (one JSON object on stdout, rank 0):
   metric  = training interactions/s, WMRB rank-64 on the ML-20M-shaped synthetic workload (BASELINE.json
@@ -122,18 +122,29 @@ def peaks():
 
 
 def gen_interactions(n_u, n_i, nnz, seed, dev):
-    """Zipf(1.0)-weighted users and items, deduplicated, row-major sorted (SURVEY 8d)."""
+    """Zipf(1.0)-weighted users and items, deduplicated, row-major sorted (SURVEY 8d).  Ids are seeded uniforms looked up in
+    a cumulative distribution summed on the host in fp64, so a seed gives the same table on every run (torch.multinomial
+    sums its distribution on the device, where the last bits are not reproducible and draws near a bin edge move).  Figures
+    stored before this generator (profiles/, BASELINE) were measured on other draws of the same law and sizes."""
     g = torch.Generator(device=dev)
     g.manual_seed(seed)
-    wu = (1.0 / torch.arange(1, n_u + 1, device=dev, dtype=torch.float64)).float()
-    wi = (1.0 / torch.arange(1, n_i + 1, device=dev, dtype=torch.float64)).float()
+
+    def zipf_cdf(n):
+        c = np.cumsum(1.0 / np.arange(1, n + 1, dtype=np.float64))
+        return torch.as_tensor(c / c[-1], device=dev)
+
+    cu, ci = zipf_cdf(n_u), zipf_cdf(n_i)
+
+    def draw(cdf, m):
+        return torch.searchsorted(cdf, torch.rand(m, generator=g, device=dev, dtype=torch.float64), right=True)
+
     keys = torch.empty(0, dtype=torch.int64, device=dev)
     for _ in range(40):
         if keys.numel() >= nnz:
             break
         m = int((nnz - keys.numel()) * 1.5) + 4096
-        u = torch.multinomial(wu, m, replacement=True, generator=g)
-        i = torch.multinomial(wi, m, replacement=True, generator=g)
+        u = draw(cu, m)
+        i = draw(ci, m)
         keys = torch.unique(torch.cat([keys, u * n_i + i]))
         del u, i
     if keys.numel() > nnz:
@@ -326,9 +337,35 @@ KERNEL_OF = {"user_pass": "user_pass_kernel", "item_pass": "spmm_seg_kernel (ite
              "embed_bwd": "spmm_seg_kernel (X^T.dE)", "adam": "adam1_kernel"}
 
 
-def train_bench(wl, comm, steps, warmup, local, world, hbm_peak, parity_kw=None):
+DUMP_BYTES = 64 << 20  # all arrays of --dump-outputs together
+
+
+def dump_outputs(wl, plan, out_dir, seed=0):
+    """Writes what fit() hands its caller after the last step run on `plan` as <out_dir>/<name>.npy: the embeddings
+    recomputed from the final weights, the trainables, the per-interaction losses of that step (the reference's loss_fn)
+    and their mean.  An array over its share of DUMP_BYTES is cut to a sample of its rows drawn from `seed`, so the same
+    workload dumps the same entries on every run and two builds can be compared output for output."""
+    r = wl.model.n_components
+    arrays = {"user_embedding": plan.u.forward()[:, :r], "item_embedding": plan.i.forward()[:, :r]}
+    for side, tower in (("user", plan.u), ("item", plan.i)):
+        for j, t in enumerate(wl.model._trainable_list(tower)):
+            arrays[f"{side}_trainable_{j}"] = t
+    arrays["loss"] = plan.ip.loss_vector().reshape(-1)  # KL's loss is a scalar
+    cap = DUMP_BYTES // (len(arrays) + 1)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        row_bytes = t[:1].numel() * 4
+        if t.shape[0] * row_bytes > cap:
+            rows = np.sort(np.random.default_rng(seed).choice(t.shape[0], cap // row_bytes, replace=False))
+            t = t[torch.as_tensor(rows, device=t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "mean_loss.npy"), np.array([plan.ip.mean_loss()], np.float64))
+
+
+def train_bench(wl, comm, steps, warmup, local, world, hbm_peak, parity_kw=None, dump_dir=None):
     """Device-resident timing of `steps` epochs of `wl` (inputs and structures already in HBM): returns the plan and a dict.
-    `parity_kw`: run the strict sampled oracle check at the initial weights first (result under "parity_init")."""
+    `parity_kw`: run the strict sampled oracle check at the initial weights first (result under "parity_init").
+    `dump_dir`: write the outputs of the last timed step there (dump_outputs)."""
     from teamoflow_b200 import _abi
     dev = torch.device("cuda", local)
     xu, xi = wl.feature_args()
@@ -364,6 +401,8 @@ def train_bench(wl, comm, steps, warmup, local, world, hbm_peak, parity_kw=None)
         torch.distributed.all_reduce(ms_total, op=torch.distributed.ReduceOp.MAX)
     ms_step = float(ms_total) / steps
     loss_now = plan.ip.mean_loss() if comm is None else comm.mean_loss(plan.ip)
+    if dump_dir is not None:  # before profile_phases, which trains the plan further
+        dump_outputs(wl, plan, dump_dir)
     phases = profile_phases(plan, wl.lr)
     phase_bytes = {"user_pass": wl.bytes["user_pass"], "item_pass": wl.bytes["item_pass"],
                    "embed_fwd": wl.bytes["features"] / 2, "embed_bwd": wl.bytes["features"] / 2, "adam": wl.bytes["adam"]}
@@ -985,7 +1024,11 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--topk-user-sharded", action="store_true", help="also time the user-sharded alternative of the top-k (N > 1)")
     ap.add_argument("--topk-only", action="store_true", help="run only the secondary top-k bench (profiling aid)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed training step (rank 0's shard) "
+                    "as DIR/<name>.npy, at most 64 MB in all")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.topk_only):
+        ap.error("--dump-outputs needs the timed training path (--impl ours, no --topk-only)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -1043,7 +1086,8 @@ def main():
 
     # ---- device-resident measurement: inputs and structures already in HBM
     model = wl.model
-    plan, tb = train_bench(wl, comm, args.steps, args.warmup, local, world, hbm_peak, parity_kw=None if args.no_parity else {})
+    plan, tb = train_bench(wl, comm, args.steps, args.warmup, local, world, hbm_peak, parity_kw=None if args.no_parity else {},
+                           dump_dir=args.dump_outputs if rank == 0 else None)
     ms_step = tb["ms_step"]
     total_nnz = wl.total_nnz if strong else world * wl.nnz
     value = total_nnz / (ms_step * 1e-3)

@@ -1,10 +1,10 @@
-"""Golden vectors produced by the REFERENCE'S OWN SOURCE (``/root/reference/src/teamoflow/mf``, imported unmodified)
-executed over the TensorFlow stand-in in ``tests/golden/tf_shim`` (TensorFlow itself cannot be installed here).
+"""Golden vectors produced by the REFERENCE'S OWN SOURCE (``$TMF_REFERENCE_ROOT/src/teamoflow/mf``, imported unmodified)
+executed over the TensorFlow stand-in in ``tests/golden/tf_shim`` (no TensorFlow needed).
 
-    python tests/golden/make_ref_golden.py            # writes tests/golden/ref_golden.json
+    TMF_REFERENCE_ROOT=<checkout of the original TeAMOFlow> python tests/golden/make_ref_golden.py   # writes tests/golden/ref_golden.json
 
-Only runs in the build container (needs /root/reference); the JSON travels with the repo.  See tf_shim/README.md for
-what these vectors pin (the reference's Python logic) and what they do not (TensorFlow's kernels).
+Needs a checkout of the original project, which is not part of this repository; the JSON travels with the repo.  See
+tf_shim/README.md for what these vectors pin (the reference's Python logic) and what they do not (TensorFlow's kernels).
 """
 import contextlib
 import io
@@ -15,10 +15,13 @@ import sys
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("TMF_REFERENCE_ROOT", "/root/reference")
+REF = os.environ.get("TMF_REFERENCE_ROOT", "")
 
 
 def load_reference():
+    if not os.path.isdir(os.path.join(REF, "src", "teamoflow", "mf")):
+        sys.exit("make_ref_golden.py: set TMF_REFERENCE_ROOT to a checkout of the original TeAMOFlow project "
+                 f"(no src/teamoflow/mf under {REF!r})")
     sys.path.insert(0, os.path.join(HERE, "tf_shim"))
     sys.path.insert(0, REF)
     import tensorflow as tf  # the shim

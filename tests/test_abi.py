@@ -2,7 +2,9 @@
 include/tmf.h declares; the Python surface mirrors the reference's classes and signatures."""
 import ast
 import ctypes
+import importlib
 import inspect
+import json
 import os
 import re
 
@@ -10,7 +12,12 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HEADER = os.path.join(ROOT, "include", "tmf.h")
-REF = "/root/reference/src/teamoflow/mf"
+# a checkout of the original TeAMOFlow project (not part of this repository): the surface checks against its source run
+# only where one is given
+REF_ROOT = os.environ.get("TMF_REFERENCE_ROOT")
+REF = os.path.join(REF_ROOT, "src", "teamoflow", "mf") if REF_ROOT else None
+SURFACE = os.path.join(ROOT, "tests", "golden", "plugin_surface.json")
+MODULES = ["matrix_factorization", "loss_graphs", "embedding_graphs", "initializer_graphs", "input_utils", "predict_graphs", "utils"]
 
 
 def _header_symbols():
@@ -60,11 +67,24 @@ def _ref_signatures(path):
     return classes, funcs
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
-@pytest.mark.parametrize("module", ["matrix_factorization", "loss_graphs", "embedding_graphs", "initializer_graphs", "input_utils",
-                                    "predict_graphs", "utils"])
+def _surface(module):
+    """``_ref_signatures`` of teamoflow_b200/mf/<module>.py in JSON form: every class, method and function the file
+    defines (private ones included), each with its parameter names and number of defaults."""
+    classes, funcs = _ref_signatures(os.path.join(ROOT, "teamoflow_b200", "mf", f"{module}.py"))
+    return json.loads(json.dumps({"classes": classes, "functions": funcs}))
+
+
+@pytest.mark.parametrize("module", MODULES)
+def test_plugin_surface_is_the_recorded_one(module):
+    """This package's own surface, extracted exactly as test_plugin_surface_matches_reference extracts the reference's,
+    against tests/golden/plugin_surface.json.  It pins the package against unintended change, not against the reference;
+    a deliberate change of the surface rewrites the file (``python tests/test_abi.py``), which then shows in the diff."""
+    assert _surface(module) == json.load(open(SURFACE))[module]
+
+
+@pytest.mark.skipif(not (REF and os.path.isdir(REF)), reason="needs TMF_REFERENCE_ROOT: a checkout of the original TeAMOFlow source")
+@pytest.mark.parametrize("module", MODULES)
 def test_plugin_surface_matches_reference(module):
-    import importlib
     ours = importlib.import_module(f"teamoflow_b200.mf.{module}")
     classes, funcs = _ref_signatures(os.path.join(REF, f"{module}.py"))
     for cname, methods in classes.items():
@@ -79,7 +99,6 @@ def test_plugin_surface_matches_reference(module):
         assert names[:len(args)] == args, f"{module}.{fname}: {names} vs reference {args}"
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
 def test_constructor_defaults_match_reference():
     from teamoflow_b200.mf.matrix_factorization import MatrixFactorization
     from teamoflow_b200.mf import embedding_graphs as e, loss_graphs as l, initializer_graphs as i
@@ -92,3 +111,10 @@ def test_constructor_defaults_match_reference():
     sig = inspect.signature(MatrixFactorization.fit)
     assert sig.parameters["lr"].default == 1e-2
     assert inspect.signature(MatrixFactorization.recall_at_k).parameters["k"].default == 10
+
+
+if __name__ == "__main__":
+    with open(SURFACE, "w") as f:
+        json.dump({m: _surface(m) for m in MODULES}, f, indent=1, sort_keys=True)
+        f.write("\n")
+    print("wrote", SURFACE)

@@ -116,8 +116,8 @@ def _sync_grads_and_kl(rank, world):
     it.dE = torch.full((6, 4), float(rank + 1))
     g = {"W": torch.full((7, 4), float(rank + 1)), "b": torch.full((1, 4), float(10 * (rank + 1)))}
     u = _FakeTower("biased", g, {"W": torch.zeros(7, 4), "b": torch.zeros(1, 4)})
-    comm = tdist.GradientSync(shared_user_rows=5)
-    assert comm.peer is False  # no CUDA here: the collective path
+    comm = tdist.GradientSync(shared_user_rows=5, peer=False)  # CPU tensors: the collective path, also where CUDA is present
+    assert comm.peer is False
     fused = comm.sync_grads(_FakePlan(u, it), lr=0.1)
     assert fused is False
     assert torch.all(it.dE == 3.0)

@@ -141,7 +141,11 @@ def test_initializer_properties():
     assert abs(np.sqrt((W.astype(np.float64) ** 2).sum()) - 1) < 1e-6 and W.min() >= 0
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src/teamoflow/mf"), reason="the reference tree only exists in the build container")
+REF_ROOT = os.environ.get("TMF_REFERENCE_ROOT")
+
+
+@pytest.mark.skipif(not (REF_ROOT and os.path.isdir(os.path.join(REF_ROOT, "src", "teamoflow", "mf"))),
+                    reason="needs TMF_REFERENCE_ROOT: a checkout of the original TeAMOFlow source")
 def test_committed_goldens_are_what_the_reference_source_produces():
     """Re-run the generator (reference source over the shim) and compare with the committed JSON."""
     code = ("import sys, json; sys.path.insert(0, %r); import make_ref_golden as m; print(json.dumps(m.build()))"
