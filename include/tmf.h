@@ -188,8 +188,9 @@ TMF_API int tmf_pack_bf16(const float* src, int64_t n, int32_t n_comp, int32_t l
  * are exact.  Scores are never written to HBM.
  *   clamp != 0: scores <= 0 are +0.0 before ranking (recall_at_k path, :237).
  *   item_offset: global index of this GPU's first item (item-sharded scoring).
+ *   1 <= k <= min(1024, n_items); k > 128 runs a configuration with longer candidate lists (more workspace).
  *   out_idx[n_users, k] int32 (global ids), out_score[n_users, k] fp32 canonical scores.
- * Workspace from tmf_score_topk_ws_bytes. */
+ * Workspace from tmf_score_topk_ws_bytes (same n_users, n_items, n_comp and k as the call). */
 TMF_API size_t tmf_score_topk_ws_bytes(int64_t n_users, int64_t n_items, int32_t n_comp, int32_t k);
 TMF_API int tmf_score_topk(const float* U, int64_t n_users, const float* V, int64_t n_items, int32_t n_comp, int32_t ld,
                    int32_t k, int32_t clamp, int32_t item_offset, int32_t* out_idx, float* out_score, void* ws,
@@ -206,7 +207,7 @@ TMF_API int tmf_score_dense_bf16(const float* U, int64_t n_users, const float* V
  * against any subset of the items, exchanged between GPUs).  A slab then only lists candidates that can still be in
  * the global top-k, skips the per-row warm-up, and rows with fewer than k such candidates are padded with
  * (score -inf, id INT32_MAX) entries, which lose every comparison in tmf_topk_merge*.  The merged result is
- * identical to tmf_score_topk over the concatenated slabs. */
+ * identical to tmf_score_topk over the concatenated slabs.  k and the workspace as for tmf_score_topk. */
 TMF_API int tmf_score_topk_bounded(const float* U, int64_t n_users, const float* V, int64_t n_items, int32_t n_comp, int32_t ld,
                            int32_t k, int32_t clamp, int32_t item_offset, const float* row_bound, int32_t* out_idx,
                            float* out_score, void* ws, size_t ws_bytes, tmf_stream_t stream);

@@ -49,6 +49,15 @@ constexpr int NBINS = 48;      // per-row score histogram bins (16-bit counts, t
 constexpr int QCAP = 16;       // per-row survivor queue slots in shared memory (drained warp-wide)
 constexpr int HSTRIDE = NBINS / 2 + 1;  // words per row, padded against bank conflicts
 constexpr int UB_BATCH = 2048; // user blocks (x128 rows) per main-kernel launch: bounds the candidate workspace to 4 GB
+// Wide configuration, 128 < k <= 1024 (DESIGN "top-k", wide k): the same kernel with longer lists.  8192 slots leave ~5k
+// appends between saturation rebuilds even in clamp mode, where the k lowest ids stay listed besides >= k entries above the
+// threshold; 592 user blocks = exactly two waves of the 2 x 148 persistent CTAs and a 4.96 GB candidate workspace.  The
+// first rebuild streams the list through warp_rebuild_row once it holds k + 2 tiles of entries (warp_rebuild_first keeps
+// only INIT_N entries in registers).
+constexpr int NARROW_MAX_K = 128;
+constexpr int WIDE_MAX_K = 1024;
+constexpr int CAP_W = 8192;
+constexpr int UB_BATCH_W = 592;
 constexpr int TOPK_THREADS = 256;
 constexpr int A_SUB_BYTES = BM * BK * 2;   // 16 KB
 constexpr int B_STAGE_BYTES = BN * BK * 2; // 16 KB
@@ -87,7 +96,7 @@ struct TopkParams {
   int n_tiles, kb;              // item tiles of BN, k-blocks of BK
   int k, clamp, item_offset;
   const float* erow;            // [n_users_pad] error bound E of each user row against this item slab (global row index)
-  float2* cand;                 // [batch rows][CAP] (approx score, item id bits), batch-local row index
+  float2* cand;                 // [batch rows][CAP or CAP_W] (approx score, item id bits), batch-local row index
   int* cnt;                     // [batch rows] candidates per row, -1 = overflow (exact path)
   float* thr_out;               // [batch rows] final keep-threshold of the row
   int* ovf_count;               // [1]
@@ -144,6 +153,7 @@ __device__ __forceinline__ float edge_threshold(float lo, float w, int bthr, flo
 // for, threshold fixed for the duration -- so they pipeline; the threshold advances once at the end.
 struct DrainRet { float thr; int cnt, bthr, A; };
 // (out of line, state by value in registers: inlining it at every call site costs registers in the tile loop)
+template <int CAP>
 __device__ __noinline__ DrainRet drain_queues_nl(float thr, float thr_ext, float lo, float w, float inv_w, float E, int cnt, int cq, int bthr, int A,
                                                  uint32_t queue, float2* buf, uint32_t hrow, int k, int clamp) {
   int maxq = cq;
@@ -183,14 +193,16 @@ __device__ __noinline__ DrainRet drain_queues_nl(float thr, float thr_ext, float
   r.thr = thr; r.cnt = cnt; r.bthr = bthr; r.A = A;
   return r;
 }
+template <int CAP>
 __device__ __forceinline__ void drain_queues(RowState& st, uint32_t queue, float2* buf, uint32_t hrow, int k, int clamp) {
-  const DrainRet r = drain_queues_nl(st.thr, st.thr_ext, st.lo, st.w, st.inv_w, st.E, st.cnt, st.cq, st.bthr, st.A, queue, buf, hrow, k, clamp);
+  const DrainRet r = drain_queues_nl<CAP>(st.thr, st.thr_ext, st.lo, st.w, st.inv_w, st.E, st.cnt, st.cq, st.bthr, st.A, queue, buf, hrow, k, clamp);
   st.thr = r.thr; st.cnt = r.cnt; st.bthr = r.bthr; st.A = r.A;
   st.cq = 0;
 }
 
-// One 32-column slice of a row's accumulator BEFORE the row's threshold exists (first 3 tiles): every column is
-// appended directly.  (Clamp-mode "filler" items -- the k <= 128 lowest ids -- therefore need no special case.)
+// One 32-column slice of a row's accumulator BEFORE the row's threshold exists (first 3 tiles; wide k: until the row
+// holds k + 2 tiles of entries): every column is appended directly.  (Clamp-mode "filler" items -- the k lowest ids --
+// therefore need no special case.)
 template <bool DUMP>
 __device__ __forceinline__ void epilogue_chunk(uint32_t (&r)[32], int col0, int n_items, bool tail_tile, bool valid, bool warp_inited,
                                                RowState& st, uint32_t queue, float2* buf, uint32_t hrow, long long row,
@@ -238,6 +250,7 @@ __device__ __forceinline__ void group_max4(const uint32_t (&r)[32], float* m8) {
 // registers through an unrolled chain of warp-uniform blocks (51.0 ms: 16 extra branches per tile) or an indexed jump (register
 // arrays spill); issuing the next group's TMEM load under the current group's pushes (48.4 ms); slot indices from a survivor
 // mask + popc instead of the running count (47.4 ms).  The epilogue pays per instruction, not per round trip.
+template <int CAP>
 __device__ __forceinline__ void epilogue_half(uint32_t t_base, int col0, RowState& st, uint32_t queue, float2* buf, uint32_t hrow,
                                               const TopkParams& p) {
   uint32_t ra[32], rb[32];
@@ -263,7 +276,7 @@ __device__ __forceinline__ void epilogue_half(uint32_t t_base, int col0, RowStat
     gmask &= gmask - 1;
     uint32_t v[8];
     tmem_ld8(t_base + (uint32_t)(8 * g), v);
-    if (__any_sync(0xffffffffu, st.cq > QCAP - 8)) drain_queues(st, queue, buf, hrow, p.k, p.clamp);
+    if (__any_sync(0xffffffffu, st.cq > QCAP - 8)) drain_queues<CAP>(st, queue, buf, hrow, p.k, p.clamp);
     tmem_ld_wait_for8(v);
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
@@ -274,11 +287,12 @@ __device__ __forceinline__ void epilogue_half(uint32_t t_base, int col0, RowStat
     }
   }
 }
+template <int CAP>
 __device__ __forceinline__ void epilogue_tile(uint32_t t_base, int col0, RowState& st, uint32_t queue, float2* buf, uint32_t hrow,
                                               const TopkParams& p) {
 #pragma unroll 1
   for (int h = 0; h < 2; ++h)  // one copy of the code: the unrolled pass 2 is ~4 KB of sparsely executed instructions
-    epilogue_half(t_base + (uint32_t)(64 * h), col0 + 64 * h, st, queue, buf, hrow, p);
+    epilogue_half<CAP>(t_base + (uint32_t)(64 * h), col0 + 64 * h, st, queue, buf, hrow, p);
 }
 
 // exact k-th largest approximate score of a row's list (n entries in global memory, streamed through L2) by an
@@ -599,9 +613,11 @@ __device__ __noinline__ void warp_rebuild_saturated(float2* buf, int n, int k, i
 }
 
 // ------------------------------------------------------------------ the fused kernel
-template <bool DUMP, bool PROF>
+// WIDE: the configuration for 128 < k <= 1024 (CAP_W list slots, first rebuild by warp_rebuild_row)
+template <bool DUMP, bool PROF, bool WIDE>
 __global__ void __launch_bounds__(TOPK_THREADS, 2)
 score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_constant__ CUtensorMap tmapV, const TopkParams p) {
+  constexpr int cap = WIDE ? CAP_W : CAP;
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   // carve (1024-byte aligned operand tiles first)
   unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -749,7 +765,7 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
           st.lo = INFINITY;
         }
       }
-      float2* buf = p.cand + lrow * CAP;
+      float2* buf = p.cand + lrow * cap;
       long long w_tfull = 0, w_work = 0, w_init = 0;
       for (int nt = 0; nt < p.n_tiles; ++nt) {
         long long t0 = now();
@@ -761,7 +777,7 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
         const uint32_t t_base = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * BN);
         const bool tail_tile = (nt + 1) * BN > n_items;
         if (!DUMP && warp_inited && TMF_DBG(p) < 2) {
-          epilogue_tile(t_base, nt * BN, st, queue, buf, hrow, p);
+          epilogue_tile<cap>(t_base, nt * BN, st, queue, buf, hrow, p);
         } else if (TMF_DBG(p) < 3) {
           uint32_t ra[32], rb[32];
           tmem_ld32(t_base, ra);
@@ -786,18 +802,19 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
         if (!DUMP) {
           if (__any_sync(0xffffffffu, st.cq >= QCAP / 2)) {
             const long long td = now();
-            drain_queues(st, queue, buf, hrow, p.k, p.clamp);
+            drain_queues<cap>(st, queue, buf, hrow, p.k, p.clamp);
             if (PROF && lane == 0) { atomicAdd(p.prof + 10, (unsigned long long)(now() - td)); atomicAdd(p.prof + 11, 1ull); }
           }
-          // (re)build: the first time once a row holds INIT_N - BN entries (all valid rows of a warp get there at
-          // the same tile because everything is appended until then), later whenever a list is about to saturate
-          const bool first = !warp_inited && __any_sync(0xffffffffu, valid && st.cnt >= INIT_N - BN);
-          unsigned need = __ballot_sync(0xffffffffu, valid && st.cnt <= CAP && (first || (warp_inited && st.cnt > CAP - 4 * QCAP)));
+          // (re)build: the first time once a row holds INIT_N - BN entries (wide: k + 2 tiles; all valid rows of a warp
+          // get there at the same tile because everything is appended until then), later whenever a list is about to saturate
+          const int first_n = WIDE ? p.k + 2 * BN : INIT_N - BN;
+          const bool first = !warp_inited && __any_sync(0xffffffffu, valid && st.cnt >= first_n);
+          unsigned need = __ballot_sync(0xffffffffu, valid && st.cnt <= cap && (first || (warp_inited && st.cnt > cap - 4 * QCAP)));
           if (need) {  // the radix scratch aliases the queues: empty them first (lengths may grow a little)
             const long long tq = now();
-            drain_queues(st, queue, buf, hrow, p.k, p.clamp);
+            drain_queues<cap>(st, queue, buf, hrow, p.k, p.clamp);
             if (PROF && lane == 0) { atomicAdd(p.prof + 19, (unsigned long long)(now() - tq)); atomicAdd(p.prof + 18, 1ull); }
-            need = __ballot_sync(0xffffffffu, valid && st.cnt <= CAP && (first || (warp_inited && st.cnt > CAP - 4 * QCAP)));
+            need = __ballot_sync(0xffffffffu, valid && st.cnt <= cap && (first || (warp_inited && st.cnt > cap - 4 * QCAP)));
           }
           while (need) {
             const int owner = __ffs(need) - 1;
@@ -805,12 +822,12 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
             const int n_o = __shfl_sync(0xffffffffu, st.cnt, owner);
             const float E_o = __shfl_sync(0xffffffffu, st.E, owner);
             __syncwarp();
-            float2* obuf = p.cand + ((long long)ub * BM + q * 32 + owner) * CAP;
+            float2* obuf = p.cand + ((long long)ub * BM + q * 32 + owner) * cap;
             uint32_t* ohist = hist_rows + (q * 32 + owner) * HSTRIDE;
             const float lo_o = __shfl_sync(0xffffffffu, st.lo, owner);
             const long long tr = now();
             int which = 0;
-            if (first && n_o <= INIT_N) {
+            if (!WIDE && first && n_o <= INIT_N) {
               warp_rebuild_first(obuf, n_o, p.k, p.clamp, p.item_offset, E_o, ohist, radix, iout);
             } else if (lo_o < INFINITY && !first) {  // live histogram: compaction + re-centring in one pass
               which = 1;
@@ -828,8 +845,8 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
               st.bthr = __float_as_int(iout[3]); st.A = __float_as_int(iout[4]);
               st.cnt = __float_as_int(iout[5]);
               st.thr = fmaxf(edge_threshold(st.lo, st.w, st.bthr, st.E, p.clamp), st.thr_ext);
-              if (st.cnt > CAP - 8 * QCAP) {  // cannot shrink (massive ties): hand the row to the exact path
-                st.cnt = CAP + 1;
+              if (st.cnt > cap - 8 * QCAP) {  // cannot shrink (massive ties): hand the row to the exact path
+                st.cnt = cap + 1;
                 st.thr = INFINITY;
               }
             }
@@ -839,13 +856,13 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
         }
         w_init += now() - t2;
       }
-      if (!DUMP) drain_queues(st, queue, buf, hrow, p.k, p.clamp);
+      if (!DUMP) drain_queues<cap>(st, queue, buf, hrow, p.k, p.clamp);
       if (PROF && lane == 0) {
         atomicAdd(p.prof + 4, (unsigned long long)w_tfull); atomicAdd(p.prof + 5, (unsigned long long)w_work);
         atomicAdd(p.prof + 6, (unsigned long long)w_init); atomicAdd(p.prof + 7, 1ull);
       }
-      if (PROF) atomicAdd(p.prof + 20, (unsigned long long)(valid ? min(st.cnt, CAP) : 0));
-      const bool ovf = st.cnt > CAP;
+      if (PROF) atomicAdd(p.prof + 20, (unsigned long long)(valid ? min(st.cnt, cap) : 0));
+      const bool ovf = st.cnt > cap;
       if (valid && ovf) {
         const int slot = atomicAdd(p.ovf_count, 1);
         p.ovf_rows[slot] = (int)row;
@@ -867,6 +884,9 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
 constexpr int RR_WARPS = 8;
 constexpr int SEL_CAP = 512;   // survivors per row the rerank can rank; more -> exact path
 constexpr int RR_CHAINS = 4;   // independent fp64 FMA chains per lane
+// wide k: room for the ~k + near-ties survivors of k = 1024 (16 KB of keys per warp), 4 warps so two CTAs share an SM
+constexpr int RR_WARPS_W = 4;
+constexpr int SEL_CAP_W = 2048;
 
 struct RerankParams {
   long long n_users, n_items, row0;  // rows [row0, row0 + n_rows) are batch-local rows [0, n_rows)
@@ -885,7 +905,7 @@ struct RerankParams {
   float* out_score;
 };
 
-// k-th largest of m (<= SEL_CAP) scores held in shared memory pairs (score, id): 8-bit radix select, one warp
+// k-th largest of m (<= SEL_CAP / SEL_CAP_W) scores held in shared memory pairs (score, id): 8-bit radix select, one warp
 __device__ __forceinline__ float smem_select_kth(const float2* pr, int m, int k, int* radix) {
   const int lane = threadIdx.x & 31;
   uint32_t prefix = 0, mask = 0;
@@ -944,11 +964,20 @@ constexpr int STG_STRIDE = STG_COLS + 4;  // floats; 272-byte rows keep the per-
 //     copy per candidate and slice: 8 KB in flight per warp, where the per-lane strided loads of the first version
 //     exposed a full DRAM latency every 16 bytes), and every lane runs ONE candidate's fp64 FMA chain in
 //     component order -- bit-identical to oracle.canonical_scores;
-//  4. (score, id) are packed into one 64-bit key and ranked by counting (branch-free).
-__global__ void __launch_bounds__(RR_WARPS * 32) rerank_kernel(const RerankParams p) {
+//  4. (score, id) are packed into one 64-bit key and ranked by counting (branch-free, O(m^2)); the wide configuration
+//     (m up to SEL_CAP_W) orders the keys by a bitonic sort in shared memory instead (O(m log^2 m)).
+template <bool WIDE>
+__host__ __device__ __forceinline__ size_t rerank_warp_smem(int ld) {
+  return (size_t)ld * sizeof(double) + (WIDE ? SEL_CAP_W : SEL_CAP) * 8 + 32 * STG_STRIDE * 4 + 16;
+}
+template <bool WIDE>
+__global__ void __launch_bounds__((WIDE ? RR_WARPS_W : RR_WARPS) * 32) rerank_kernel(const RerankParams p) {
+  constexpr int RR_WARPS = WIDE ? RR_WARPS_W : tmf::RR_WARPS;
+  constexpr int SEL_CAP = WIDE ? SEL_CAP_W : tmf::SEL_CAP;
+  constexpr int CAP = WIDE ? CAP_W : tmf::CAP;
   extern __shared__ __align__(16) unsigned char rr_smem[];
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const size_t per_warp = (size_t)p.ld * sizeof(double) + SEL_CAP * 8 + 32 * STG_STRIDE * 4 + 16;
+  const size_t per_warp = rerank_warp_smem<WIDE>(p.ld);
   unsigned char* base = rr_smem + (size_t)w * per_warp;
   double* ud = reinterpret_cast<double*>(base);                       // [ld] this user's row, widened once
   float2* pr = reinterpret_cast<float2*>(ud + p.ld);                  // [SEL_CAP] (approx score, id), later 64-bit rank keys
@@ -997,13 +1026,17 @@ __global__ void __launch_bounds__(RR_WARPS * 32) rerank_kernel(const RerankParam
       float mx;
       kth = warp_select_kth(buf, n, k, radix, mx);
     }
-    thr = fmaxf(thr, keep_threshold(kth, p.erow[row], p.clamp));
+    const float E = p.erow[row];
+    thr = fmaxf(thr, keep_threshold(kth, E, p.clamp));
+    // Clamp mode, wide k: with kth - 2E > 0 at least k listed items score above zero, so no zero-score filler can be in the
+    // answer and the k lowest ids are kept only on their own merit (kept unconditionally they would double m past SEL_CAP_W).
+    const bool fill = p.clamp && !(WIDE && kth - 2.f * E > 0.f);
     if (m <= SEL_CAP) {
       int m2 = 0;
       for (int e0 = 0; e0 < m; e0 += 32) {
         const int e = e0 + lane;
         const float2 x = e < m ? pr[e] : make_float2(-INFINITY, 0.f);
-        const bool keep = e < m && (x.x >= thr || (p.clamp && __float_as_int(x.y) - p.item_offset < k));
+        const bool keep = e < m && (x.x >= thr || (fill && __float_as_int(x.y) - p.item_offset < k));
         const unsigned bal = __ballot_sync(0xffffffffu, keep);
         __syncwarp();  // all reads of this batch precede its writes (which land at or below e0)
         if (keep) pr[m2 + __popc(bal & lt)] = x;
@@ -1022,7 +1055,7 @@ __global__ void __launch_bounds__(RR_WARPS * 32) rerank_kernel(const RerankParam
 #pragma unroll
         for (int t = 0; t < 4; ++t) {
           const int e = b0 + 32 * t + lane;
-          const bool keep = e < n && (x[t].x >= thr || (p.clamp && __float_as_int(x[t].y) - p.item_offset < k));
+          const bool keep = e < n && (x[t].x >= thr || (fill && __float_as_int(x[t].y) - p.item_offset < k));
           const unsigned bal = __ballot_sync(0xffffffffu, keep);
           const int pos = m + __popc(bal & lt);
           if (keep && pos < SEL_CAP) pr[pos] = x[t];
@@ -1086,27 +1119,50 @@ __global__ void __launch_bounds__(RR_WARPS * 32) rerank_kernel(const RerankParam
     }
   }
   __syncwarp();
-  // ---- 4. rank by counting: larger key = (higher score, then lower item id); ids are distinct so ranks are too
-  for (int g0 = 0; g0 < m; g0 += 128) {
-    unsigned long long mk[4];
-    int rank[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int t = g0 + 32 * i + lane;
-      mk[i] = t < m ? keys[t] : ~0ull;
-      rank[i] = 0;
+  if (WIDE) {
+    // ---- 4'. bitonic sort, descending: larger key = (higher score, then lower item id); zero keys pad to a power of two
+    int np2 = 1;
+    while (np2 < m) np2 <<= 1;
+    for (int t = m + lane; t < np2; t += 32) keys[t] = 0ull;
+    __syncwarp();
+    for (int size = 2; size <= np2; size <<= 1) {
+      for (int stride = size >> 1; stride > 0; stride >>= 1) {
+        for (int i = lane; i < np2 / 2; i += 32) {
+          const int a = 2 * i - (i & (stride - 1));  // partner pair (a, a + stride), bit `stride` of a clear
+          const unsigned long long ka = keys[a], kb = keys[a + stride];
+          if ((ka < kb) == ((a & size) == 0)) { keys[a] = kb; keys[a + stride] = ka; }
+        }
+        __syncwarp();
+      }
     }
-    for (int o = 0; o < m; ++o) {
-      const unsigned long long ko = keys[o];
-#pragma unroll
-      for (int i = 0; i < 4; ++i) rank[i] += ko > mk[i] ? 1 : 0;
+    for (int t = lane; t < min(m, k); t += 32) {
+      const unsigned long long kt = keys[t];
+      p.out_idx[row * k + t] = (int)(0xffffffffu - (uint32_t)(kt & 0xffffffffull));
+      p.out_score[row * k + t] = key2f((uint32_t)(kt >> 32));
     }
+  } else {
+    // ---- 4. rank by counting: larger key = (higher score, then lower item id); ids are distinct so ranks are too
+    for (int g0 = 0; g0 < m; g0 += 128) {
+      unsigned long long mk[4];
+      int rank[4];
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int t = g0 + 32 * i + lane;
-      if (t < m && rank[i] < k) {
-        p.out_idx[row * k + rank[i]] = (int)(0xffffffffu - (uint32_t)(mk[i] & 0xffffffffull));
-        p.out_score[row * k + rank[i]] = key2f((uint32_t)(mk[i] >> 32));
+      for (int i = 0; i < 4; ++i) {
+        const int t = g0 + 32 * i + lane;
+        mk[i] = t < m ? keys[t] : ~0ull;
+        rank[i] = 0;
+      }
+      for (int o = 0; o < m; ++o) {
+        const unsigned long long ko = keys[o];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) rank[i] += ko > mk[i] ? 1 : 0;
+      }
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const int t = g0 + 32 * i + lane;
+        if (t < m && rank[i] < k) {
+          p.out_idx[row * k + rank[i]] = (int)(0xffffffffu - (uint32_t)(mk[i] & 0xffffffffull));
+          p.out_score[row * k + rank[i]] = key2f((uint32_t)(mk[i] >> 32));
+        }
       }
     }
   }
@@ -1120,12 +1176,13 @@ __global__ void __launch_bounds__(RR_WARPS * 32) rerank_kernel(const RerankParam
 // exact path for rows whose candidate list overflowed (huge tie groups, adversarially ordered scores): all
 // canonical scores of the row go to scratch; a block-wide radix select finds the k-th largest score T; entries > T
 // plus the lowest-indexed entries == T are collected (k in total) and ranked by (score desc, id asc).
-__global__ void __launch_bounds__(256) exact_rows_kernel(const RerankParams p, const int* __restrict__ ovf_count,
+// (At most 32 CTAs run it, so registers matter more than occupancy: minimum 1 block per SM.)
+__global__ void __launch_bounds__(256, 1) exact_rows_kernel(const RerankParams p, const int* __restrict__ ovf_count,
                                                          const int* __restrict__ ovf_rows, float* __restrict__ scratch) {
   __shared__ int hist[256];
   __shared__ int s_bin, s_krem, s_cnt_gt, s_cnt_eq, s_warp_tot[8];
-  __shared__ float sel_s[128];
-  __shared__ int sel_i[128];
+  __shared__ float sel_s[WIDE_MAX_K];
+  __shared__ int sel_i[WIDE_MAX_K];
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   const int n_ovf = *ovf_count;
   const int n = (int)p.n_items;
@@ -1202,9 +1259,9 @@ __global__ void __launch_bounds__(256) exact_rows_kernel(const RerankParams p, c
       __syncthreads();
     }
     // ---- rank the k selected entries
-    if (tid < k) {
-      const float s = sel_s[tid];
-      const int id = sel_i[tid];
+    for (int t = tid; t < k; t += 256) {
+      const float s = sel_s[t];
+      const int id = sel_i[t];
       int rank = 0;
       for (int j = 0; j < k; ++j) rank += (sel_s[j] > s) || (sel_s[j] == s && sel_i[j] < id);
       p.out_idx[row * k + rank] = id + p.item_offset;
@@ -1342,17 +1399,22 @@ static int make_tmap(CUtensorMap* map, void* base, long long rows, int k_pad, in
 struct TopkLayout {
   long long nu_pad, ni_pad, batch_rows;
   int k_pad, kb;
+  bool wide;                  // k > NARROW_MAX_K: the CAP_W / UB_BATCH_W configuration
+  int cap, ub_batch;
   size_t off_ub, off_vb, off_unorm, off_ures, off_erow, off_vnorm, off_vmax, off_cand, off_cnt, off_thr, off_ovfc, off_ovfr, off_scratch, total;
   int scratch_rows;
 };
 
 static size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
-static TopkLayout topk_layout(long long n_users, long long n_items, int r) {
+static TopkLayout topk_layout(long long n_users, long long n_items, int r, int k) {
   TopkLayout L{};
+  L.wide = k > NARROW_MAX_K;
+  L.cap = L.wide ? CAP_W : CAP;
+  L.ub_batch = L.wide ? UB_BATCH_W : UB_BATCH;
   L.nu_pad = cdiv(n_users, BM) * BM;
   L.ni_pad = cdiv(n_items, BN) * BN;
-  L.batch_rows = std::min<long long>(L.nu_pad, (long long)UB_BATCH * BM);
+  L.batch_rows = std::min<long long>(L.nu_pad, (long long)L.ub_batch * BM);
   L.k_pad = (int)(cdiv(r, BK) * BK);
   L.kb = L.k_pad / BK;
   size_t o = 0;
@@ -1363,7 +1425,7 @@ static TopkLayout topk_layout(long long n_users, long long n_items, int r) {
   L.off_erow = o; o = align_up(o + (size_t)L.nu_pad * 4, 256);
   L.off_vnorm = o; o = align_up(o + (size_t)L.ni_pad * 4, 256);
   L.off_vmax = o; o += 256;
-  L.off_cand = o; o = align_up(o + (size_t)L.batch_rows * CAP * 8, 256);
+  L.off_cand = o; o = align_up(o + (size_t)L.batch_rows * L.cap * 8, 256);
   L.off_cnt = o; o = align_up(o + (size_t)L.batch_rows * 4, 256);
   L.off_thr = o; o = align_up(o + (size_t)L.batch_rows * 4, 256);
   L.off_ovfc = o; o += 256;
@@ -1389,8 +1451,7 @@ extern "C" int tmf_pack_bf16(const float* src, int64_t n, int32_t n_comp, int32_
 }
 
 extern "C" size_t tmf_score_topk_ws_bytes(int64_t n_users, int64_t n_items, int32_t n_comp, int32_t k) {
-  (void)k;
-  return topk_layout(n_users, n_items, n_comp).total;
+  return topk_layout(n_users, n_items, n_comp, k).total;
 }
 
 static int score_topk_impl(const float* U, int64_t n_users, const float* V, int64_t n_items, int32_t n_comp, int32_t ld,
@@ -1398,10 +1459,10 @@ static int score_topk_impl(const float* U, int64_t n_users, const float* V, int6
                            size_t ws_bytes, tmf_stream_t stream, float* dump, const float* row_bound = nullptr, int force_fmt = -1) {
   TMF_REQUIRE(n_users >= 0 && n_items > 0 && n_comp > 0 && n_comp <= ld, "tmf_score_topk: bad shape");
   TMF_REQUIRE(n_comp <= MAX_KB * BK, "tmf_score_topk: n_components up to %d supported", MAX_KB * BK);
-  TMF_REQUIRE(k >= 1 && k <= 128 && k <= n_items, "tmf_score_topk: need 1 <= k <= min(128, n_items) (k=%d)", k);
+  TMF_REQUIRE(k >= 1 && k <= WIDE_MAX_K && k <= n_items, "tmf_score_topk: need 1 <= k <= min(%d, n_items) (k=%d)", WIDE_MAX_K, k);
   TMF_REQUIRE(n_items < (1ll << 31) - BN && n_users < (1ll << 31) - BM, "tmf_score_topk: sizes must fit int32");
   if (n_users == 0) return TMF_OK;
-  const TopkLayout L = topk_layout(n_users, n_items, n_comp);
+  const TopkLayout L = topk_layout(n_users, n_items, n_comp, k);
   TMF_REQUIRE(ws_bytes >= L.total, "tmf_score_topk: workspace too small");
   unsigned char* w = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 1023) & ~(uintptr_t)1023);
   __nv_bfloat16* Ub = reinterpret_cast<__nv_bfloat16*>(w + L.off_ub);
@@ -1473,26 +1534,27 @@ static int score_topk_impl(const float* U, int64_t n_users, const float* V, int6
 
   const size_t smem = 1024 + (size_t)L.kb * A_SUB_BYTES + (size_t)NSTAGES * B_STAGE_BYTES + 256 +
                       (size_t)BM * HSTRIDE * sizeof(uint32_t) + 16 + (size_t)BM * QCAP * 8 + 4 * 8 * sizeof(float);
-  TMF_CUDA(cudaFuncSetAttribute(score_topk_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  TMF_CUDA(cudaFuncSetAttribute(score_topk_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  TMF_CUDA(cudaFuncSetAttribute(score_topk_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const size_t rr_smem = (size_t)RR_WARPS * ((size_t)ld * sizeof(double) + SEL_CAP * 8 + 32 * STG_STRIDE * 4 + 16);
-  TMF_CUDA(cudaFuncSetAttribute(rerank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rr_smem));
+  auto main_kernel = L.wide ? (p.prof ? score_topk_kernel<false, true, true> : score_topk_kernel<false, false, true>)
+                            : dump != nullptr ? score_topk_kernel<true, false, false>
+                            : p.prof ? score_topk_kernel<false, true, false> : score_topk_kernel<false, false, false>;
+  TMF_CUDA(cudaFuncSetAttribute(main_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const int rr_warps = L.wide ? RR_WARPS_W : RR_WARPS;
+  const size_t rr_smem = (size_t)rr_warps * (L.wide ? rerank_warp_smem<true>(ld) : rerank_warp_smem<false>(ld));
+  auto rr_kernel = L.wide ? rerank_kernel<true> : rerank_kernel<false>;
+  TMF_CUDA(cudaFuncSetAttribute(rr_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rr_smem));
 
-  // users go through in batches of UB_BATCH blocks so the candidate workspace stays bounded; V stays packed
+  // users go through in batches of ub_batch blocks so the candidate workspace stays bounded; V stays packed
   const int total_ublocks = (int)(L.nu_pad / BM);
-  for (int ub0 = 0; ub0 < total_ublocks; ub0 += UB_BATCH) {
+  for (int ub0 = 0; ub0 < total_ublocks; ub0 += L.ub_batch) {
     p.ub0 = ub0;
-    p.n_ublocks = std::min(UB_BATCH, total_ublocks - ub0);
+    p.n_ublocks = std::min(L.ub_batch, total_ublocks - ub0);
     const int grid = std::min(2 * kNumSMs, p.n_ublocks);  // two CTAs per SM (smem- and TMEM-limited)
-    if (dump != nullptr) score_topk_kernel<true, false><<<grid, TOPK_THREADS, smem, st>>>(tmapU, tmapV, p);
-    else if (p.prof) score_topk_kernel<false, true><<<grid, TOPK_THREADS, smem, st>>>(tmapU, tmapV, p);
-    else score_topk_kernel<false, false><<<grid, TOPK_THREADS, smem, st>>>(tmapU, tmapV, p);
+    main_kernel<<<grid, TOPK_THREADS, smem, st>>>(tmapU, tmapV, p);
     TMF_LAUNCH_CHECK();
     if (dump != nullptr) continue;
     q.row0 = (long long)ub0 * BM;
     q.n_rows = std::min<long long>((long long)p.n_ublocks * BM, n_users - q.row0);
-    rerank_kernel<<<(unsigned)cdiv(q.n_rows, RR_WARPS), RR_WARPS * 32, rr_smem, st>>>(q);
+    rr_kernel<<<(unsigned)cdiv(q.n_rows, rr_warps), rr_warps * 32, rr_smem, st>>>(q);
     TMF_LAUNCH_CHECK();
   }
   if (dump != nullptr) return TMF_OK;

@@ -28,7 +28,10 @@ from .utils import gather_matrix_indices, random_sampler  # noqa: F401  (ref:20)
 
 # the fused tcgen05 top-k kernel keeps at most this many results per row; larger k (full rankings)
 # go through dense canonical scores + a segmented sort
-TOPK_FUSED_MAX_K = 128
+TOPK_FUSED_MAX_K = 1024
+# k up to this runs the kernel's narrow configuration (shorter candidate lists); recommend() keeps its
+# over-fetched list within it whenever k does
+TOPK_NARROW_MAX_K = 128
 
 
 def _public(st, r):
@@ -353,7 +356,8 @@ class MatrixFactorization:
         EXCLUDING the non-zero cells of the interaction table ``seen`` (sparse or dense, never densified).  int32 ``[n, k]``
         on the device; a user with fewer than ``k`` unseen items has its row padded with -1.
 
-        The fused tcgen05 top-k produces each row's top-``kc`` list (``kc = min(k + heaviest row, 128)``) and
+        The fused tcgen05 top-k produces each row's top-``kc`` list (``kc = min(k + heaviest row, 128)``, or ``1024`` in
+        place of ``128`` for ``128 < k <= 1024``) and
         ``tmf_filter_seen`` keeps the first ``k`` unseen entries; the few rows that have more seen items among their
         top-``kc`` than the list can absorb are ranked exactly (dense canonical scores of those rows, seen cells masked)."""
         n_u, n_i = self.user_embedding.shape[0], self.item_embedding.shape[0]
@@ -377,7 +381,7 @@ class MatrixFactorization:
             return out
         row_nnz = (a_ptr[1:] - a_ptr[:-1])
         kk = min(k, n_i)
-        kc = min(n_i, TOPK_FUSED_MAX_K, kk + int(row_nnz.max()))
+        kc = min(n_i, TOPK_NARROW_MAX_K if kk <= TOPK_NARROW_MAX_K else TOPK_FUSED_MAX_K, kk + int(row_nnz.max()))
         short = torch.ones(n, dtype=torch.int32, device=dev)
         if kc >= kk and kk <= TOPK_FUSED_MAX_K:
             cand = self._topk(kc, clamp=False, users=rows)
