@@ -178,10 +178,6 @@ TMF_API int tmf_wmrb_forward(int64_t n_pos, const int32_t* pos_rows, const float
 
 /* ------------------------------------------------------------------ scoring / top-k / metrics */
 
-/* fp32 [n, ld] -> bf16 [n_pad, k_pad] (zero padded) + per-row l2 norms; operands of the tcgen05 GEMM. */
-TMF_API int tmf_pack_bf16(const float* src, int64_t n, int32_t n_comp, int32_t ld, uint16_t* dst, int64_t n_pad,
-                  int32_t k_pad, float* norms, tmf_stream_t stream);
-
 /* U.V^T (matrix_factorization.py:195) + per-row top-k (tf.math.top_k, :245,:429) as ONE kernel:
  * tcgen05 GEMM on 16-bit operands (fp16 or bf16, whichever rounds the given embeddings more accurately),
  * accumulators in TMEM, fused threshold/candidate epilogue; then an fp32/fp64 canonical rerank so indices
@@ -196,12 +192,6 @@ TMF_API int tmf_score_topk(const float* U, int64_t n_users, const float* V, int6
                    int32_t k, int32_t clamp, int32_t item_offset, int32_t* out_idx, float* out_score, void* ws,
                    size_t ws_bytes, tmf_stream_t stream);
 
-/* The raw tensor-core scores of the same kernel, written densely (P[n_users, n_items], small shapes only):
- * used to test the bf16 error bound |s~ - s| <= 2^-8 * 1.05 * |u| * |v| that the exactness argument rests on.
- * Workspace as for tmf_score_topk with k = 1. */
-TMF_API int tmf_score_dense_bf16(const float* U, int64_t n_users, const float* V, int64_t n_items, int32_t n_comp, int32_t ld,
-                         float* P, void* ws, size_t ws_bytes, tmf_stream_t stream);
-
 /* Item-sharded scoring with an externally supplied per-row bound: row_bound[n_users] (may be NULL) holds, per
  * user, a LOWER bound of the k-th best canonical score over ALL item slabs (e.g. the k-th best score of the user
  * against any subset of the items, exchanged between GPUs).  A slab then only lists candidates that can still be in
@@ -212,8 +202,11 @@ TMF_API int tmf_score_topk_bounded(const float* U, int64_t n_users, const float*
                            int32_t k, int32_t clamp, int32_t item_offset, const float* row_bound, int32_t* out_idx,
                            float* out_score, void* ws, size_t ws_bytes, tmf_stream_t stream);
 
-/* Same with an explicit operand format: -1 = chosen from the data like tmf_score_topk does (fp16 where the embeddings fit
- * its range and it rounds them more accurately than bf16), 0 = bf16, 1 = fp16. */
+/* The raw tensor-core scores s~ of tmf_score_topk's GEMM, written densely (P[n_users, n_items], small shapes only), to
+ * test the error bound the exact top-k rests on.  With u~ = u rounded to the operand format and du = u - u~ (likewise v~, dv):
+ *   |s~ - s| <= |du| |v| + |u~| |dv| + 2.4e-7 * k_pad * |u~| |v|,   k_pad = n_comp rounded up to a multiple of 64.
+ * operand_format: -1 = chosen from the data like tmf_score_topk does (fp16 where the embeddings fit its range and it
+ * rounds them more accurately than bf16), 0 = bf16, 1 = fp16.  Workspace as for tmf_score_topk with k = 1. */
 TMF_API int tmf_score_dense_tc(const float* U, int64_t n_users, const float* V, int64_t n_items, int32_t n_comp, int32_t ld,
                        int32_t operand_format, float* P, void* ws, size_t ws_bytes, tmf_stream_t stream);
 

@@ -52,11 +52,9 @@ SIGNATURES = {
     "tmf_gather_rows2d": (_i32, [_p, _i32, _i64, _p, _i32, _p, _p]),
     "tmf_gather_nd2": (_i32, [_p, _i64, _p, _i64, _p, _p]),
     "tmf_wmrb_forward": (_i32, [_i64, _p, _p, _p, _i32, _f32, _p, _p]),
-    "tmf_pack_bf16": (_i32, [_p, _i64, _i32, _i32, _p, _i64, _i32, _p, _p]),
     "tmf_score_topk_ws_bytes": (_sz, [_i64, _i64, _i32, _i32]),
     "tmf_score_topk": (_i32, [_p, _i64, _p, _i64, _i32, _i32, _i32, _i32, _i32, _p, _p, _p, _sz, _p]),
     "tmf_score_topk_bounded": (_i32, [_p, _i64, _p, _i64, _i32, _i32, _i32, _i32, _i32, _p, _p, _p, _p, _sz, _p]),
-    "tmf_score_dense_bf16": (_i32, [_p, _i64, _p, _i64, _i32, _i32, _p, _p, _sz, _p]),
     "tmf_score_dense_tc": (_i32, [_p, _i64, _p, _i64, _i32, _i32, _i32, _p, _p, _sz, _p]),
     "tmf_topk_merge": (_i32, [_p, _p, _i32, _i64, _i32, _p, _p, _p]),
     "tmf_predict_dense": (_i32, [_p, _i64, _p, _i64, _i32, _i32, _p, _p]),

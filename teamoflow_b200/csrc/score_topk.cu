@@ -52,7 +52,7 @@ constexpr int UB_BATCH = 2048; // user blocks (x128 rows) per main-kernel launch
 // Wide configuration, 128 < k <= 1024 (DESIGN "top-k", wide k): the same kernel with longer lists.  8192 slots leave ~5k
 // appends between saturation rebuilds even in clamp mode, where the k lowest ids stay listed besides >= k entries above the
 // threshold; 592 user blocks = exactly two waves of the 2 x 148 persistent CTAs and a 4.96 GB candidate workspace.  The
-// first rebuild streams the list through warp_rebuild_row once it holds k + 2 tiles of entries (warp_rebuild_first keeps
+// first rebuild streams the list through warp_rebuild_selected once it holds k + 2 tiles of entries (warp_rebuild_first keeps
 // only INIT_N entries in registers).
 constexpr int NARROW_MAX_K = 128;
 constexpr int WIDE_MAX_K = 1024;
@@ -117,6 +117,13 @@ __device__ __forceinline__ float keep_threshold(float kth, float E, int clamp) {
   return clamp ? fmaxf(kth - E, 0.f) - E : kth - 2.f * E;
 }
 
+// Whether a list entry (approx score, item id) stays listed under keep-threshold thr.  Clamp mode also keeps the k lowest
+// item ids of the slab whatever their score: when fewer than k items score above zero, the answer is filled with zero-score
+// items in id order, and those fillers must still be listed.  Every filter of a candidate list goes through here.
+__device__ __forceinline__ bool keep_entry(float2 x, float thr, int clamp, int item_offset, int k) {
+  return x.x >= thr || (clamp && __float_as_int(x.y) - item_offset < k);
+}
+
 // ---- per-row running threshold: a lane-private 48-bin histogram of the appended scores (16-bit counts, two
 // bins per shared-memory word).  bthr = the highest bin whose "at or above" count A is still >= k, so the lower
 // edge of bin bthr is a valid lower bound of the k-th largest score seen so far; it only ever rises.
@@ -142,10 +149,13 @@ __device__ __forceinline__ void sts_u32(uint32_t a, uint32_t v) { asm volatile("
 __device__ __forceinline__ float2 lds_f2(uint32_t a) { float2 v; asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(a)); return v; }
 __device__ __forceinline__ int hist_get_s(uint32_t hrow, int b) { return (int)((lds_u32(hrow + 4u * (uint32_t)(b >> 1)) >> ((b & 1) * 16)) & 0xffffu); }
 
+// lower edge of bin bthr, less the rounding of the bin arithmetic: >= k entries are >= it (histogram invariant)
+__device__ __forceinline__ float bin_edge(float lo, float w, int bthr) {
+  const float slack = 4e-7f * (fabsf(lo) + (float)NBINS * w);
+  return lo + (float)bthr * w - slack;
+}
 __device__ __forceinline__ float edge_threshold(float lo, float w, int bthr, float E, int clamp) {
-  const float edge = lo + (float)bthr * w;
-  const float slack = 4e-7f * (fabsf(lo) + (float)NBINS * w);  // rounding of the bin arithmetic
-  return keep_threshold(edge - slack, E, clamp);
+  return keep_threshold(bin_edge(lo, w, bthr), E, clamp);
 }
 
 // warp-wide drain of the per-lane queues (all lanes must call; st.cq may differ per lane).  Iterations are
@@ -204,7 +214,7 @@ __device__ __forceinline__ void drain_queues(RowState& st, uint32_t queue, float
 // holds k + 2 tiles of entries): every column is appended directly.  (Clamp-mode "filler" items -- the k lowest ids --
 // therefore need no special case.)
 template <bool DUMP>
-__device__ __forceinline__ void epilogue_chunk(uint32_t (&r)[32], int col0, int n_items, bool tail_tile, bool valid, bool warp_inited,
+__device__ __forceinline__ void epilogue_chunk(uint32_t (&r)[32], int col0, int n_items, bool valid, bool warp_inited,
                                                RowState& st, uint32_t queue, float2* buf, uint32_t hrow, long long row,
                                                const TopkParams& p) {
   if (DUMP) {
@@ -295,18 +305,72 @@ __device__ __forceinline__ void epilogue_tile(uint32_t t_base, int col0, RowStat
     epilogue_half<CAP>(t_base + (uint32_t)(64 * h), col0 + 64 * h, st, queue, buf, hrow, p);
 }
 
-// exact k-th largest approximate score of a row's list (n entries in global memory, streamed through L2) by an
-// 8-bit-per-pass radix select; also returns the list maximum.  radix: 256 ints of shared-memory scratch.
-__device__ __noinline__ float warp_select_kth(const float2* buf, int n, int k, int* radix, float& mx_out) {
+// One step of an 8-bit radix select over 256 shared-memory counters: returns the bin that holds the krem-th largest counted
+// entry (bins ranked from 255 down) and sets krem to that entry's rank within the bin.  All lanes; the counted entries
+// must number >= krem.
+__device__ __forceinline__ int pick_bin(const int* cnt256, int& krem) {
+  const int lane = threadIdx.x & 31;
+  int c[8];
+  int lsum = 0;
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {  // lane L owns bins 255-8L .. 248-8L, visited in descending order
+    c[i] = cnt256[255 - 8 * lane - i];
+    lsum += c[i];
+  }
+  int incl = lsum;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int v = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += v;
+  }
+  const unsigned reach = __ballot_sync(0xffffffffu, incl >= krem);
+  const int F = reach ? __ffs(reach) - 1 : 31;
+  int bin = 0, knew = 0;
+  if (lane == F) {
+    int cum = incl - lsum;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      if (cum + c[i] >= krem) { bin = 255 - 8 * lane - i; knew = krem - cum; break; }
+      cum += c[i];
+    }
+  }
+  krem = __shfl_sync(0xffffffffu, knew, F);
+  return __shfl_sync(0xffffffffu, bin, F);
+}
+
+// Exact k-th largest of a warp's entries by an 8-bit-per-pass radix select.  count(shift, mask, prefix) visits the entries
+// and counts each whose key matches prefix under mask into radix[(key >> shift) & 255] (256 ints of shared-memory scratch,
+// see count_key).  Needs >= k entries.
+template <class Count>
+__device__ __forceinline__ float radix_select_kth(int k, int* radix, Count count) {
   const int lane = threadIdx.x & 31;
   uint32_t prefix = 0, mask = 0;
   int krem = k;
-  float mx = -INFINITY;
 #pragma unroll 1
   for (int shift = 24; shift >= 0; shift -= 8) {
 #pragma unroll
     for (int i = 0; i < 8; ++i) radix[lane * 8 + i] = 0;
     __syncwarp();
+    count(shift, mask, prefix);
+    __syncwarp();
+    const int bin = pick_bin(radix, krem);
+    prefix |= (uint32_t)bin << shift;
+    mask |= 255u << shift;
+    __syncwarp();
+  }
+  return key2f(prefix);
+}
+__device__ __forceinline__ void count_key(int* radix, float x, int shift, uint32_t mask, uint32_t prefix) {
+  const uint32_t key = f2key(x);
+  if ((key & mask) == prefix) smem_inc(&radix[(key >> shift) & 255u]);
+}
+
+// exact k-th largest approximate score of a row's list (n >= k entries in global memory, streamed through L2); also
+// returns the list maximum
+__device__ __noinline__ float warp_select_kth(const float2* buf, int n, int k, int* radix, float& mx_out) {
+  const int lane = threadIdx.x & 31;
+  float mx = -INFINITY;
+  const float kth = radix_select_kth(k, radix, [&](int shift, uint32_t mask, uint32_t prefix) {
     for (int e0 = 0; e0 < n; e0 += 32 * 8) {  // 8 independent loads in flight per lane (one L2 round trip per 256 entries)
       float sc[8];
 #pragma unroll
@@ -318,105 +382,48 @@ __device__ __noinline__ float warp_select_kth(const float2* buf, int n, int k, i
       for (int t = 0; t < 8; ++t) {
         if (e0 + 32 * t + lane < n) {
           mx = fmaxf(mx, sc[t]);
-          const uint32_t key = f2key(sc[t]);
-          if ((key & mask) == prefix) smem_inc(&radix[(key >> shift) & 255u]);
+          count_key(radix, sc[t], shift, mask, prefix);
         }
       }
     }
-    __syncwarp();
-    int c[8];
-    int lsum = 0;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {  // lane L owns bins 255-8L .. 248-8L, visited in descending order
-      c[i] = radix[255 - 8 * lane - i];
-      lsum += c[i];
-    }
-    int incl = lsum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int v = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= o) incl += v;
-    }
-    const unsigned reach = __ballot_sync(0xffffffffu, incl >= krem);
-    const int F = reach ? __ffs(reach) - 1 : 31;  // reach != 0 whenever n >= k
-    int bin = 0, knew = 0;
-    if (lane == F) {
-      int cum = incl - lsum;
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        if (cum + c[i] >= krem) { bin = 255 - 8 * lane - i; knew = krem - cum; break; }
-        cum += c[i];
-      }
-    }
-    bin = __shfl_sync(0xffffffffu, bin, F);
-    krem = __shfl_sync(0xffffffffu, knew, F);
-    prefix |= (uint32_t)bin << shift;
-    mask |= 255u << shift;
-    __syncwarp();
-  }
+  });
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
   mx_out = mx;
-  return key2f(prefix);
+  return kth;
 }
 
-// Warp-cooperative (re)build of one row's threshold state from its list of n (<= CAP) entries, streamed from L2:
-// exact k-th largest by radix select, histogram re-centred on [kth, kth + 4 (max - kth)), list compacted in place
-// against the new threshold (clamp mode also keeps the k lowest item ids).  Used once when a row has seen its first
-// 3 tiles and again whenever its list is about to saturate, so a badly placed histogram range heals itself.
-// Results in out[0..5] (shared memory): lo, w, inv_w, bthr, A, n_new.
-__device__ __noinline__ void warp_rebuild_row(float2* buf, int n, int k, int clamp, int item_offset, float E, uint32_t* hrow,
-                                              int* radix, float* out) {
+// Bin width of a row histogram re-centred on [lo, lo + range (row max - lo)); a degenerate range (all entries equal, or
+// not finite) falls back to a narrow one above lo.
+__device__ __forceinline__ void hist_range(float lo, float row_max, float range, float& w, float& inv_w) {
+  float W = range * (row_max - lo);
+  if (!(W > 0.f) || !(W < 3e38f)) W = fmaxf(fabsf(lo), 1.0f) * 1e-3f;
+  w = W / (float)NBINS;
+  inv_w = (float)NBINS / W;
+}
+
+// Empties a row's histogram and records the row maximum (word NBINS/2 holds its key).  All lanes.
+__device__ __forceinline__ void hist_reset(uint32_t* hrow, float row_max) {
   const int lane = threadIdx.x & 31;
-  const unsigned lt = (1u << lane) - 1u;
-  float mx;
-  const float kth = warp_select_kth(buf, n, k, radix, mx);
-  float W = 4.0f * (mx - kth);
-  if (!(W > 0.f) || !(W < 3e38f)) W = fmaxf(fabsf(kth), 1.0f) * 1e-3f;
-  const float lo = kth;
-  const float w = W / (float)NBINS;
-  const float inv_w = (float)NBINS / W;
-  const float thr = keep_threshold(kth, E, clamp);  // exact k-th: the tightest valid threshold
-  // ---- compact in place against thr and rebuild the histogram from the kept entries >= lo
   for (int i = lane; i < HSTRIDE; i += 32) hrow[i] = 0u;
   __syncwarp();
-  if (lane == 0) hrow[NBINS / 2] = f2key(mx);
-  int base = 0;
-  for (int b0 = 0; b0 < n; b0 += 32 * 8) {
-    float2 x[8];
-#pragma unroll
-    for (int t = 0; t < 8; ++t) {
-      const int e = b0 + 32 * t + lane;
-      x[t] = (e < n) ? __ldcg(buf + e) : make_float2(-INFINITY, 0.f);
+  if (lane == 0) hrow[NBINS / 2] = f2key(row_max);
+}
+
+// One step of the in-place list compaction of a rebuild, an entry per lane: kept entries are written in lane order from
+// buf[base] (every read of the step precedes its writes, which land at or below the entries read) and those >= lo are
+// counted into the histogram.  All lanes; returns the new base.
+__device__ __forceinline__ int compact_step(float2* buf, int base, float2 x, bool keep, uint32_t* hrow, float lo, float inv_w) {
+  const int lane = threadIdx.x & 31;
+  const unsigned bal = __ballot_sync(0xffffffffu, keep);
+  if (keep) {
+    __stcg(buf + base + __popc(bal & ((1u << lane) - 1u)), x);
+    if (x.x >= lo) {
+      const int b = (int)fminf((x.x - lo) * inv_w, (float)(NBINS - 1));
+      asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(smem_u32(&hrow[b >> 1])), "r"(1u << ((b & 1) * 16)) : "memory");
     }
-    __syncwarp();  // every read of this batch precedes its writes (writes land at or below b0)
-#pragma unroll
-    for (int t = 0; t < 8; ++t) {
-      const int e = b0 + 32 * t + lane;
-      const bool keep = e < n && (x[t].x >= thr || (clamp && __float_as_int(x[t].y) - item_offset < k));
-      const unsigned bal = __ballot_sync(0xffffffffu, keep);
-      if (keep) {
-        __stcg(buf + base + __popc(bal & lt), x[t]);
-        if (x[t].x >= lo) {
-          const int b = (int)fminf((x[t].x - lo) * inv_w, (float)(NBINS - 1));
-          asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(smem_u32(&hrow[b >> 1])), "r"(1u << ((b & 1) * 16)) : "memory");
-        }
-      }
-      base += __popc(bal);
-    }
-    __syncwarp();
   }
-  if (lane == 0) {
-    // highest bin with at least k entries at or above it (bin 0 qualifies: >= k entries are >= kth)
-    int A = 0, bthr = 0;
-    for (int b = NBINS - 1; b >= 0; --b) {
-      A += hist_get(hrow, b);
-      if (A >= k) { bthr = b; break; }
-    }
-    out[0] = lo; out[1] = w; out[2] = inv_w; out[3] = __int_as_float(bthr); out[4] = __int_as_float(A);
-    out[5] = __int_as_float(base);
-  }
-  __syncwarp();
+  return base + __popc(bal);
 }
 
 // all lanes: highest bin with at least k entries at or above it (bin 0 qualifies whenever >= k entries are >= lo).
@@ -449,17 +456,59 @@ __device__ __forceinline__ void finish_rebuild(const uint32_t* hrow, int k, floa
   }
 }
 
+// Warp-cooperative rebuild of one row's threshold state from its list of n (<= CAP) entries, ONE streaming pass through L2:
+// given a lower bound lo of the row's k-th largest approximate score and the row maximum, the list is compacted in place
+// against max(keep_threshold(lo), thr_floor) (clamp mode also keeps the k lowest item ids) and the kept entries are re-binned
+// into a histogram re-centred on [lo, lo + range (row max - lo)).  Two uses:
+//  - SATURATION of a row whose histogram is live: lo = the current bin edge (a valid lower bound by the histogram
+//    invariant, so no selection is needed), range 2 -- finer bins, hence a tighter running threshold from here on;
+//  - the first rebuild at wide k, and a bounded row (idle histogram) that filled up anyway: lo = the exact k-th largest
+//    (warp_select_kth), range 4, no floor.
+// Results in out[0..5] (shared memory): lo, w, inv_w, bthr, A, n_new.
+__device__ __noinline__ void warp_rebuild(float2* buf, int n, int k, int clamp, int item_offset, float E, uint32_t* hrow,
+                                          float lo, float row_max, float range, float thr_floor, float* out) {
+  const int lane = threadIdx.x & 31;
+  const float thr = fmaxf(keep_threshold(lo, E, clamp), thr_floor);
+  float w, inv_w;
+  hist_range(lo, row_max, range, w, inv_w);
+  __syncwarp();
+  hist_reset(hrow, row_max);
+  int base = 0;
+  for (int b0 = 0; b0 < n; b0 += 32 * 8) {
+    float2 x[8];
+#pragma unroll
+    for (int t = 0; t < 8; ++t) {
+      const int e = b0 + 32 * t + lane;
+      x[t] = (e < n) ? __ldcg(buf + e) : make_float2(-INFINITY, 0.f);
+    }
+    __syncwarp();  // every read of this batch precedes its writes (writes land at or below b0)
+#pragma unroll
+    for (int t = 0; t < 8; ++t)
+      base = compact_step(buf, base, x[t], b0 + 32 * t + lane < n && keep_entry(x[t], thr, clamp, item_offset, k), hrow, lo, inv_w);
+    __syncwarp();
+  }
+  finish_rebuild(hrow, k, lo, w, inv_w, base, out);
+  __syncwarp();
+}
+
+// the rebuild from the exact k-th largest entry (no valid lower bound of it is known): selection first, no floor
+__device__ __noinline__ void warp_rebuild_selected(float2* buf, int n, int k, int clamp, int item_offset, float E, uint32_t* hrow,
+                                                   int* radix, float* out) {
+  float mx;
+  const float kth = warp_select_kth(buf, n, k, radix, mx);
+  warp_rebuild(buf, n, k, clamp, item_offset, E, hrow, kth, mx, 4.0f, -INFINITY, out);
+}
+
 // ---- FIRST (re)build of a row (n <= INIT_N entries), entirely in registers.  The entries are loaded once (CPL per lane,
 // one L2 round trip) and bucketed linearly over [min, max] into 256 shared-memory counters -- low contention, where the
 // radix passes of warp_select_kth pile most keys onto one exponent bucket; the bucket holding the k-th largest is
 // re-bucketed once over its own [min, max].  The smallest member of the final bucket is the bound: by construction at
 // least k entries are >= it, and it lies within 2^-16 of the score range of the exact k-th.  ~400 instructions per row
 // where the four streaming radix passes took ~42 k cycles (25 % of a 125k-item sweep, measured with TMF_TOPK_PROF).
-// Outputs as warp_rebuild_row; word NBINS/2 of the histogram row receives the key of the row maximum.
+// Outputs as warp_rebuild.
 __device__ __noinline__ void warp_rebuild_first(float2* buf, int n, int k, int clamp, int item_offset, float E, uint32_t* hrow,
                                                 int* cnt256, float* out) {
   const int lane = threadIdx.x & 31;
-  const unsigned lt = (1u << lane) - 1u;
   float2 x[CPL];
 #pragma unroll
   for (int t = 0; t < CPL; ++t) {
@@ -493,32 +542,7 @@ __device__ __noinline__ void warp_rebuild_first(float2* buf, int n, int k, int c
       if ((mem >> t) & 1u) smem_inc(&cnt256[bk[t]]);
     }
     __syncwarp();
-    int c[8];
-    int lsum = 0;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {  // lane L owns buckets 255-8L .. 248-8L, visited in descending order
-      c[i] = cnt256[255 - 8 * lane - i];
-      lsum += c[i];
-    }
-    int incl = lsum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int v = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= o) incl += v;
-    }
-    const unsigned reach = __ballot_sync(0xffffffffu, incl >= krem);
-    const int F = reach ? __ffs(reach) - 1 : 31;  // reach != 0: the members number >= krem
-    int bin = 0, knew = 1;
-    if (lane == F) {
-      int cum = incl - lsum;
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        if (cum + c[i] >= krem) { bin = 255 - 8 * lane - i; knew = krem - cum; break; }
-        cum += c[i];
-      }
-    }
-    bin = __shfl_sync(0xffffffffu, bin, F);
-    krem = __shfl_sync(0xffffffffu, knew, F);
+    const int bin = pick_bin(cnt256, krem);  // the members number >= krem
     float nlo = INFINITY, nhi = -INFINITY;
 #pragma unroll
     for (int t = 0; t < CPL; ++t) {
@@ -534,106 +558,56 @@ __device__ __noinline__ void warp_rebuild_first(float2* buf, int n, int k, int c
     __syncwarp();
   }
   const float kth = lo_b;  // >= k entries are >= kth
-  float W = 4.0f * (row_max - kth);
-  if (!(W > 0.f) || !(W < 3e38f)) W = fmaxf(fabsf(kth), 1.0f) * 1e-3f;
-  const float lo = kth;
-  const float w = W / (float)NBINS;
-  const float inv_w = (float)NBINS / W;
   const float thr = keep_threshold(kth, E, clamp);
-  for (int i = lane; i < HSTRIDE; i += 32) hrow[i] = 0u;
-  __syncwarp();
-  if (lane == 0) hrow[NBINS / 2] = f2key(row_max);
+  float w, inv_w;
+  hist_range(kth, row_max, 4.0f, w, inv_w);
+  hist_reset(hrow, row_max);
   int base = 0;
 #pragma unroll
-  for (int t = 0; t < CPL; ++t) {
-    const bool keep = (lane + 32 * t < n) && (x[t].x >= thr || (clamp && __float_as_int(x[t].y) - item_offset < k));
-    const unsigned bal = __ballot_sync(0xffffffffu, keep);
-    if (keep) {
-      __stcg(buf + base + __popc(bal & lt), x[t]);
-      if (x[t].x >= lo) {
-        const int b = (int)fminf((x[t].x - lo) * inv_w, (float)(NBINS - 1));
-        asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(smem_u32(&hrow[b >> 1])), "r"(1u << ((b & 1) * 16)) : "memory");
-      }
-    }
-    base += __popc(bal);
-  }
+  for (int t = 0; t < CPL; ++t)
+    base = compact_step(buf, base, x[t], lane + 32 * t < n && keep_entry(x[t], thr, clamp, item_offset, k), hrow, kth, inv_w);
   __syncwarp();
-  finish_rebuild(hrow, k, lo, w, inv_w, base, out);
-  __syncwarp();
-}
-
-// ---- SATURATION rebuild of a row whose histogram is live: ONE streaming pass.  The current bin edge is already a valid
-// lower bound of the k-th largest, so no selection is needed: the list is compacted against the current threshold and the
-// kept entries are re-binned into a histogram re-centred on [edge, edge + 2 (row max - edge)) -- finer bins, hence a tighter
-// running threshold from here on.  (The select-based rebuild streamed the ~2000 entries five times.)
-__device__ __noinline__ void warp_rebuild_saturated(float2* buf, int n, int k, int clamp, int item_offset, float E, uint32_t* hrow,
-                                                    float lo_old, float w_old, int bthr_old, float thr_floor, float* out) {
-  const int lane = threadIdx.x & 31;
-  const unsigned lt = (1u << lane) - 1u;
-  const float slack = 4e-7f * (fabsf(lo_old) + (float)NBINS * w_old);
-  const float edge = lo_old + (float)bthr_old * w_old - slack;   // >= k entries are >= edge (histogram invariant)
-  const float row_max = key2f(hrow[NBINS / 2]);
-  const float thr = fmaxf(keep_threshold(edge, E, clamp), thr_floor);
-  float W = 2.0f * (row_max - edge);
-  if (!(W > 0.f) || !(W < 3e38f)) W = fmaxf(fabsf(edge), 1.0f) * 1e-3f;
-  const float lo = edge;
-  const float w = W / (float)NBINS;
-  const float inv_w = (float)NBINS / W;
-  __syncwarp();
-  for (int i = lane; i < HSTRIDE; i += 32) hrow[i] = 0u;
-  __syncwarp();
-  if (lane == 0) hrow[NBINS / 2] = f2key(row_max);
-  int base = 0;
-  for (int b0 = 0; b0 < n; b0 += 32 * 8) {
-    float2 x[8];
-#pragma unroll
-    for (int t = 0; t < 8; ++t) {
-      const int e = b0 + 32 * t + lane;
-      x[t] = (e < n) ? __ldcg(buf + e) : make_float2(-INFINITY, 0.f);
-    }
-    __syncwarp();  // every read of this batch precedes its writes (writes land at or below b0)
-#pragma unroll
-    for (int t = 0; t < 8; ++t) {
-      const int e = b0 + 32 * t + lane;
-      const bool keep = e < n && (x[t].x >= thr || (clamp && __float_as_int(x[t].y) - item_offset < k));
-      const unsigned bal = __ballot_sync(0xffffffffu, keep);
-      if (keep) {
-        __stcg(buf + base + __popc(bal & lt), x[t]);
-        if (x[t].x >= lo) {
-          const int b = (int)fminf((x[t].x - lo) * inv_w, (float)(NBINS - 1));
-          asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(smem_u32(&hrow[b >> 1])), "r"(1u << ((b & 1) * 16)) : "memory");
-        }
-      }
-      base += __popc(bal);
-    }
-    __syncwarp();
-  }
-  finish_rebuild(hrow, k, lo, w, inv_w, base, out);
+  finish_rebuild(hrow, k, kth, w, inv_w, base, out);
   __syncwarp();
 }
 
 // ------------------------------------------------------------------ the fused kernel
-// WIDE: the configuration for 128 < k <= 1024 (CAP_W list slots, first rebuild by warp_rebuild_row)
+// Byte offsets of the kernel's dynamic shared memory from a 1024-byte aligned base (the swizzled operand tiles need it).
+// The kernel carves with it and the host sizes the allocation with it (total + 1024 bytes of room to align the base).
+struct TopkSmem { int b, bars, tmem_slot, hist, queues, rebuild_out, total; };
+__host__ __device__ __forceinline__ TopkSmem topk_smem(int kb) {
+  TopkSmem s;
+  s.b = kb * A_SUB_BYTES;                                      // A: kb sub-tiles of [BM][64] bf16
+  s.bars = s.b + NSTAGES * B_STAGE_BYTES;                      // B: NSTAGES x [BN][64] bf16
+  s.tmem_slot = s.bars + (2 * NSTAGES + 6) * 8;                // mbarriers: full/empty per stage, A full/empty, TMEM full/empty x2
+  s.hist = s.tmem_slot + 16;                                   // [BM][HSTRIDE] per-row score histograms
+  s.queues = (s.hist + BM * HSTRIDE * 4 + 15) & ~15;           // [BM][QCAP] survivor queues
+  s.rebuild_out = s.queues + BM * QCAP * 8;                    // [4 warps][8] rebuild results
+  s.total = s.rebuild_out + 4 * 8 * 4;
+  return s;
+}
+
+// WIDE: the configuration for 128 < k <= 1024 (CAP_W list slots, first rebuild by warp_rebuild_selected)
 template <bool DUMP, bool PROF, bool WIDE>
 __global__ void __launch_bounds__(TOPK_THREADS, 2)
 score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_constant__ CUtensorMap tmapV, const TopkParams p) {
   constexpr int cap = WIDE ? CAP_W : CAP;
   extern __shared__ __align__(1024) unsigned char smem_raw[];
-  // carve (1024-byte aligned operand tiles first)
   unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  unsigned char* sA = smem;                                   // kb sub-tiles of [128][64] bf16
-  unsigned char* sB = sA + p.kb * A_SUB_BYTES;                // NSTAGES x [BN][64] bf16
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sB + NSTAGES * B_STAGE_BYTES);
+  const TopkSmem S = topk_smem(p.kb);
+  unsigned char* sA = smem;
+  unsigned char* sB = smem + S.b;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + S.bars);
   uint64_t* full_bar = bars;                  // [NSTAGES]
   uint64_t* empty_bar = bars + NSTAGES;       // [NSTAGES]
   uint64_t* a_full = bars + 2 * NSTAGES;      // [1]
   uint64_t* a_empty = a_full + 1;             // [1]
   uint64_t* tfull = a_empty + 1;              // [2]
   uint64_t* tempty = tfull + 2;               // [2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 2);
-  uint32_t* hist_rows = reinterpret_cast<uint32_t*>(tmem_slot + 4);             // [BM][HSTRIDE] per-row score histograms
-  float2* queues = reinterpret_cast<float2*>((reinterpret_cast<uintptr_t>(hist_rows + BM * HSTRIDE) + 15) & ~(uintptr_t)15);  // [BM][QCAP]
-  float* init_out = reinterpret_cast<float*>(queues + BM * QCAP);  // [4 warps][8]
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + S.tmem_slot);
+  uint32_t* hist_rows = reinterpret_cast<uint32_t*>(smem + S.hist);
+  float2* queues = reinterpret_cast<float2*>(smem + S.queues);
+  float* init_out = reinterpret_cast<float*>(smem + S.rebuild_out);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   auto now = [] () -> long long { return PROF ? clock64() : 0ll; };  // cycle counters only in the profiling build
@@ -775,7 +749,6 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
         w_tfull += t1 - t0;
         tcgen05_fence_after();
         const uint32_t t_base = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * BN);
-        const bool tail_tile = (nt + 1) * BN > n_items;
         if (!DUMP && warp_inited && TMF_DBG(p) < 2) {
           epilogue_tile<cap>(t_base, nt * BN, st, queue, buf, hrow, p);
         } else if (TMF_DBG(p) < 3) {
@@ -786,10 +759,10 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
             // chunk ch is in ra; chunk ch+1 is fetched into rb while ra is filtered (and vice versa)
             tmem_ld_wait_for(ra);
             tmem_ld32(t_base + (uint32_t)((ch + 1) * 32), rb);
-            epilogue_chunk<DUMP>(ra, nt * BN + ch * 32, n_items, tail_tile, valid, warp_inited, st, queue, buf, hrow, row, p);
+            epilogue_chunk<DUMP>(ra, nt * BN + ch * 32, n_items, valid, warp_inited, st, queue, buf, hrow, row, p);
             tmem_ld_wait_for(rb);
             if (ch + 2 < BN / 32) tmem_ld32(t_base + (uint32_t)((ch + 2) * 32), ra);
-            epilogue_chunk<DUMP>(rb, nt * BN + (ch + 1) * 32, n_items, tail_tile, valid, warp_inited, st, queue, buf, hrow, row, p);
+            epilogue_chunk<DUMP>(rb, nt * BN + (ch + 1) * 32, n_items, valid, warp_inited, st, queue, buf, hrow, row, p);
           }
         }
         // accumulator drained: hand it back to the MMA warp before any list maintenance
@@ -834,10 +807,11 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
               const float w_o = __shfl_sync(0xffffffffu, st.w, owner);
               const int bthr_o = __shfl_sync(0xffffffffu, st.bthr, owner);
               const float ext_o = __shfl_sync(0xffffffffu, st.thr_ext, owner);
-              warp_rebuild_saturated(obuf, n_o, p.k, p.clamp, p.item_offset, E_o, ohist, lo_o, w_o, bthr_o, ext_o, iout);
-            } else {  // a bounded row (idle histogram) that filled up anyway: full selection
+              warp_rebuild(obuf, n_o, p.k, p.clamp, p.item_offset, E_o, ohist, bin_edge(lo_o, w_o, bthr_o), key2f(ohist[NBINS / 2]), 2.0f,
+                           ext_o, iout);
+            } else {  // first rebuild at wide k, or a bounded row (idle histogram) that filled up anyway: full selection
               which = 2;
-              warp_rebuild_row(obuf, n_o, p.k, p.clamp, p.item_offset, E_o, ohist, radix, iout);
+              warp_rebuild_selected(obuf, n_o, p.k, p.clamp, p.item_offset, E_o, ohist, radix, iout);
             }
             if (PROF && lane == 0) { atomicAdd(p.prof + 13 + 2 * which, (unsigned long long)(now() - tr)); atomicAdd(p.prof + 12 + 2 * which, 1ull); }
             if (lane == owner) {
@@ -905,52 +879,30 @@ struct RerankParams {
   float* out_score;
 };
 
-// k-th largest of m (<= SEL_CAP / SEL_CAP_W) scores held in shared memory pairs (score, id): 8-bit radix select, one warp
-__device__ __forceinline__ float smem_select_kth(const float2* pr, int m, int k, int* radix) {
+// Streams a row's list of n entries from global memory (DEPTH loads in flight per lane) and gathers those that pass
+// keep_entry into pr[0, SEL_CAP), in list order.  Returns how many passed: beyond SEL_CAP they are counted, not stored.
+template <int SEL_CAP, int DEPTH>
+__device__ __forceinline__ int gather_kept(const float2* buf, int n, float thr, int clamp, int item_offset, int k, float2* pr) {
   const int lane = threadIdx.x & 31;
-  uint32_t prefix = 0, mask = 0;
-  int krem = k;
-#pragma unroll 1
-  for (int shift = 24; shift >= 0; shift -= 8) {
+  const unsigned lt = (1u << lane) - 1u;
+  int m = 0;
+  for (int b0 = 0; b0 < n; b0 += 32 * DEPTH) {
+    float2 x[DEPTH];
 #pragma unroll
-    for (int i = 0; i < 8; ++i) radix[lane * 8 + i] = 0;
-    __syncwarp();
-    for (int e = lane; e < m; e += 32) {
-      const uint32_t key = f2key(pr[e].x);
-      if ((key & mask) == prefix) smem_inc(&radix[(key >> shift) & 255u]);
+    for (int t = 0; t < DEPTH; ++t) {
+      const int e = b0 + 32 * t + lane;
+      x[t] = (e < n) ? __ldcg(buf + e) : make_float2(-INFINITY, 0.f);
     }
-    __syncwarp();
-    int c[8];
-    int lsum = 0;
 #pragma unroll
-    for (int i = 0; i < 8; ++i) {  // lane L owns bins 255-8L .. 248-8L, visited in descending order
-      c[i] = radix[255 - 8 * lane - i];
-      lsum += c[i];
+    for (int t = 0; t < DEPTH; ++t) {
+      const bool keep = b0 + 32 * t + lane < n && keep_entry(x[t], thr, clamp, item_offset, k);
+      const unsigned bal = __ballot_sync(0xffffffffu, keep);
+      const int pos = m + __popc(bal & lt);
+      if (keep && pos < SEL_CAP) pr[pos] = x[t];
+      m += __popc(bal);
     }
-    int incl = lsum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int v = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= o) incl += v;
-    }
-    const unsigned reach = __ballot_sync(0xffffffffu, incl >= krem);
-    const int F = reach ? __ffs(reach) - 1 : 31;
-    int bin = 0, knew = 0;
-    if (lane == F) {
-      int cum = incl - lsum;
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        if (cum + c[i] >= krem) { bin = 255 - 8 * lane - i; knew = krem - cum; break; }
-        cum += c[i];
-      }
-    }
-    bin = __shfl_sync(0xffffffffu, bin, F);
-    krem = __shfl_sync(0xffffffffu, knew, F);
-    prefix |= (uint32_t)bin << shift;
-    mask |= 255u << shift;
-    __syncwarp();
   }
-  return key2f(prefix);
+  return m;
 }
 
 constexpr int STG_COLS = 64;              // fp32 components per staged slice of an item row
@@ -998,30 +950,15 @@ __global__ void __launch_bounds__((WIDE ? RR_WARPS_W : RR_WARPS) * 32) rerank_ke
   for (int c = lane; c < p.ld; c += 32) ud[c] = (double)p.U[row * p.ld + c];
   float thr = p.thr[lrow];
   // ---- 1. superset by the main kernel's final threshold (or the clamp-mode filler rule)
-  int m = 0;
-  for (int b0 = 0; b0 < n; b0 += 256) {
-    float2 x[8];
-#pragma unroll
-    for (int t = 0; t < 8; ++t) {
-      const int e = b0 + 32 * t + lane;
-      x[t] = (e < n) ? __ldcg(buf + e) : make_float2(-INFINITY, 0.f);
-    }
-#pragma unroll
-    for (int t = 0; t < 8; ++t) {
-      const int e = b0 + 32 * t + lane;
-      const bool keep = e < n && (x[t].x >= thr || (p.clamp && __float_as_int(x[t].y) - p.item_offset < k));
-      const unsigned bal = __ballot_sync(0xffffffffu, keep);
-      const int pos = m + __popc(bal & lt);
-      if (keep && pos < SEL_CAP) pr[pos] = x[t];
-      m += __popc(bal);
-    }
-  }
+  int m = gather_kept<SEL_CAP, 8>(buf, n, thr, p.clamp, p.item_offset, k, pr);
   __syncwarp();
   // ---- 2. exact k-th largest approximate score -> final keep-threshold, compact in place
   if (n > k && m > k) {  // (m <= k: an externally bounded row with few local candidates keeps them all)
     float kth;
     if (m <= SEL_CAP) {
-      kth = smem_select_kth(pr, m, k, radix);
+      kth = radix_select_kth(k, radix, [&](int shift, uint32_t mask, uint32_t prefix) {
+        for (int e = lane; e < m; e += 32) count_key(radix, pr[e].x, shift, mask, prefix);
+      });
     } else {  // loose running threshold (badly placed histogram): select over the whole list in global memory
       float mx;
       kth = warp_select_kth(buf, n, k, radix, mx);
@@ -1036,7 +973,7 @@ __global__ void __launch_bounds__((WIDE ? RR_WARPS_W : RR_WARPS) * 32) rerank_ke
       for (int e0 = 0; e0 < m; e0 += 32) {
         const int e = e0 + lane;
         const float2 x = e < m ? pr[e] : make_float2(-INFINITY, 0.f);
-        const bool keep = e < m && (x.x >= thr || (fill && __float_as_int(x.y) - p.item_offset < k));
+        const bool keep = e < m && keep_entry(x, thr, fill, p.item_offset, k);
         const unsigned bal = __ballot_sync(0xffffffffu, keep);
         __syncwarp();  // all reads of this batch precede its writes (which land at or below e0)
         if (keep) pr[m2 + __popc(bal & lt)] = x;
@@ -1044,24 +981,7 @@ __global__ void __launch_bounds__((WIDE ? RR_WARPS_W : RR_WARPS) * 32) rerank_ke
       }
       m = m2;
     } else {
-      m = 0;
-      for (int b0 = 0; b0 < n; b0 += 128) {
-        float2 x[4];
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-          const int e = b0 + 32 * t + lane;
-          x[t] = (e < n) ? __ldcg(buf + e) : make_float2(-INFINITY, 0.f);
-        }
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-          const int e = b0 + 32 * t + lane;
-          const bool keep = e < n && (x[t].x >= thr || (fill && __float_as_int(x[t].y) - p.item_offset < k));
-          const unsigned bal = __ballot_sync(0xffffffffu, keep);
-          const int pos = m + __popc(bal & lt);
-          if (keep && pos < SEL_CAP) pr[pos] = x[t];
-          m += __popc(bal);
-        }
-      }
+      m = gather_kept<SEL_CAP, 4>(buf, n, thr, fill, p.item_offset, k, pr);
     }
   }
   if (m > SEL_CAP) {  // too many near-ties to rank here
@@ -1289,7 +1209,7 @@ __device__ __forceinline__ bool use_fp16(const float* stats) {
   return e16 < ebf;
 }
 
-__global__ void __launch_bounds__(256) operand_stats_kernel(const float* __restrict__ src, long long n, int r, int ld, float* __restrict__ stats) {
+__global__ void __launch_bounds__(256) operand_stats_kernel(const float* __restrict__ src, long long n, int ld, float* __restrict__ stats) {
   float ss = 0.f, s16 = 0.f, sbf = 0.f, mx = 0.f;
   const int lane = threadIdx.x & 31;
   const long long warps = ((long long)gridDim.x * blockDim.x) >> 5;
@@ -1310,7 +1230,6 @@ __global__ void __launch_bounds__(256) operand_stats_kernel(const float* __restr
       }
     }
   }
-  (void)r;
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     ss += __shfl_xor_sync(0xffffffffu, ss, o);
@@ -1440,16 +1359,6 @@ static TopkLayout topk_layout(long long n_users, long long n_items, int r, int k
 
 using namespace tmf;
 
-extern "C" int tmf_pack_bf16(const float* src, int64_t n, int32_t n_comp, int32_t ld, uint16_t* dst, int64_t n_pad,
-                             int32_t k_pad, float* norms, tmf_stream_t stream) {
-  TMF_REQUIRE(n_pad >= n && k_pad >= n_comp && n_comp <= ld, "tmf_pack_bf16: bad shape");
-  if (n_pad == 0) return TMF_OK;
-  pack_bf16_kernel<<<(unsigned)cdiv(n_pad * 32, 256), 256, 0, as_stream(stream)>>>(src, n, n_comp, ld, reinterpret_cast<__nv_bfloat16*>(dst),
-                                                                                n_pad, k_pad, norms, nullptr, nullptr, nullptr, 0, nullptr, 0);
-  TMF_LAUNCH_CHECK();
-  return TMF_OK;
-}
-
 extern "C" size_t tmf_score_topk_ws_bytes(int64_t n_users, int64_t n_items, int32_t n_comp, int32_t k) {
   return topk_layout(n_users, n_items, n_comp, k).total;
 }
@@ -1492,8 +1401,8 @@ static int score_topk_impl(const float* U, int64_t n_users, const float* V, int6
   if (force_fmt < 0) {
     TMF_CUDA(cudaMemsetAsync(fmt_stats, 0, 32, st));
     const int sgrid = 8 * kNumSMs;
-    operand_stats_kernel<<<sgrid, 256, 0, st>>>(U, n_users, n_comp, ld, fmt_stats);
-    operand_stats_kernel<<<sgrid, 256, 0, st>>>(V, n_items, n_comp, ld, fmt_stats + 4);
+    operand_stats_kernel<<<sgrid, 256, 0, st>>>(U, n_users, ld, fmt_stats);
+    operand_stats_kernel<<<sgrid, 256, 0, st>>>(V, n_items, ld, fmt_stats + 4);
   }
   pack_bf16_kernel<<<(unsigned)cdiv(L.nu_pad * 32, 256), 256, 0, st>>>(U, n_users, n_comp, ld, Ub, L.nu_pad, L.k_pad, nullptr, unorm, ures,
                                                                        nullptr, 0, fmt_stats, force_fmt);
@@ -1532,11 +1441,12 @@ static int score_topk_impl(const float* U, int64_t n_users, const float* V, int6
   q.U = U; q.V = V; q.erow = erow; q.prof = p.prof; q.cand = cand; q.cnt = cnt; q.thr = thr; q.ovf_count = ovfc; q.ovf_rows = ovfr;
   q.out_idx = out_idx; q.out_score = out_score;
 
-  const size_t smem = 1024 + (size_t)L.kb * A_SUB_BYTES + (size_t)NSTAGES * B_STAGE_BYTES + 256 +
-                      (size_t)BM * HSTRIDE * sizeof(uint32_t) + 16 + (size_t)BM * QCAP * 8 + 4 * 8 * sizeof(float);
-  auto main_kernel = L.wide ? (p.prof ? score_topk_kernel<false, true, true> : score_topk_kernel<false, false, true>)
-                            : dump != nullptr ? score_topk_kernel<true, false, false>
-                            : p.prof ? score_topk_kernel<false, true, false> : score_topk_kernel<false, false, false>;
+  const size_t smem = 1024 + topk_smem(L.kb).total;  // + room to align the base
+  auto main_kernel = L.wide ? score_topk_kernel<false, false, true>
+                            : dump != nullptr ? score_topk_kernel<true, false, false> : score_topk_kernel<false, false, false>;
+#ifdef TMF_DEVTOOLS
+  if (p.prof && dump == nullptr) main_kernel = L.wide ? score_topk_kernel<false, true, true> : score_topk_kernel<false, true, false>;
+#endif
   TMF_CUDA(cudaFuncSetAttribute(main_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int rr_warps = L.wide ? RR_WARPS_W : RR_WARPS;
   const size_t rr_smem = (size_t)rr_warps * (L.wide ? rerank_warp_smem<true>(ld) : rerank_warp_smem<false>(ld));
@@ -1560,6 +1470,7 @@ static int score_topk_impl(const float* U, int64_t n_users, const float* V, int6
   if (dump != nullptr) return TMF_OK;
   exact_rows_kernel<<<L.scratch_rows, 256, 0, st>>>(q, ovfc, ovfr, scratch);
   TMF_LAUNCH_CHECK();
+#ifdef TMF_DEVTOOLS
   if (p.prof) {  // profiling aid only: synchronises
     unsigned long long h[24]; int novf = 0;
     TMF_CUDA(cudaStreamSynchronize(st));
@@ -1568,10 +1479,11 @@ static int score_topk_impl(const float* U, int64_t n_users, const float* V, int6
     fprintf(stderr, "[tmf prof] producer wait empty %.3g, a_empty %.3g | mma wait tempty %.3g, full %.3g | epilogue (per warp-sweep, n=%llu) "
                     "wait tfull %.3g, work %.3g, init %.3g cycles | overflow rows %d (main %llu, rerank %llu) | tile-end drains: %llu, %.0f cycles each\n",
             (double)h[0], (double)h[1], (double)h[2], (double)h[3], h[7], (double)h[4] / h[7], (double)h[5] / h[7], (double)h[6] / h[7], novf, h[8], h[9], h[11], h[11] ? (double)h[10] / h[11] : 0.0);
-    fprintf(stderr, "[tmf prof] rebuilds: first %llu x %.0f cycles, saturated %llu x %.0f, generic %llu x %.0f | pre-rebuild drains %llu x %.0f | appended entries %.4g (%.1f per row-sweep)\n",
+    fprintf(stderr, "[tmf prof] rebuilds: first %llu x %.0f cycles, saturated %llu x %.0f, selected %llu x %.0f | pre-rebuild drains %llu x %.0f | appended entries %.4g (%.1f per row-sweep)\n",
             h[12], h[12] ? (double)h[13] / h[12] : 0.0, h[14], h[14] ? (double)h[15] / h[14] : 0.0, h[16], h[16] ? (double)h[17] / h[16] : 0.0,
             h[18], h[18] ? (double)h[19] / h[18] : 0.0, (double)h[20], h[7] ? (double)h[20] / (32.0 * h[7]) : 0.0);
   }
+#endif
   return TMF_OK;
 }
 
@@ -1586,12 +1498,6 @@ extern "C" int tmf_score_topk_bounded(const float* U, int64_t n_users, const flo
                                       float* out_score, void* ws, size_t ws_bytes, tmf_stream_t stream) {
   return score_topk_impl(U, n_users, V, n_items, n_comp, ld, k, clamp, item_offset, out_idx, out_score, ws, ws_bytes, stream, nullptr,
                          row_bound);
-}
-
-extern "C" int tmf_score_dense_bf16(const float* U, int64_t n_users, const float* V, int64_t n_items, int32_t n_comp, int32_t ld,
-                                    float* P, void* ws, size_t ws_bytes, tmf_stream_t stream) {
-  TMF_REQUIRE(P != nullptr, "tmf_score_dense_bf16: null output");
-  return score_topk_impl(U, n_users, V, n_items, n_comp, ld, 1, 0, 0, nullptr, nullptr, ws, ws_bytes, stream, P, nullptr, 0);
 }
 
 extern "C" int tmf_score_dense_tc(const float* U, int64_t n_users, const float* V, int64_t n_items, int32_t n_comp, int32_t ld,

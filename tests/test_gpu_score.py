@@ -209,10 +209,6 @@ def test_tensor_core_scores_within_stated_error_bound(n_u, n_i, r, fmt):
     ws_bytes = _abi.query("tmf_score_topk_ws_bytes", n_u, n_i, r, 1)
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device="cuda")
     _abi.call("tmf_score_dense_tc", _abi.ptr(Us), n_u, _abi.ptr(Vs), n_i, r, Us.shape[1], fmt, _abi.ptr(P), _abi.ptr(ws), ws_bytes)
-    if fmt == 0:  # the older entry point is the bf16 case
-        P0 = torch.full((n_u, n_i), float("nan"), device="cuda")
-        _abi.call("tmf_score_dense_bf16", _abi.ptr(Us), n_u, _abi.ptr(Vs), n_i, r, Us.shape[1], _abi.ptr(P0), _abi.ptr(ws), ws_bytes)
-        assert torch.equal(P, P0)
     torch.cuda.synchronize()
     got = cpu(P).astype(np.float64)
     exact = U.astype(np.float64) @ V.astype(np.float64).T
@@ -335,7 +331,8 @@ def _bounded_slabs(U, V, k, clamp, bounds, n_virtual, sample_frac=1.0):
 
 
 @pytest.mark.parametrize("clamp", [False, True])
-@pytest.mark.parametrize("sample_frac", [1.0, 0.3])
+# sample_frac 0.0125: each bound is the k-th best of only k items, so loose that bounded rows fill their lists
+@pytest.mark.parametrize("sample_frac", [1.0, 0.3, 0.0125])
 def test_bounded_item_slabs_merge_equals_single_shot(clamp, sample_frac):
     rng = np.random.default_rng(12)
     n_u, n_i, r, k = 700, 6000, 48, 25
