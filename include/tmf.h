@@ -135,15 +135,11 @@ TMF_API int tmf_user_pass_fixup(int32_t loss, int32_t n_split, const int32_t* sp
 TMF_API int tmf_pair_dots(int64_t nnz, const int32_t* rows, const int32_t* cols, const float* Eu, const float* Ei,
                   int32_t ld, float* p, tmf_stream_t stream);
 
-/* KL loss (loss_graphs.py:111-122): scalar loss_out[0] and d loss / d p[k] in coef_out[nnz]. ws >= tmf_reduce_ws_bytes(). */
-TMF_API int tmf_kl_coef(int64_t nnz, const float* p, const float* val, float* loss_out, float* coef_out, void* ws,
-                tmf_stream_t stream);
-
-/* The same loss under user sharding (SURVEY 8e): the two groups' moments (tf.nn.moments, loss_graphs.py:116,118) are
- * global, so each rank first reduces ITS interactions to six additive fp64 sums
- *     moments_out[6] = {n+, sum p+, sum p+^2, n-, sum p-, sum p-^2}          (tmf_kl_moments)
- * the host sums them over the ranks (one 48-byte all-reduce), and tmf_kl_coef_from_moments derives the global means /
- * variances, the scalar loss and this rank's d loss / d p[k].  ws >= tmf_reduce_ws_bytes() for both. */
+/* KL loss (loss_graphs.py:111-122) in two steps.  tmf_kl_moments reduces the interactions to six additive fp64 sums
+ *     moments_out[6] = {n+, sum p+, sum p+^2, n-, sum p-, sum p-^2}
+ * and tmf_kl_coef_from_moments derives from them the two groups' means / variances (tf.nn.moments, :116,118), the scalar
+ * loss_out[0] and d loss / d p[k] in coef_out[nnz].  Under user sharding (SURVEY 8e) the moments are global: the host sums
+ * each rank's six sums (one 48-byte all-reduce) between the two calls.  ws >= tmf_reduce_ws_bytes() for both. */
 TMF_API int tmf_kl_moments(int64_t nnz, const float* p, const float* val, double* moments_out, void* ws, tmf_stream_t stream);
 TMF_API int tmf_kl_coef_from_moments(int64_t nnz, const float* p, const float* val, const double* moments, float* loss_out,
                              float* coef_out, void* ws, tmf_stream_t stream);

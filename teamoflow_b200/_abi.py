@@ -37,7 +37,6 @@ SIGNATURES = {
                              _p, _p, _p, _p, _p]),
     "tmf_user_pass_fixup": (_i32, [_i32, _i32, _p, _p, _p, _p, _i32, _p, _i32, _i64, _p, _p, _p, _p, _p, _p]),
     "tmf_pair_dots": (_i32, [_i64, _p, _p, _p, _p, _i32, _p, _p]),
-    "tmf_kl_coef": (_i32, [_i64, _p, _p, _p, _p, _p, _p]),
     "tmf_kl_moments": (_i32, [_i64, _p, _p, _p, _p, _p]),
     "tmf_kl_coef_from_moments": (_i32, [_i64, _p, _p, _p, _p, _p, _p, _p]),
     "tmf_adam1": (_i32, [_p, _p, _i64, _f32, _p]),
@@ -81,7 +80,7 @@ _lib = None
 call_count = 0
 launch_count = 0
 # kernels per ABI call where it is not 1 (memsets are not counted)
-KERNELS_PER_CALL = {"tmf_spmm_seg": 2, "tmf_transpose_build": 3, "tmf_l2_normalize_global": 3, "tmf_kl_coef": 5, "tmf_kl_moments": 2, "tmf_kl_coef_from_moments": 2,
+KERNELS_PER_CALL = {"tmf_spmm_seg": 2, "tmf_transpose_build": 3, "tmf_l2_normalize_global": 3, "tmf_kl_moments": 2, "tmf_kl_coef_from_moments": 2,
                     "tmf_reduce_sum": 2, "tmf_gemm_tc": 4, "tmf_col_sum": 2, "tmf_rank_rows": 2, "tmf_score_topk": 8, "tmf_score_topk_bounded": 8}
 
 

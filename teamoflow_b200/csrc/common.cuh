@@ -35,6 +35,12 @@ inline int64_t cdiv(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
 constexpr int kNumSMs = 148;  // B200
 
+// blocks of a grid-stride launch that needs `blocks` to cover its range: at most per_sm resident per SM, the loop does the rest
+inline unsigned grid_stride_blocks(int64_t blocks, int per_sm) {
+  const int64_t cap = (int64_t)kNumSMs * per_sm;
+  return (unsigned)(blocks < cap ? blocks : cap);
+}
+
 // ---- sub-warp "row groups": LPR lanes (power of two) cooperate on one embedding row,
 //      each lane owning one float4 (128-bit) column slice.
 template <int LPR>

@@ -309,7 +309,7 @@ extern "C" int tmf_rank_rows(const float* P, int64_t n_rows, int64_t n_cols, int
   void* temp = offs + ((n_rows + 64) & ~63ll);
   size_t temp_bytes = seg_sort_temp_bytes(total, n_rows);
   cudaStream_t st = as_stream(stream);
-  rank_prep_kernel<<<(unsigned)std::min<long long>(cdiv(total, 256), 148 * 32), 256, 0, st>>>(P, n_rows, n_cols, clamp, keys, vals, offs);
+  rank_prep_kernel<<<grid_stride_blocks(cdiv(total, 256), 32), 256, 0, st>>>(P, n_rows, n_cols, clamp, keys, vals, offs);
   TMF_LAUNCH_CHECK();
   // stable LSD radix sort: equal keys keep ascending column order == tf.math.top_k tie order
   TMF_CUDA(cub::DeviceSegmentedRadixSort::SortPairsDescending(temp, temp_bytes, (const float*)keys, keys_out, (const int*)vals, out_idx,

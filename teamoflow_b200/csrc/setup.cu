@@ -161,7 +161,7 @@ extern "C" int tmf_coo_split(const void* indices, int32_t index_bytes, int64_t n
   cudaStream_t st = as_stream(stream);
   TMF_CUDA(cudaMemsetAsync(flags, 0, sizeof(int), st));
   if (nnz == 0) return TMF_OK;
-  const unsigned grid = (unsigned)std::min<long long>(cdiv(nnz, 256), 148 * 16);
+  const unsigned grid = grid_stride_blocks(cdiv(nnz, 256), 16);
   if (index_bytes == 8)
     coo_split_kernel<long long><<<grid, 256, 0, st>>>(reinterpret_cast<const long long*>(indices), nnz, n_rows, n_cols, rows, cols, flags);
   else
@@ -192,7 +192,7 @@ extern "C" int tmf_transpose_build(const int32_t* keys, int64_t n, int32_t n_key
   void* temp = iota + nn;
   size_t temp_bytes = ws_bytes - 2 * nn * sizeof(int);
   if (n > 0) {
-    iota_kernel<<<(unsigned)std::min<long long>(cdiv(n, 256), 148 * 16), 256, 0, st>>>(iota, n);
+    iota_kernel<<<grid_stride_blocks(cdiv(n, 256), 16), 256, 0, st>>>(iota, n);
     int end_bit = 1;
     while (end_bit < 31 && (1ll << end_bit) < (long long)n_keys) ++end_bit;
     TMF_CUDA(cub::DeviceRadixSort::SortPairs(temp, temp_bytes, keys, keys_out, (const int*)iota, perm, (int)n, 0, end_bit, st));
@@ -206,7 +206,7 @@ extern "C" int tmf_tlist_users(const int32_t* perm, int64_t n, int64_t nnz, cons
                                int32_t* users_out, tmf_stream_t stream) {
   if (n == 0) return TMF_OK;
   TMF_REQUIRE(n_samples > 0 || n <= nnz, "tmf_tlist_users: n_samples must be > 0 when the list holds samples");
-  tlist_users_kernel<<<(unsigned)std::min<long long>(cdiv(n, 256), 148 * 16), 256, 0, as_stream(stream)>>>(
+  tlist_users_kernel<<<grid_stride_blocks(cdiv(n, 256), 16), 256, 0, as_stream(stream)>>>(
       perm, n, nnz, coo_rows, n_samples > 0 ? n_samples : 1, users_out);
   TMF_LAUNCH_CHECK();
   return TMF_OK;
@@ -232,7 +232,7 @@ static int fill_common(int normal, float* w, int64_t n_rows, int32_t n_cols, int
   TMF_REQUIRE(w && n_rows >= 0 && n_cols >= 0 && n_cols <= ld, "tmf_fill: bad shape");
   const long long quads = cdiv(n_rows * n_cols, 4);
   if (quads == 0) return TMF_OK;
-  const unsigned grid = (unsigned)std::min<long long>(cdiv(quads, 256), 148 * 32);
+  const unsigned grid = grid_stride_blocks(cdiv(quads, 256), 32);
   if (normal) fill_kernel<1><<<grid, 256, 0, as_stream(stream)>>>(w, n_rows, n_cols, ld, seed);
   else fill_kernel<0><<<grid, 256, 0, as_stream(stream)>>>(w, n_rows, n_cols, ld, seed);
   TMF_LAUNCH_CHECK();

@@ -19,7 +19,7 @@ namespace tmf {
 // =====================================================================================
 
 struct UserPassParams {
-  int n_users, n_items, ld, n_comp, n_samples, s_pad;
+  int ld, n_samples, s_pad;
   long long nnz;
   const int* row_ptr;
   const int* col_idx;
@@ -42,6 +42,27 @@ struct UserPassParams {
   float* dEu;
   float scale;  // n_items / n_samples (python true division, loss_graphs.py:86)
 };
+
+// where coefficient slot e is stored: coef_pos[e] when a slot map is given, e otherwise
+__device__ __forceinline__ long long coef_slot(const int* coef_pos, long long e) { return coef_pos ? coef_pos[e] : e; }
+
+// sums over the lane groups whose lane ids differ in bits >= `from` (xor tree: fixed order => deterministic)
+__device__ __forceinline__ void xor_reduce(float2& a, int from) {
+#pragma unroll
+  for (int o = from; o < 32; o <<= 1) {
+    a.x += __shfl_xor_sync(0xffffffffu, a.x, o);
+    a.y += __shfl_xor_sync(0xffffffffu, a.y, o);
+  }
+}
+__device__ __forceinline__ void xor_reduce(float4& a, int from) {
+#pragma unroll
+  for (int o = from; o < 32; o <<= 1) {
+    a.x += __shfl_xor_sync(0xffffffffu, a.x, o);
+    a.y += __shfl_xor_sync(0xffffffffu, a.y, o);
+    a.z += __shfl_xor_sync(0xffffffffu, a.z, o);
+    a.w += __shfl_xor_sync(0xffffffffu, a.w, o);
+  }
+}
 
 template <int LPR, int VPL>
 __device__ __forceinline__ void load_row(const float* __restrict__ base, long long row, int ld, int nv, int lg,
@@ -94,6 +115,7 @@ __global__ void __launch_bounds__(kUserPassThreads, (JPL >= 0 && JPL <= 8 && VPL
 user_pass_kernel(const UserPassParams p) {
   constexpr int NT = kUserPassThreads;
   static_assert(NT == 32, "one warp per work item");
+  static_assert(JPL >= 0 || LPR == 32, "the generic WMRB path is only reached with 32 lanes per row");
   constexpr int NG = NT / LPR;
   constexpr int JH = JPL > 0 ? JPL / 2 : 1;
   constexpr int PD = (JPL >= 0 && JPL <= 4 && VPL == 1) ? 4 : 2;   // row buffers of the interaction loop
@@ -126,10 +148,7 @@ user_pass_kernel(const UserPassParams p) {
 
     if (a == b) {  // no interactions: all gradients of this user are zero
       if (LOSS == TMF_LOSS_WMRB)
-        for (int j = tid; j < S; j += NT) {
-          const long long e = p.nnz + (long long)u * S + j;
-          p.coef_out[p.coef_pos ? p.coef_pos[e] : e] = 0.f;
-        }
+        for (int j = tid; j < S; j += NT) p.coef_out[coef_slot(p.coef_pos, p.nnz + (long long)u * S + j)] = 0.f;
       for (int c = tid; c < ld; c += NT) p.dEu[(long long)u * ld + c] = 0.f;
       continue;
     }
@@ -298,7 +317,7 @@ user_pass_kernel(const UserPassParams p) {
       const int kc = min(k, b - 1);
       idx = p.col_idx[kc];
       a_k = p.val[kc];
-      pos = cpos ? cpos[kc] : kc;
+      pos = (int)coef_slot(cpos, kc);
     };
     {
       const int n_it = (b - a + NG - 1) / NG;
@@ -328,22 +347,21 @@ user_pass_kernel(const UserPassParams p) {
     if constexpr (LOSS == TMF_LOSS_WMRB) {
       __syncwarp();  // every lane's (1 + m) stores are visible to the warp; sS (sample scores) is no longer read
       for (int k = a + tid; k < b; k += NT) p.loss_out[k] = logf(p.loss_out[k]);  // log(1 + m), loss_graphs.py:88
+      // A whole user's G_uj is final and goes to its coefficient slot; a slice's is a partial sum, written to its part_G
+      // row and added up by the fix-up kernel.  sS keeps G for the sample term below.  (The JPL > 0 store stays split by
+      // destination: a single store through a selected pointer costs the 64-register variants extra spill bytes.)
       if constexpr (JPL > 0) {
-        // G_j = sum of the row groups' partial sums (xor tree over the groups: fixed order => deterministic)
+        // G_j = sum of the row groups' partial sums
 #pragma unroll
         for (int t = 0; t < JH; ++t) {
-#pragma unroll
-          for (int o = LPR; o < 32; o <<= 1) {
-            gj2[t].x += __shfl_xor_sync(FULL, gj2[t].x, o);
-            gj2[t].y += __shfl_xor_sync(FULL, gj2[t].y, o);
-          }
+          xor_reduce(gj2[t], LPR);
           if (g == 0) {
             const int j0 = lg + LPR * (2 * t), j1 = lg + LPR * (2 * t + 1);
-            if (slot < 0) {  // whole user: final G_uj (scattered to the item-major slot when coef_pos is given)
+            if (slot < 0) {
               const long long e0 = p.nnz + (long long)u * S;
-              if (j0 < S) { p.coef_out[cpos ? cpos[e0 + j0] : e0 + j0] = gj2[t].x; sS[j0] = gj2[t].x; }
-              if (j1 < S) { p.coef_out[cpos ? cpos[e0 + j1] : e0 + j1] = gj2[t].y; sS[j1] = gj2[t].y; }
-            } else {         // slice: partial sums, added up by the fix-up kernel
+              if (j0 < S) { p.coef_out[coef_slot(cpos, e0 + j0)] = gj2[t].x; sS[j0] = gj2[t].x; }
+              if (j1 < S) { p.coef_out[coef_slot(cpos, e0 + j1)] = gj2[t].y; sS[j1] = gj2[t].y; }
+            } else {
               float* dst = p.part_G + (long long)slot * p.s_pad;
               if (j0 < S) { dst[j0] = gj2[t].x; sS[j0] = gj2[t].x; }
               if (j1 < S) { dst[j1] = gj2[t].y; sS[j1] = gj2[t].y; }
@@ -354,10 +372,8 @@ user_pass_kernel(const UserPassParams p) {
         for (int j = tid; j < S; j += NT) {  // fixed group order => deterministic
           float G = sG[j];
           for (int gg = 1; gg < NG; ++gg) G += sG[gg * p.s_pad + j];
-          if (slot < 0) {
-            const long long e = p.nnz + (long long)u * S + j;
-            p.coef_out[cpos ? cpos[e] : e] = G;
-          } else p.part_G[(long long)slot * p.s_pad + j] = G;
+          if (slot < 0) p.coef_out[coef_slot(cpos, p.nnz + (long long)u * S + j)] = G;
+          else p.part_G[(long long)slot * p.s_pad + j] = G;
           sS[j] = G;
         }
       }
@@ -368,12 +384,7 @@ user_pass_kernel(const UserPassParams p) {
 #pragma unroll 4
         for (int j = (slot < 0 ? sg : S); j < S; j += NSG)
           fma4(accg, sS[j], __ldg(reinterpret_cast<const float4*>(ei_sub + (unsigned long long)(unsigned)su[j] * ld_bytes)));
-        for (int o = SW; o < 32; o <<= 1) {  // over the sub-groups (xor tree: fixed order)
-          accg.x += __shfl_xor_sync(FULL, accg.x, o);
-          accg.y += __shfl_xor_sync(FULL, accg.y, o);
-          accg.z += __shfl_xor_sync(FULL, accg.z, o);
-          accg.w += __shfl_xor_sync(FULL, accg.w, o);
-        }
+        xor_reduce(accg, SW);  // over the sub-groups
         if (g == 0 && lg < SW) add4(acc[0], accg);  // lane lg < SW owns column lg in both layouts
       } else {
 #pragma unroll 4
@@ -387,16 +398,10 @@ user_pass_kernel(const UserPassParams p) {
       }
     }
 
-    // ---- dE_u[u] = sum over the row groups (xor tree: fixed order)
+    // ---- dE_u[u] = sum over the row groups
 #pragma unroll
     for (int v = 0; v < VPL; ++v) {
-#pragma unroll
-      for (int o = LPR; o < 32; o <<= 1) {
-        acc[v].x += __shfl_xor_sync(FULL, acc[v].x, o);
-        acc[v].y += __shfl_xor_sync(FULL, acc[v].y, o);
-        acc[v].z += __shfl_xor_sync(FULL, acc[v].z, o);
-        acc[v].w += __shfl_xor_sync(FULL, acc[v].w, o);
-      }
+      xor_reduce(acc[v], LPR);
       const int col = lg + LPR * v;
       if (g == 0 && col < nv) {
         float* dst = slot < 0 ? p.dEu + (long long)u * ld : p.part_E + (long long)slot * ld;
@@ -426,8 +431,7 @@ __global__ void __launch_bounds__(256) user_fixup_kernel(const UserPassParams p,
       for (int j = tid; j < S; j += 256) {
         float G = 0.f;
         for (int sg = 0; sg < nseg; ++sg) G += p.part_G[(long long)(first + sg) * p.s_pad + j];
-        const long long e = p.nnz + (long long)u * S + j;
-        p.coef_out[p.coef_pos ? p.coef_pos[e] : e] = G;
+        p.coef_out[coef_slot(p.coef_pos, p.nnz + (long long)u * S + j)] = G;
         sG[j] = G;
       }
     }
@@ -486,7 +490,12 @@ static int dispatch_user_pass_j(const UserPassParams& p, int loss, cudaStream_t 
   if (jpl <= 4) return launch_user_pass<LPR, VPL, 4, TMF_LOSS_WMRB>(p, st);
   if (jpl <= 8) return launch_user_pass<LPR, VPL, 8, TMF_LOSS_WMRB>(p, st);
   if (jpl <= 16) return launch_user_pass<LPR, VPL, 16, TMF_LOSS_WMRB>(p, st);
-  return launch_user_pass<LPR, VPL, -1, TMF_LOSS_WMRB>(p, st);
+  // tmf_user_pass widens LPR to 32 before ceil(S / LPR) exceeds 16, so only LPR = 32 gets here and only that generic
+  // kernel is compiled
+  TMF_REQUIRE(LPR == 32, "tmf_user_pass: %d samples at %d lanes per row need a generic kernel that is not compiled",
+              p.n_samples, LPR);
+  if constexpr (LPR == 32) return launch_user_pass<LPR, VPL, -1, TMF_LOSS_WMRB>(p, st);
+  else return TMF_E_INVALID;
 }
 
 // =====================================================================================
@@ -507,6 +516,25 @@ struct SpmmParams {
   float* part_first;  // [n_chunks][ld_out]
   float* part_carry;  // [n_chunks][ld_out]
 };
+
+// acc += c * row for the NB entries t .. t + NB - 1 of the batch the group holds (lane t: index my_i, coefficient my_c):
+// NB row gathers in flight, summed in entry order
+template <int NB, int LPR>
+__device__ __forceinline__ void seg_batch(float4& acc, const float* src_lane, unsigned long long ld_src, unsigned gm, int my_i,
+                                          float my_c, int t) {
+  int i[NB];
+  float c[NB];
+  float4 r[NB];
+#pragma unroll
+  for (int q = 0; q < NB; ++q) {
+    i[q] = __shfl_sync(gm, my_i, t + q, LPR);
+    c[q] = __shfl_sync(gm, my_c, t + q, LPR);
+  }
+#pragma unroll
+  for (int q = 0; q < NB; ++q) r[q] = ldg4(src_lane + (unsigned long long)(unsigned)i[q] * ld_src);
+#pragma unroll
+  for (int q = 0; q < NB; ++q) fma4(acc, c[q], r[q]);
+}
 
 // group `gid` owns entries [gid*chunk, (gid+1)*chunk); walks the segments that intersect it.
 template <int LPR>
@@ -542,7 +570,7 @@ __global__ void __launch_bounds__(kSpmmThreads) spmm_seg_kernel(const SpmmParams
     my_c = 0.f;
     if (e < ce) {
       my_i = p.idx[e];
-      my_c = p.coef ? p.coef[p.cpos ? p.cpos[e] : e] : 1.0f;
+      my_c = p.coef ? p.coef[coef_slot(p.cpos, e)] : 1.0f;
     }
   };
   int nxt_i;
@@ -557,40 +585,12 @@ __global__ void __launch_bounds__(kSpmmThreads) spmm_seg_kernel(const SpmmParams
     int t = 0;
     while (t < nb) {
       const int te = (int)min((long long)nb, sb - base);  // entries of this batch that belong to segment s
-      for (; t + 8 <= te; t += 8) {
-        int i[8];
-        float c[8];
-        float4 r[8];
-#pragma unroll
-        for (int q = 0; q < 8; ++q) {
-          i[q] = __shfl_sync(gm, my_i, t + q, LPR);
-          c[q] = __shfl_sync(gm, my_c, t + q, LPR);
-        }
-#pragma unroll
-        for (int q = 0; q < 8; ++q) r[q] = ldg4(src_lane + (unsigned long long)(unsigned)i[q] * ld_src);
-#pragma unroll
-        for (int q = 0; q < 8; ++q) fma4(acc, c[q], r[q]);
-      }
+      for (; t + 8 <= te; t += 8) seg_batch<8, LPR>(acc, src_lane, ld_src, gm, my_i, my_c, t);
       if (t + 4 <= te) {
-        int i[4];
-        float c[4];
-        float4 r[4];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          i[q] = __shfl_sync(gm, my_i, t + q, LPR);
-          c[q] = __shfl_sync(gm, my_c, t + q, LPR);
-        }
-#pragma unroll
-        for (int q = 0; q < 4; ++q) r[q] = ldg4(src_lane + (unsigned long long)(unsigned)i[q] * ld_src);
-#pragma unroll
-        for (int q = 0; q < 4; ++q) fma4(acc, c[q], r[q]);
+        seg_batch<4, LPR>(acc, src_lane, ld_src, gm, my_i, my_c, t);
         t += 4;
       }
-      for (; t < te; ++t) {
-        const int i0 = __shfl_sync(gm, my_i, t, LPR);
-        const float c0 = __shfl_sync(gm, my_c, t, LPR);
-        fma4(acc, c0, ldg4(src_lane + (unsigned long long)(unsigned)i0 * ld_src));
-      }
+      for (; t < te; ++t) seg_batch<1, LPR>(acc, src_lane, ld_src, gm, my_i, my_c, t);
       if (base + t == sb || base + t == ce) {  // segment (or this chunk's part of it) complete
         if (active) {
           float* dst;
@@ -737,15 +737,20 @@ __device__ __forceinline__ void block_reduce_store(double (&v)[NV], double* out)
   }
 }
 
-// MODE 0: sum(x)            MODE 1: sum(x^2)
-// MODE 2: KL first moments  {cnt+, sum+, cnt-, sum-}
-// MODE 3: KL second moments {ssd+, ssd-} around stats[0]=mu+, stats[1]=mu-
-// MODE 4: KL raw moments    {cnt+, sum+, sumsq+, cnt-, sum-, sumsq-}  (additive over user shards: data-parallel KL)
+// Reduction modes and the number of fp64 sums each one produces per block:
+//   kRedSum: sum(x)    kRedSumSq: sum(x^2)
+//   kRedKLMoments: KL raw moments {cnt+, sum+, sumsq+, cnt-, sum-, sumsq-}, additive over user shards
+enum RedMode { kRedSum, kRedSumSq, kRedKLMoments };
+template <int MODE>
+constexpr int kRedWidth = MODE == kRedKLMoments ? 6 : 1;
+constexpr int kRedMaxWidth = std::max({kRedWidth<kRedSum>, kRedWidth<kRedSumSq>, kRedWidth<kRedKLMoments>});
+// reduce workspace: kRedStats doubles of statistics, then up to kRedBlocks partial rows of the widest mode
+constexpr int kRedStats = 16;
+
 template <int MODE>
 __global__ void __launch_bounds__(kRedThreads) reduce_partial_kernel(const float* __restrict__ x, const float* __restrict__ val,
-                                                                    long long n, const double* __restrict__ stats,
-                                                                    double* __restrict__ partial) {
-  constexpr int NV = MODE == 2 ? 4 : (MODE == 3 ? 2 : (MODE == 4 ? 6 : 1));
+                                                                    long long n, double* __restrict__ partial) {
+  constexpr int NV = kRedWidth<MODE>;
   double v[NV];
 #pragma unroll
   for (int i = 0; i < NV; ++i) v[i] = 0.0;
@@ -753,68 +758,43 @@ __global__ void __launch_bounds__(kRedThreads) reduce_partial_kernel(const float
   const long long lo = per * blockIdx.x, hi = min(lo + per, n);
   for (long long i = lo + threadIdx.x; i < hi; i += kRedThreads) {
     const double xi = x[i];
-    if (MODE == 0) v[0] += xi;
-    if (MODE == 1) v[0] += xi * xi;
-    if (MODE == 2) {
-      if (val[i] > 0.f) { v[0] += 1.0; v[1] += xi; } else { v[2] += 1.0; v[3] += xi; }
-    }
-    if (MODE == 3) {
-      if (val[i] > 0.f) { const double d = xi - stats[0]; v[0] += d * d; } else { const double d = xi - stats[1]; v[1] += d * d; }
-    }
-    if (MODE == 4) {
+    if (MODE == kRedSum) v[0] += xi;
+    if (MODE == kRedSumSq) v[0] += xi * xi;
+    if (MODE == kRedKLMoments) {
       if (val[i] > 0.f) { v[0] += 1.0; v[1] += xi; v[2] += xi * xi; } else { v[3] += 1.0; v[4] += xi; v[5] += xi * xi; }
     }
   }
   block_reduce_store<NV>(v, partial + (long long)blockIdx.x * NV);
 }
 
-// FIN 0: out_f[0] = sum                      FIN 1: scale = rsqrt(max(sum, 1e-12)) -> stats[0]
-// FIN 2: KL means -> stats[0..3] = {mu+, mu-, n+, n-}
-// FIN 3: KL finish: stats[4..] = {s, z, phi}; out_f[0] = loss
-// FIN 4: KL raw moments -> stats[0..5] (the six sums, nothing derived)
-template <int FIN>
+// kRedSum: out_f[0] = sum    kRedSumSq: scale = rsqrt(max(sum, 1e-12)) -> stats[0]
+// kRedKLMoments: the six sums -> stats[0..5], nothing derived
+template <int MODE>
 __global__ void __launch_bounds__(kRedThreads) reduce_final_kernel(const double* __restrict__ partial, int n_blocks,
                                                                   double* __restrict__ stats, float* __restrict__ out_f) {
-  constexpr int NV = FIN == 2 ? 4 : (FIN == 3 ? 2 : (FIN == 4 ? 6 : 1));
+  constexpr int NV = kRedWidth<MODE>;
   double v[NV];
 #pragma unroll
   for (int i = 0; i < NV; ++i) v[i] = 0.0;
   for (int b = threadIdx.x; b < n_blocks; b += kRedThreads)
 #pragma unroll
     for (int i = 0; i < NV; ++i) v[i] += partial[(long long)b * NV + i];
-  __shared__ double res[6];
+  __shared__ double res[NV];
   block_reduce_store<NV>(v, res);
   __syncthreads();
   if (threadIdx.x == 0) {
-    if (FIN == 0) out_f[0] = (float)res[0];
-    if (FIN == 1) stats[0] = 1.0 / sqrt(fmax(res[0], 1e-12));
-    if (FIN == 2) {
-      stats[0] = (double)(float)(res[1] / res[0]);  // mu+ rounded to fp32 like tf.nn.moments
-      stats[1] = (double)(float)(res[3] / res[2]);
-      stats[2] = res[0];
-      stats[3] = res[2];
-    }
-    if (FIN == 4) {
+    if (MODE == kRedSum) out_f[0] = (float)res[0];
+    if (MODE == kRedSumSq) stats[0] = 1.0 / sqrt(fmax(res[0], 1e-12));
+    if (MODE == kRedKLMoments) {
 #pragma unroll
       for (int i = 0; i < NV; ++i) stats[i] = res[i];
-    }
-    if (FIN == 3) {
-      const float vp = (float)(res[0] / stats[2]);  // population variance
-      const float vn = (float)(res[1] / stats[3]);
-      const float s = sqrtf(vp + vn);
-      const float z = ((float)stats[0] - (float)stats[1]) / s;
-      const float phi = expf(-0.5f * z * z) * 0.3989422804014327f;
-      stats[4] = s;
-      stats[5] = z;
-      stats[6] = phi;
-      out_f[0] = 1.0f - 0.5f * erfcf(-z * 0.7071067811865476f);  // 1 - ndtr(z), loss_graphs.py:120-122
     }
   }
 }
 
-// Global KL statistics from the six (summed-over-ranks) raw moments m = {n+, S+, Q+, n-, S-, Q-}: means rounded to fp32
-// like tf.nn.moments, population variances about those means (Q - 2 mu S + n mu^2, fp64), then s, z, phi and the loss
-// exactly as FIN 3 derives them on one GPU.
+// KL statistics from the six raw moments m = {n+, S+, Q+, n-, S-, Q-} (summed over the ranks under user sharding): means
+// rounded to fp32 like tf.nn.moments, population variances about those means (Q - 2 mu S + n mu^2, fp64), s, z, phi and
+// the scalar loss.
 __global__ void kl_from_moments_kernel(const double* __restrict__ m, double* __restrict__ stats, float* __restrict__ out_f) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
   const double np_ = m[0], nn_ = m[3];
@@ -826,7 +806,7 @@ __global__ void kl_from_moments_kernel(const double* __restrict__ m, double* __r
   const float phi = expf(-0.5f * z * z) * 0.3989422804014327f;
   stats[0] = mp; stats[1] = mn; stats[2] = np_; stats[3] = nn_;
   stats[4] = s; stats[5] = z; stats[6] = phi;
-  out_f[0] = 1.0f - 0.5f * erfcf(-z * 0.7071067811865476f);
+  out_f[0] = 1.0f - 0.5f * erfcf(-z * 0.7071067811865476f);  // 1 - ndtr(z), loss_graphs.py:120-122
 }
 
 __global__ void kl_coef_kernel(long long nnz, const float* __restrict__ p, const float* __restrict__ val,
@@ -979,7 +959,7 @@ extern "C" int tmf_user_pass(int32_t loss, int32_t n_users, int32_t n_items, int
   if (loss == TMF_LOSS_WMRB) TMF_REQUIRE(samp && n_samples > 0, "tmf_user_pass: WMRB needs samples (random_ind)");
   if (n_users == 0) return TMF_OK;
   UserPassParams p{};
-  p.n_users = n_users; p.n_items = n_items; p.ld = ld; p.n_comp = n_comp;
+  p.ld = ld;
   p.n_samples = loss == TMF_LOSS_WMRB ? n_samples : 0;
   p.s_pad = (p.n_samples + 3) & ~3;
   p.row_ptr = row_ptr; p.col_idx = col_idx; p.val = val; p.Eu = Eu; p.Ei = Ei; p.samp = samp;
@@ -1039,17 +1019,18 @@ extern "C" int tmf_pair_dots(int64_t nnz, const int32_t* rows, const int32_t* co
   return TMF_OK;
 }
 
-extern "C" size_t tmf_reduce_ws_bytes(void) { return (size_t)(kRedBlocks * 4 + 16) * sizeof(double); }
+extern "C" size_t tmf_reduce_ws_bytes(void) { return (size_t)(kRedBlocks * kRedMaxWidth + kRedStats) * sizeof(double); }
 
 static int red_blocks(long long n) { return (int)std::max<long long>(1, std::min<long long>(kRedBlocks, cdiv(n, 4096))); }
 
 extern "C" int tmf_reduce_sum(const float* x, int64_t n, float* out, void* ws, tmf_stream_t stream) {
   TMF_REQUIRE(ws && out, "tmf_reduce_sum: null");
-  double* partial = reinterpret_cast<double*>(ws) + 16;
+  double* stats = reinterpret_cast<double*>(ws);
+  double* partial = stats + kRedStats;
   const int nb = red_blocks(n);
   cudaStream_t st = as_stream(stream);
-  reduce_partial_kernel<0><<<nb, kRedThreads, 0, st>>>(x, nullptr, n, nullptr, partial);
-  reduce_final_kernel<0><<<1, kRedThreads, 0, st>>>(partial, nb, reinterpret_cast<double*>(ws), out);
+  reduce_partial_kernel<kRedSum><<<nb, kRedThreads, 0, st>>>(x, nullptr, n, partial);
+  reduce_final_kernel<kRedSum><<<1, kRedThreads, 0, st>>>(partial, nb, stats, out);
   TMF_LAUNCH_CHECK();
   return TMF_OK;
 }
@@ -1057,39 +1038,23 @@ extern "C" int tmf_reduce_sum(const float* x, int64_t n, float* out, void* ws, t
 extern "C" int tmf_l2_normalize_global(float* w, int64_t n, void* ws, tmf_stream_t stream) {
   TMF_REQUIRE(ws && w, "tmf_l2_normalize_global: null");
   double* stats = reinterpret_cast<double*>(ws);
-  double* partial = stats + 16;
+  double* partial = stats + kRedStats;
   const int nb = red_blocks(n);
   cudaStream_t st = as_stream(stream);
-  reduce_partial_kernel<1><<<nb, kRedThreads, 0, st>>>(w, nullptr, n, nullptr, partial);
-  reduce_final_kernel<1><<<1, kRedThreads, 0, st>>>(partial, nb, stats, nullptr);
-  scale_kernel<<<(unsigned)std::min<long long>(cdiv(n, 256), 148 * 16), 256, 0, st>>>(w, n, stats);
-  TMF_LAUNCH_CHECK();
-  return TMF_OK;
-}
-
-extern "C" int tmf_kl_coef(int64_t nnz, const float* p, const float* val, float* loss_out, float* coef_out, void* ws,
-                           tmf_stream_t stream) {
-  TMF_REQUIRE(ws && p && val && loss_out && coef_out, "tmf_kl_coef: null");
-  double* stats = reinterpret_cast<double*>(ws);
-  double* partial = stats + 16;
-  const int nb = red_blocks(nnz);
-  cudaStream_t st = as_stream(stream);
-  reduce_partial_kernel<2><<<nb, kRedThreads, 0, st>>>(p, val, nnz, nullptr, partial);
-  reduce_final_kernel<2><<<1, kRedThreads, 0, st>>>(partial, nb, stats, nullptr);
-  reduce_partial_kernel<3><<<nb, kRedThreads, 0, st>>>(p, val, nnz, stats, partial);
-  reduce_final_kernel<3><<<1, kRedThreads, 0, st>>>(partial, nb, stats, loss_out);
-  if (nnz > 0) kl_coef_kernel<<<(unsigned)cdiv(nnz, 256), 256, 0, st>>>(nnz, p, val, stats, coef_out);
+  reduce_partial_kernel<kRedSumSq><<<nb, kRedThreads, 0, st>>>(w, nullptr, n, partial);
+  reduce_final_kernel<kRedSumSq><<<1, kRedThreads, 0, st>>>(partial, nb, stats, nullptr);
+  scale_kernel<<<grid_stride_blocks(cdiv(n, 256), 16), 256, 0, st>>>(w, n, stats);
   TMF_LAUNCH_CHECK();
   return TMF_OK;
 }
 
 extern "C" int tmf_kl_moments(int64_t nnz, const float* p, const float* val, double* moments_out, void* ws, tmf_stream_t stream) {
   TMF_REQUIRE(ws && moments_out && (nnz == 0 || (p && val)), "tmf_kl_moments: null");
-  double* partial = reinterpret_cast<double*>(ws) + 16;
+  double* partial = reinterpret_cast<double*>(ws) + kRedStats;
   const int nb = red_blocks(nnz);
   cudaStream_t st = as_stream(stream);
-  reduce_partial_kernel<4><<<nb, kRedThreads, 0, st>>>(p, val, nnz, nullptr, partial);
-  reduce_final_kernel<4><<<1, kRedThreads, 0, st>>>(partial, nb, moments_out, nullptr);
+  reduce_partial_kernel<kRedKLMoments><<<nb, kRedThreads, 0, st>>>(p, val, nnz, partial);
+  reduce_final_kernel<kRedKLMoments><<<1, kRedThreads, 0, st>>>(partial, nb, moments_out, nullptr);
   TMF_LAUNCH_CHECK();
   return TMF_OK;
 }
@@ -1108,7 +1073,7 @@ extern "C" int tmf_kl_coef_from_moments(int64_t nnz, const float* p, const float
 extern "C" int tmf_adam1(float* w, const float* g, int64_t n, float lr, tmf_stream_t stream) {
   if (n == 0) return TMF_OK;
   const int vec = aligned16(w) && aligned16(g);  // views at odd offsets take the scalar path
-  adam1_kernel<<<(unsigned)std::min<long long>(cdiv(cdiv(n, vec ? 4 : 1), 256), 148 * 16), 256, 0, as_stream(stream)>>>(w, g, n, lr, vec);
+  adam1_kernel<<<grid_stride_blocks(cdiv(cdiv(n, vec ? 4 : 1), 256), 16), 256, 0, as_stream(stream)>>>(w, g, n, lr, vec);
   TMF_LAUNCH_CHECK();
   return TMF_OK;
 }
@@ -1117,7 +1082,7 @@ extern "C" int tmf_adam(float* w, const float* g, float* m, float* v, int64_t n,
   TMF_REQUIRE(step >= 1, "tmf_adam: step counts from 1");
   if (n == 0) return TMF_OK;
   const float alpha = lr * sqrtf(1.0f - powf(0.999f, (float)step)) / (1.0f - powf(0.9f, (float)step));
-  adam_kernel<<<(unsigned)std::min<long long>(cdiv(n, 256), 148 * 32), 256, 0, as_stream(stream)>>>(w, g, m, v, n, alpha);
+  adam_kernel<<<grid_stride_blocks(cdiv(n, 256), 32), 256, 0, as_stream(stream)>>>(w, g, m, v, n, alpha);
   TMF_LAUNCH_CHECK();
   return TMF_OK;
 }
@@ -1125,7 +1090,7 @@ extern "C" int tmf_adam(float* w, const float* g, float* m, float* v, int64_t n,
 extern "C" int tmf_bias_add(float* E, int64_t n_rows, int32_t n_cols, int32_t ld, const float* bias, int32_t relu,
                             tmf_stream_t stream) {
   if (n_rows == 0) return TMF_OK;
-  bias_add_kernel<<<(unsigned)std::min<long long>(cdiv(n_rows * ld, 256), 148 * 32), 256, 0, as_stream(stream)>>>(
+  bias_add_kernel<<<grid_stride_blocks(cdiv(n_rows * ld, 256), 32), 256, 0, as_stream(stream)>>>(
       E, n_rows, n_cols, ld, bias, relu);
   TMF_LAUNCH_CHECK();
   return TMF_OK;
@@ -1133,7 +1098,7 @@ extern "C" int tmf_bias_add(float* E, int64_t n_rows, int32_t n_cols, int32_t ld
 
 extern "C" int tmf_relu_mask(float* dH, const float* H, int64_t n, tmf_stream_t stream) {
   if (n == 0) return TMF_OK;
-  relu_mask_kernel<<<(unsigned)std::min<long long>(cdiv(n, 256), 148 * 32), 256, 0, as_stream(stream)>>>(dH, H, n);
+  relu_mask_kernel<<<grid_stride_blocks(cdiv(n, 256), 32), 256, 0, as_stream(stream)>>>(dH, H, n);
   TMF_LAUNCH_CHECK();
   return TMF_OK;
 }
@@ -1201,7 +1166,7 @@ extern "C" int tmf_user_pass_fixup(int32_t loss, int32_t n_split, const int32_t*
   p.coef_out = coef_out; p.coef_pos = coef_pos; p.dEu = dEu;
   const size_t smem = (size_t)(p.s_pad + ld + 1024) * sizeof(float);  // (256 / nvp) partial rows of ld floats <= 1024 floats
   TMF_REQUIRE(smem <= 48 * 1024 && ld <= 256, "tmf_user_pass_fixup: n_samples too large");
-  user_fixup_kernel<<<std::min(n_split, 148 * 4), 256, smem, as_stream(stream)>>>(p, loss, n_split, split_user, split_first, split_nseg);
+  user_fixup_kernel<<<grid_stride_blocks(n_split, 4), 256, smem, as_stream(stream)>>>(p, loss, n_split, split_user, split_first, split_nseg);
   TMF_LAUNCH_CHECK();
   return TMF_OK;
 }

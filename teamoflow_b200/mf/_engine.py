@@ -223,13 +223,13 @@ class InteractionPlan:
         self.samp = None
         self.t_user = None
         self.comm = None        # set by TrainPlan under user sharding (KL needs the global moments)
-        self.kl_moments = None
         self.set_samples(random_ind)
         self._build_work_list()
         self.counter = torch.zeros(1, dtype=torch.int32, device=dev)
         self.coef = torch.zeros(max(self.nnz + self.n_users * self.S, 1), dtype=torch.float32, device=dev)
         self.loss_k = torch.zeros(max(self.nnz, 1), dtype=torch.float32, device=dev)
         self.p = torch.zeros(max(self.nnz, 1), dtype=torch.float32, device=dev) if loss == KL else None
+        self.kl_moments = torch.zeros(6, dtype=torch.float64, device=dev) if loss == KL else None
         self.kl_loss = torch.zeros(1, dtype=torch.float32, device=dev)
         self.red_ws = reduce_ws()
         self.red_out = torch.zeros(1, dtype=torch.float32, device=dev)
@@ -338,17 +338,12 @@ class InteractionPlan:
         else:
             _abi.call("tmf_pair_dots", self.nnz, _abi.ptr(self.coo_rows), _abi.ptr(self.col_idx), _abi.ptr(Eu),
                       _abi.ptr(Ei), Eu.shape[1], _abi.ptr(self.p))
-            if self.comm is None:
-                _abi.call("tmf_kl_coef", self.nnz, _abi.ptr(self.p), _abi.ptr(self.vals), _abi.ptr(self.kl_loss),
-                          _abi.ptr(self.coef), _abi.ptr(self.red_ws))
-            else:  # user-sharded: the two groups' moments are global (loss_graphs.py:116,118) -> one 48-byte all-reduce
-                if self.kl_moments is None:
-                    self.kl_moments = torch.zeros(6, dtype=torch.float64, device=self.vals.device)
-                _abi.call("tmf_kl_moments", self.nnz, _abi.ptr(self.p), _abi.ptr(self.vals), _abi.ptr(self.kl_moments),
-                          _abi.ptr(self.red_ws))
+            _abi.call("tmf_kl_moments", self.nnz, _abi.ptr(self.p), _abi.ptr(self.vals), _abi.ptr(self.kl_moments),
+                      _abi.ptr(self.red_ws))
+            if self.comm is not None:  # user-sharded: the two groups' moments are global (loss_graphs.py:116,118)
                 self.comm.allreduce_kl_moments(self.kl_moments)
-                _abi.call("tmf_kl_coef_from_moments", self.nnz, _abi.ptr(self.p), _abi.ptr(self.vals), _abi.ptr(self.kl_moments),
-                          _abi.ptr(self.kl_loss), _abi.ptr(self.coef), _abi.ptr(self.red_ws))
+            _abi.call("tmf_kl_coef_from_moments", self.nnz, _abi.ptr(self.p), _abi.ptr(self.vals), _abi.ptr(self.kl_moments),
+                      _abi.ptr(self.kl_loss), _abi.ptr(self.coef), _abi.ptr(self.red_ws))
             self.spmm_ws = self._spmm_ws(dEu.shape[1])
             spmm(self.n_users, self.row_ptr, self.nnz, self.col_idx, None, self.coef, Ei, r, out=dEu, ws=self.spmm_ws)
 

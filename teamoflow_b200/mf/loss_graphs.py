@@ -2,8 +2,9 @@
 
 ``get_loss`` keeps the reference's argument names and returns the same tensors (forward only --
 there is no autodiff here).  During ``MatrixFactorization.fit`` the classes are descriptors: the
-loss, its gradient and the embedding gradients come out of the fused kernels (``tmf_user_pass``,
-``tmf_kl_coef``) and the dense ``predictions`` matrix these signatures expect is never formed.
+loss, its gradient and the embedding gradients come out of the fused kernels (``tmf_user_pass``;
+``tmf_kl_moments`` then ``tmf_kl_coef_from_moments`` for KL) and the dense ``predictions`` matrix these
+signatures expect is never formed.
 """
 from abc import ABC, abstractmethod
 
@@ -65,6 +66,9 @@ class KLDivergenceLoss(LossGraph):
         serial = to_device(tf_prediction_serial, torch.float32).reshape(-1)
         loss = torch.empty(1, dtype=torch.float32, device=serial.device)
         coef = torch.empty(max(serial.numel(), 1), dtype=torch.float32, device=serial.device)
-        _abi.call("tmf_kl_coef", serial.numel(), _abi.ptr(serial), _abi.ptr(inter.values), _abi.ptr(loss), _abi.ptr(coef),
-                  _abi.ptr(reduce_ws()))
+        moments = torch.empty(6, dtype=torch.float64, device=serial.device)
+        ws = reduce_ws()
+        _abi.call("tmf_kl_moments", serial.numel(), _abi.ptr(serial), _abi.ptr(inter.values), _abi.ptr(moments), _abi.ptr(ws))
+        _abi.call("tmf_kl_coef_from_moments", serial.numel(), _abi.ptr(serial), _abi.ptr(inter.values), _abi.ptr(moments),
+                  _abi.ptr(loss), _abi.ptr(coef), _abi.ptr(ws))
         return loss.reshape(())

@@ -127,32 +127,62 @@ def test_minibatch_mode_matches_oracle_per_block():
         assert (np.abs(got - ref) < 1e-4 * max(np.abs(ref).max(), 1.0)).mean() > 0.97, loss
 
 
-def test_kl_moments_path_equals_single_gpu_kl():
-    """The data-parallel KL entry points (raw additive moments -> global statistics) reproduce tmf_kl_coef."""
+def _kl_from_moments(shards, p, val, ws):
+    """KL loss and coefficients with the interactions split into ``shards`` (ranks): each shard's six moments, summed on
+    the host side of the ABI, then each shard's coefficients from the global moments."""
+    from teamoflow_b200 import _abi
+    n = p.numel()
+    mom = torch.zeros(len(shards), 6, dtype=torch.float64, device="cuda")
+    for g, (a, b) in enumerate(shards):
+        _abi.call("tmf_kl_moments", b - a, _abi.ptr(p[a:b]), _abi.ptr(val[a:b]), _abi.ptr(mom[g]), _abi.ptr(ws))
+    tot = mom.sum(0).contiguous()
+    loss, coef = torch.zeros(1, device="cuda"), torch.zeros(n, device="cuda")
+    for a, b in shards:
+        _abi.call("tmf_kl_coef_from_moments", b - a, _abi.ptr(p[a:b]), _abi.ptr(val[a:b]), _abi.ptr(tot), _abi.ptr(loss),
+                  _abi.ptr(coef[a:b]), _abi.ptr(ws))
+    torch.cuda.synchronize()
+    return cpu(loss), cpu(coef)
+
+
+def test_kl_moments_summed_over_shards_equal_one_shard():
+    """Two ranks' moments summed give the KL loss and coefficients of one rank holding every interaction."""
     from teamoflow_b200 import _abi
     rng = np.random.default_rng(3)
     n = 5000
     p = torch.as_tensor(rng.standard_normal(n).astype(np.float32) * 0.3 + 0.1, device="cuda")
     val = torch.as_tensor(rng.choice([-1.0, 1.0, 2.0], n).astype(np.float32), device="cuda")
     ws = torch.empty(_abi.query("tmf_reduce_ws_bytes"), dtype=torch.uint8, device="cuda")
-    l1, c1 = torch.zeros(1, device="cuda"), torch.zeros(n, device="cuda")
-    _abi.call("tmf_kl_coef", n, _abi.ptr(p), _abi.ptr(val), _abi.ptr(l1), _abi.ptr(c1), _abi.ptr(ws))
-    # two "ranks": moments of each half, summed on the host side of the ABI, then the coefficients of each half
-    mom = torch.zeros(2, 6, dtype=torch.float64, device="cuda")
+    l1, c1 = _kl_from_moments(((0, n),), p, val, ws)
     h = n // 3
-    for g, (a, b) in enumerate(((0, h), (h, n))):
-        _abi.call("tmf_kl_moments", b - a, _abi.ptr(p[a:b]), _abi.ptr(val[a:b]), _abi.ptr(mom[g]), _abi.ptr(ws))
-    tot = mom.sum(0).contiguous()
-    l2, c2 = torch.zeros(1, device="cuda"), torch.zeros(n, device="cuda")
-    for a, b in ((0, h), (h, n)):
-        _abi.call("tmf_kl_coef_from_moments", b - a, _abi.ptr(p[a:b]), _abi.ptr(val[a:b]), _abi.ptr(tot), _abi.ptr(l2), _abi.ptr(c2[a:b]),
-                  _abi.ptr(ws))
-    torch.cuda.synchronize()
-    np.testing.assert_allclose(cpu(l2), cpu(l1), rtol=1e-6)
-    np.testing.assert_allclose(cpu(c2), cpu(c1), rtol=2e-5, atol=1e-9)
+    l2, c2 = _kl_from_moments(((0, h), (h, n)), p, val, ws)
+    np.testing.assert_allclose(l2, l1, rtol=1e-6)
+    np.testing.assert_allclose(c2, c1, rtol=2e-5, atol=1e-9)
     want_loss, want_c = o.kl_loss(cpu(p).astype(np.float64), cpu(val)), o.kl_coef(cpu(val), cpu(p).astype(np.float64))
-    np.testing.assert_allclose(cpu(l2)[0], float(want_loss), rtol=1e-5)
-    close(cpu(c2), want_c, name="kl coef from moments")
+    np.testing.assert_allclose(l2[0], float(want_loss), rtol=1e-5)
+    close(c2, want_c, name="kl coef from moments")
+
+
+def test_kl_moments_stay_inside_the_reduce_workspace():
+    """tmf_reduce_ws_bytes() covers the widest reduction: 4M interactions take 977 blocks of six partial sums each, which
+    must all land inside the workspace (a canary right after it stays intact) and add up to the float64 host sums."""
+    from teamoflow_b200 import _abi
+    rng = np.random.default_rng(11)
+    n = 4_000_000
+    p_h = (rng.standard_normal(n) * 0.5 + 0.25).astype(np.float32)
+    val_h = rng.choice([-1.0, 0.0, 1.0, 3.0], n).astype(np.float32)
+    p, val = torch.as_tensor(p_h, device="cuda"), torch.as_tensor(val_h, device="cuda")
+    ws_bytes, tail = _abi.query("tmf_reduce_ws_bytes"), 4096
+    buf = torch.zeros(ws_bytes + tail, dtype=torch.uint8, device="cuda")
+    buf[ws_bytes:] = 0xA5
+    mom = torch.zeros(6, dtype=torch.float64, device="cuda")
+    _abi.call("tmf_kl_moments", n, _abi.ptr(p), _abi.ptr(val), _abi.ptr(mom), _abi.ptr(buf))
+    torch.cuda.synchronize()
+    assert bool((buf[ws_bytes:] == 0xA5).all()), "tmf_kl_moments wrote past tmf_reduce_ws_bytes()"
+    x, pos = p_h.astype(np.float64), val_h > 0
+    want = [pos.sum(), x[pos].sum(), (x[pos] ** 2).sum(), (~pos).sum(), x[~pos].sum(), (x[~pos] ** 2).sum()]
+    got = cpu(mom)
+    assert got[0] == want[0] and got[3] == want[3]
+    np.testing.assert_allclose(got, want, rtol=1e-11)
 
 
 def test_predict_with_sparse_A_and_predict_ranks_without_densifying():
