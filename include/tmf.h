@@ -198,6 +198,18 @@ TMF_API int tmf_score_topk_bounded(const float* U, int64_t n_users, const float*
                            int32_t k, int32_t clamp, int32_t item_offset, const float* row_bound, int32_t* out_idx,
                            float* out_score, void* ws, size_t ws_bytes, tmf_stream_t stream);
 
+/* Top-k over each row's UNSEEN items (SURVEY 8f-3: "the best k items this user has not interacted with"; the reference
+ * ranks seen items too).  ex_ptr[n_users + 1] / ex_idx form a CSR of GLOBAL item ids to exclude, each row sorted ascending
+ * with distinct ids; ids outside [item_offset, item_offset + n_items) are ignored.  The result is the top-k of the unseen
+ * items by (canonical score desc, id asc), bit-exact like tmf_score_topk: excluded ids are dropped inside the fused kernel
+ * before they reach a row's candidate list or its threshold histogram, so the exactness argument holds with "items" read
+ * as "unseen items".  clamp != 0 ranks by max(s, 0) like tmf_score_topk (zero-score ties are the lowest unseen ids).
+ * Rows with fewer than k unseen items end in (score -inf, id INT32_MAX) padding, as tmf_score_topk_bounded writes it, so
+ * item slabs merge with tmf_topk_merge.  k and the workspace as for tmf_score_topk. */
+TMF_API int tmf_score_topk_masked(const float* U, int64_t n_users, const float* V, int64_t n_items, int32_t n_comp, int32_t ld,
+                          int32_t k, int32_t clamp, int32_t item_offset, const int32_t* ex_ptr, const int32_t* ex_idx,
+                          int32_t* out_idx, float* out_score, void* ws, size_t ws_bytes, tmf_stream_t stream);
+
 /* The raw tensor-core scores s~ of tmf_score_topk's GEMM, written densely (P[n_users, n_items], small shapes only), to
  * test the error bound the exact top-k rests on.  With u~ = u rounded to the operand format and du = u - u~ (likewise v~, dv):
  *   |s~ - s| <= |du| |v| + |u~| |dv| + 2.4e-7 * k_pad * |u~| |v|,   k_pad = n_comp rounded up to a multiple of 64.
@@ -224,13 +236,6 @@ TMF_API int tmf_rank_rows(const float* P, int64_t n_rows, int64_t n_cols, int32_
  * CSR (a_ptr, a_idx: sorted columns) of the NON-ZERO cells of A -- no dense A.  out has n_users*n_items - nnz entries. */
 TMF_API int tmf_gather_unobserved(const float* P, int64_t n_users, int64_t n_items, const int32_t* a_ptr, const int32_t* a_idx,
                           float* out, tmf_stream_t stream);
-
-/* Masked top-k (SURVEY 8f-3, new-build: the reference does not exclude seen items, A.7): keeps, in order, the first k entries
- * of each row of cand_idx [n_users, kc] (the top-kc list of tmf_score_topk) that are not stored in row u of the CSR; rows with
- * fewer than k survivors get short_rows[u] = 1 (the caller ranks those rows exactly).  out_score may be NULL. */
-TMF_API int tmf_filter_seen(const int32_t* cand_idx, const float* cand_score, int64_t n_users, int32_t kc, int32_t k,
-                    const int32_t* a_ptr, const int32_t* a_idx, int32_t* out_idx, float* out_score, int32_t* short_rows,
-                    tmf_stream_t stream);
 
 /* Measurement aid (no reference counterpart): reads the rows table[idx[e]] (ld = 64 or 128 floats) for e < n the way
  * tmf_user_pass gathers embedding rows, folds them into per-thread sums written to out[148 * 8 * 256].  bench.py times it on

@@ -54,13 +54,13 @@ SIGNATURES = {
     "tmf_score_topk_ws_bytes": (_sz, [_i64, _i64, _i32, _i32]),
     "tmf_score_topk": (_i32, [_p, _i64, _p, _i64, _i32, _i32, _i32, _i32, _i32, _p, _p, _p, _sz, _p]),
     "tmf_score_topk_bounded": (_i32, [_p, _i64, _p, _i64, _i32, _i32, _i32, _i32, _i32, _p, _p, _p, _p, _sz, _p]),
+    "tmf_score_topk_masked": (_i32, [_p, _i64, _p, _i64, _i32, _i32, _i32, _i32, _i32, _p, _p, _p, _p, _p, _sz, _p]),
     "tmf_score_dense_tc": (_i32, [_p, _i64, _p, _i64, _i32, _i32, _i32, _p, _p, _sz, _p]),
     "tmf_topk_merge": (_i32, [_p, _p, _i32, _i64, _i32, _p, _p, _p]),
     "tmf_predict_dense": (_i32, [_p, _i64, _p, _i64, _i32, _i32, _p, _p]),
     "tmf_rank_rows_ws_bytes": (_sz, [_i64, _i64]),
     "tmf_rank_rows": (_i32, [_p, _i64, _i64, _i32, _p, _p, _sz, _p]),
     "tmf_gather_unobserved": (_i32, [_p, _i64, _i64, _p, _p, _p, _p]),
-    "tmf_filter_seen": (_i32, [_p, _p, _i64, _i32, _i32, _p, _p, _p, _p, _p, _p]),
     "tmf_gather_rate": (_i32, [_p, _i64, _i32, _p, _i64, _p, _i64, _p]),
     "tmf_metrics_hits": (_i32, [_p, _i64, _i32, _p, _p, _p, _p, _p, _p]),
     "tmf_dcg": (_i32, [_p, _i64, _i32, _p, _p, _p, _p, _p]),
@@ -81,7 +81,8 @@ call_count = 0
 launch_count = 0
 # kernels per ABI call where it is not 1 (memsets are not counted)
 KERNELS_PER_CALL = {"tmf_spmm_seg": 2, "tmf_transpose_build": 3, "tmf_l2_normalize_global": 3, "tmf_kl_moments": 2, "tmf_kl_coef_from_moments": 2,
-                    "tmf_reduce_sum": 2, "tmf_gemm_tc": 4, "tmf_col_sum": 2, "tmf_rank_rows": 2, "tmf_score_topk": 8, "tmf_score_topk_bounded": 8}
+                    "tmf_reduce_sum": 2, "tmf_gemm_tc": 4, "tmf_col_sum": 2, "tmf_rank_rows": 2, "tmf_score_topk": 8, "tmf_score_topk_bounded": 8,
+                    "tmf_score_topk_masked": 8}
 
 
 class TmfError(RuntimeError):

@@ -168,41 +168,6 @@ __global__ void gather_unobserved_kernel(const float* __restrict__ P, long long 
   out[t - lo] = P[t];                    // lo = number of non-zero cells before (u, i) in row-major order
 }
 
-// Masked top-k ("recommend unseen items"): row u of `cand` holds the top-kc items by (score desc, id asc); the first k of them
-// that are NOT stored in row u of the CSR `a` are the top-k over the unobserved items whenever at least k survive.  One warp per
-// row, order-preserving compaction by ballot; rows with fewer than k survivors are flagged (short[u] = 1) for the exact fallback.
-__global__ void filter_seen_kernel(const int* __restrict__ cand, const float* __restrict__ cand_sc, long long n_users, int kc, int k,
-                                   const int* __restrict__ a_ptr, const int* __restrict__ a_idx, int* __restrict__ out_idx,
-                                   float* __restrict__ out_sc, int* __restrict__ short_rows) {
-  const long long u = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  if (u >= n_users) return;
-  const int a = a_ptr[u], b = a_ptr[u + 1];
-  int kept = 0;
-  for (int q0 = 0; q0 < kc && kept < k; q0 += 32) {
-    const int q = q0 + lane;
-    int item = -1;
-    bool keep = false;
-    if (q < kc) {
-      item = cand[u * kc + q];
-      int lo = a, hi = b;
-      while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        if (a_idx[mid] < item) lo = mid + 1; else hi = mid;
-      }
-      keep = !(lo < b && a_idx[lo] == item);
-    }
-    const unsigned bal = __ballot_sync(0xffffffffu, keep);
-    const int pos = kept + __popc(bal & ((1u << lane) - 1u));
-    if (keep && pos < k) {
-      out_idx[u * k + pos] = item;
-      if (out_sc) out_sc[u * k + pos] = cand_sc[u * kc + q];
-    }
-    kept += __popc(bal);
-  }
-  if (lane == 0) short_rows[u] = kept < k ? 1 : 0;
-}
-
 }  // namespace tmf
 
 using namespace tmf;
@@ -213,18 +178,6 @@ extern "C" int tmf_gather_unobserved(const float* P, int64_t n_users, int64_t n_
   const long long total = n_users * n_items;
   if (total == 0) return TMF_OK;
   gather_unobserved_kernel<<<(unsigned)cdiv(total, 256), 256, 0, as_stream(stream)>>>(P, n_users, n_items, a_ptr, a_idx, out);
-  TMF_LAUNCH_CHECK();
-  return TMF_OK;
-}
-
-extern "C" int tmf_filter_seen(const int32_t* cand_idx, const float* cand_score, int64_t n_users, int32_t kc, int32_t k,
-                               const int32_t* a_ptr, const int32_t* a_idx, int32_t* out_idx, float* out_score, int32_t* short_rows,
-                               tmf_stream_t stream) {
-  TMF_REQUIRE(cand_idx && a_ptr && out_idx && short_rows && k >= 1 && kc >= k, "tmf_filter_seen: bad arguments");
-  TMF_REQUIRE(out_score == nullptr || cand_score != nullptr, "tmf_filter_seen: scores requested without candidate scores");
-  if (n_users == 0) return TMF_OK;
-  filter_seen_kernel<<<(unsigned)cdiv(n_users * 32, 256), 256, 0, as_stream(stream)>>>(cand_idx, cand_score, n_users, kc, k, a_ptr, a_idx,
-                                                                                   out_idx, out_score, short_rows);
   TMF_LAUNCH_CHECK();
   return TMF_OK;
 }

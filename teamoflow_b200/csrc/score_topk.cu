@@ -19,6 +19,7 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
+#include <limits.h>
 #include <math.h>
 #include <stdlib.h>
 
@@ -108,6 +109,8 @@ struct TopkParams {
   const float* row_bound;       // optional [n_users]: lower bounds of the rows' k-th best TRUE score (cross-GPU exchange), raw mode only
   unsigned long long* prof;     // optional [8] cycle counters (env TMF_TOPK_PROF=1): where the warps wait
   int dbg;                      // profiling aid (env TMF_TOPK_DEBUG): 1 = no appends, 2 = no filtering, 3 = no TMEM reads
+  const int* ex_ptr;            // MASK: [n_users + 1] CSR of the global item ids excluded per row (sorted, distinct)
+  const int* ex_idx;
 };
 
 // Keep-threshold from a lower bound `kth` of the row's k-th largest approximate score.
@@ -158,21 +161,45 @@ __device__ __forceinline__ float edge_threshold(float lo, float w, int bthr, flo
   return keep_threshold(bin_edge(lo, w, bthr), E, clamp);
 }
 
+// ---- masked top-k: each row's cursor into its sorted list of excluded item ids, three words in shared memory
+// {position, end, id at the position (INT_MAX past the end)}.  Entries reach a row's list in ascending id order (tiles
+// sweep the ids upward, a tile's groups and columns are queued in order, queues drain slot by slot), so the cursor only
+// moves forward -- O(row length) over the whole sweep -- and an excluded id is recognised by one compare with the cursor's id.
+constexpr int EXCUR_BYTES = 16;  // per row
+__device__ __forceinline__ int ex_step(const int* ex_idx, int& pos, int end) {
+  ++pos;
+  return pos < end ? __ldg(ex_idx + pos) : INT_MAX;
+}
+
 // warp-wide drain of the per-lane queues (all lanes must call; st.cq may differ per lane).  Iterations are
 // independent of each other -- fire-and-forget histogram increments (red.shared), list stores that nobody waits
 // for, threshold fixed for the duration -- so they pipeline; the threshold advances once at the end.
+// MASK: excluded ids are dropped here, before the list store and the histogram increment.
 struct DrainRet { float thr; int cnt, bthr, A; };
-// (out of line, state by value in registers: inlining it at every call site costs registers in the tile loop)
-template <int CAP>
-__device__ __noinline__ DrainRet drain_queues_nl(float thr, float thr_ext, float lo, float w, float inv_w, float E, int cnt, int cq, int bthr, int A,
-                                                 uint32_t queue, float2* buf, uint32_t hrow, int k, int clamp) {
+template <int CAP, bool MASK>
+__device__ __forceinline__ DrainRet drain_body(float thr, float thr_ext, float lo, float w, float inv_w, float E, int cnt, int cq, int bthr,
+                                               int A, uint32_t queue, float2* buf, uint32_t hrow, int k, int clamp, uint32_t excur,
+                                               const int* ex_idx) {
   int maxq = cq;
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) maxq = max(maxq, __shfl_xor_sync(0xffffffffu, maxq, o));
+  int ex_pos = 0, ex_end = 0, ex_next = 0;
+  if constexpr (MASK) {
+    ex_pos = (int)lds_u32(excur);
+    ex_end = (int)lds_u32(excur + 4u);
+    ex_next = (int)lds_u32(excur + 8u);
+  }
 #pragma unroll 4
   for (int s = 0; s < maxq; ++s) {
     const float2 e = lds_f2(queue + 8u * (uint32_t)s);
-    const bool ok = (s < cq) && (e.x >= thr);
+    bool ok = (s < cq) && (e.x >= thr);
+    if constexpr (MASK) {
+      if (ok) {
+        const int id = __float_as_int(e.y);
+        while (ex_next < id) ex_next = ex_step(ex_idx, ex_pos, ex_end);
+        ok = ex_next != id;
+      }
+    }
     const bool okh = ok && (e.x >= lo);
     const int b = (int)fminf(fmaxf((e.x - lo) * inv_w, 0.f), (float)(NBINS - 1));
     const int st_ok = ok && (cnt < CAP);
@@ -190,6 +217,10 @@ __device__ __noinline__ DrainRet drain_queues_nl(float thr, float thr_ext, float
     A += (okh && b >= bthr) ? 1 : 0;
   }
   __syncwarp();
+  if constexpr (MASK) {
+    sts_u32(excur, (uint32_t)ex_pos);
+    sts_u32(excur + 8u, (uint32_t)ex_next);
+  }
   bool moved = false;
   while (bthr < NBINS - 1) {
     const int hb = hist_get_s(hrow, bthr);
@@ -203,20 +234,38 @@ __device__ __noinline__ DrainRet drain_queues_nl(float thr, float thr_ext, float
   r.thr = thr; r.cnt = cnt; r.bthr = bthr; r.A = A;
   return r;
 }
+// (out of line, state by value in registers: inlining it at every call site costs registers in the tile loop)
 template <int CAP>
-__device__ __forceinline__ void drain_queues(RowState& st, uint32_t queue, float2* buf, uint32_t hrow, int k, int clamp) {
-  const DrainRet r = drain_queues_nl<CAP>(st.thr, st.thr_ext, st.lo, st.w, st.inv_w, st.E, st.cnt, st.cq, st.bthr, st.A, queue, buf, hrow, k, clamp);
+__device__ __noinline__ DrainRet drain_queues_nl(float thr, float thr_ext, float lo, float w, float inv_w, float E, int cnt, int cq, int bthr, int A,
+                                                 uint32_t queue, float2* buf, uint32_t hrow, int k, int clamp) {
+  return drain_body<CAP, false>(thr, thr_ext, lo, w, inv_w, E, cnt, cq, bthr, A, queue, buf, hrow, k, clamp, 0u, nullptr);
+}
+template <int CAP>
+__device__ __noinline__ DrainRet drain_queues_masked_nl(float thr, float thr_ext, float lo, float w, float inv_w, float E, int cnt, int cq,
+                                                        int bthr, int A, uint32_t queue, float2* buf, uint32_t hrow, int k, int clamp,
+                                                        uint32_t excur, const int* ex_idx) {
+  return drain_body<CAP, true>(thr, thr_ext, lo, w, inv_w, E, cnt, cq, bthr, A, queue, buf, hrow, k, clamp, excur, ex_idx);
+}
+template <int CAP, bool MASK>
+__device__ __forceinline__ void drain_queues(RowState& st, uint32_t queue, float2* buf, uint32_t hrow, int k, int clamp, uint32_t excur,
+                                             const int* ex_idx) {
+  DrainRet r;
+  if constexpr (MASK)
+    r = drain_queues_masked_nl<CAP>(st.thr, st.thr_ext, st.lo, st.w, st.inv_w, st.E, st.cnt, st.cq, st.bthr, st.A, queue, buf, hrow, k,
+                                    clamp, excur, ex_idx);
+  else
+    r = drain_queues_nl<CAP>(st.thr, st.thr_ext, st.lo, st.w, st.inv_w, st.E, st.cnt, st.cq, st.bthr, st.A, queue, buf, hrow, k, clamp);
   st.thr = r.thr; st.cnt = r.cnt; st.bthr = r.bthr; st.A = r.A;
   st.cq = 0;
 }
 
 // One 32-column slice of a row's accumulator BEFORE the row's threshold exists (first 3 tiles; wide k: until the row
 // holds k + 2 tiles of entries): every column is appended directly.  (Clamp-mode "filler" items -- the k lowest ids --
-// therefore need no special case.)
-template <bool DUMP>
+// therefore need no special case.)  MASK: except the row's excluded ids.
+template <bool DUMP, bool MASK>
 __device__ __forceinline__ void epilogue_chunk(uint32_t (&r)[32], int col0, int n_items, bool valid, bool warp_inited,
                                                RowState& st, uint32_t queue, float2* buf, uint32_t hrow, long long row,
-                                               const TopkParams& p) {
+                                               const TopkParams& p, uint32_t excur) {
   if (DUMP) {
     if (valid) {
 #pragma unroll
@@ -229,9 +278,20 @@ __device__ __forceinline__ void epilogue_chunk(uint32_t (&r)[32], int col0, int 
   const int id0 = p.item_offset + col0;
   if (!warp_inited) {  // warp-uniform: no threshold yet, keep everything (coalesced per lane, no queue)
     if (valid) {
+      uint32_t seen = 0;  // MASK: bit j = id0 + j is excluded
+      if constexpr (MASK) {
+        int pos = (int)lds_u32(excur), next = (int)lds_u32(excur + 8u);
+        const int end = (int)lds_u32(excur + 4u);
+        while (next < id0 + 32) {
+          if (next >= id0) seen |= 1u << (next - id0);
+          next = ex_step(p.ex_idx, pos, end);
+        }
+        sts_u32(excur, (uint32_t)pos);
+        sts_u32(excur + 8u, (uint32_t)next);
+      }
 #pragma unroll
       for (int j = 0; j < 32; ++j) {
-        if (col0 + j < n_items) {
+        if (col0 + j < n_items && !((seen >> j) & 1u)) {
           __stcg(buf + st.cnt, make_float2(__uint_as_float(r[j]), __int_as_float(id0 + j)));
           ++st.cnt;
         }
@@ -260,9 +320,9 @@ __device__ __forceinline__ void group_max4(const uint32_t (&r)[32], float* m8) {
 // registers through an unrolled chain of warp-uniform blocks (51.0 ms: 16 extra branches per tile) or an indexed jump (register
 // arrays spill); issuing the next group's TMEM load under the current group's pushes (48.4 ms); slot indices from a survivor
 // mask + popc instead of the running count (47.4 ms).  The epilogue pays per instruction, not per round trip.
-template <int CAP>
+template <int CAP, bool MASK>
 __device__ __forceinline__ void epilogue_half(uint32_t t_base, int col0, RowState& st, uint32_t queue, float2* buf, uint32_t hrow,
-                                              const TopkParams& p) {
+                                              const TopkParams& p, uint32_t excur) {
   uint32_t ra[32], rb[32];
   float m8[4];
   const float thr = st.thr;  // invalid rows carry thr = +inf; NaN-padded columns never win a max or a compare
@@ -286,7 +346,7 @@ __device__ __forceinline__ void epilogue_half(uint32_t t_base, int col0, RowStat
     gmask &= gmask - 1;
     uint32_t v[8];
     tmem_ld8(t_base + (uint32_t)(8 * g), v);
-    if (__any_sync(0xffffffffu, st.cq > QCAP - 8)) drain_queues<CAP>(st, queue, buf, hrow, p.k, p.clamp);
+    if (__any_sync(0xffffffffu, st.cq > QCAP - 8)) drain_queues<CAP, MASK>(st, queue, buf, hrow, p.k, p.clamp, excur, p.ex_idx);
     tmem_ld_wait_for8(v);
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
@@ -297,12 +357,12 @@ __device__ __forceinline__ void epilogue_half(uint32_t t_base, int col0, RowStat
     }
   }
 }
-template <int CAP>
+template <int CAP, bool MASK>
 __device__ __forceinline__ void epilogue_tile(uint32_t t_base, int col0, RowState& st, uint32_t queue, float2* buf, uint32_t hrow,
-                                              const TopkParams& p) {
+                                              const TopkParams& p, uint32_t excur) {
 #pragma unroll 1
   for (int h = 0; h < 2; ++h)  // one copy of the code: the unrolled pass 2 is ~4 KB of sparsely executed instructions
-    epilogue_half<CAP>(t_base + (uint32_t)(64 * h), col0 + 64 * h, st, queue, buf, hrow, p);
+    epilogue_half<CAP, MASK>(t_base + (uint32_t)(64 * h), col0 + 64 * h, st, queue, buf, hrow, p, excur);
 }
 
 // One step of an 8-bit radix select over 256 shared-memory counters: returns the bin that holds the krem-th largest counted
@@ -588,7 +648,9 @@ __host__ __device__ __forceinline__ TopkSmem topk_smem(int kb) {
 }
 
 // WIDE: the configuration for 128 < k <= 1024 (CAP_W list slots, first rebuild by warp_rebuild_selected)
-template <bool DUMP, bool PROF, bool WIDE>
+// MASK: the rows' excluded ids (p.ex_ptr / p.ex_idx) never reach a list or a histogram; the cursors need EXCUR_BYTES per
+// row of dynamic shared memory beyond topk_smem(kb).total
+template <bool DUMP, bool PROF, bool WIDE, bool MASK = false>
 __global__ void __launch_bounds__(TOPK_THREADS, 2)
 score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_constant__ CUtensorMap tmapV, const TopkParams p) {
   constexpr int cap = WIDE ? CAP_W : CAP;
@@ -708,6 +770,7 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
     int* radix = reinterpret_cast<int*>(queues + q * 32 * QCAP);  // radix-select scratch aliases the warp's (empty) queues
     const uint32_t hrow = smem_u32(hist_rows + (q * 32 + lane) * HSTRIDE);
     const uint32_t queue = smem_u32(queues + (q * 32 + lane) * QCAP);
+    const uint32_t excur = smem_u32(smem + S.total + (q * 32 + lane) * EXCUR_BYTES);
     float* iout = init_out + q * 8;
     const int n_items = (int)p.n_items;
     int acc = 0;
@@ -722,6 +785,20 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
       st.E = p.erow[row];
       st.cnt = 0; st.cq = 0; st.bthr = 0; st.A = 0;
       bool warp_inited = false;
+      if constexpr (MASK) {  // cursor at the row's first excluded id >= item_offset
+        int pos = 0, end = 0;
+        if (valid) {
+          pos = p.ex_ptr[row];
+          end = p.ex_ptr[row + 1];
+          for (int hi = end; pos < hi;) {
+            const int mid = (pos + hi) >> 1;
+            if (p.ex_idx[mid] < p.item_offset) pos = mid + 1; else hi = mid;
+          }
+        }
+        sts_u32(excur, (uint32_t)pos);
+        sts_u32(excur + 4u, (uint32_t)end);
+        sts_u32(excur + 8u, (uint32_t)(pos < end ? p.ex_idx[pos] : INT_MAX));
+      }
       // External bound (item-sharded scoring): B = a lower bound of the row's k-th best CANONICAL score over all
       // slabs, so a member of the global top-k has s~ >= B - E.  Clamp mode: only a positive bound says anything
       // (with B <= 0 the zero-score fillers matter).  When every valid row of the warp has such a floor the
@@ -750,7 +827,7 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
         tcgen05_fence_after();
         const uint32_t t_base = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * BN);
         if (!DUMP && warp_inited && TMF_DBG(p) < 2) {
-          epilogue_tile<cap>(t_base, nt * BN, st, queue, buf, hrow, p);
+          epilogue_tile<cap, MASK>(t_base, nt * BN, st, queue, buf, hrow, p, excur);
         } else if (TMF_DBG(p) < 3) {
           uint32_t ra[32], rb[32];
           tmem_ld32(t_base, ra);
@@ -759,10 +836,10 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
             // chunk ch is in ra; chunk ch+1 is fetched into rb while ra is filtered (and vice versa)
             tmem_ld_wait_for(ra);
             tmem_ld32(t_base + (uint32_t)((ch + 1) * 32), rb);
-            epilogue_chunk<DUMP>(ra, nt * BN + ch * 32, n_items, valid, warp_inited, st, queue, buf, hrow, row, p);
+            epilogue_chunk<DUMP, MASK>(ra, nt * BN + ch * 32, n_items, valid, warp_inited, st, queue, buf, hrow, row, p, excur);
             tmem_ld_wait_for(rb);
             if (ch + 2 < BN / 32) tmem_ld32(t_base + (uint32_t)((ch + 2) * 32), ra);
-            epilogue_chunk<DUMP>(rb, nt * BN + (ch + 1) * 32, n_items, valid, warp_inited, st, queue, buf, hrow, row, p);
+            epilogue_chunk<DUMP, MASK>(rb, nt * BN + (ch + 1) * 32, n_items, valid, warp_inited, st, queue, buf, hrow, row, p, excur);
           }
         }
         // accumulator drained: hand it back to the MMA warp before any list maintenance
@@ -775,19 +852,25 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
         if (!DUMP) {
           if (__any_sync(0xffffffffu, st.cq >= QCAP / 2)) {
             const long long td = now();
-            drain_queues<cap>(st, queue, buf, hrow, p.k, p.clamp);
+            drain_queues<cap, MASK>(st, queue, buf, hrow, p.k, p.clamp, excur, p.ex_idx);
             if (PROF && lane == 0) { atomicAdd(p.prof + 10, (unsigned long long)(now() - td)); atomicAdd(p.prof + 11, 1ull); }
           }
           // (re)build: the first time once a row holds INIT_N - BN entries (wide: k + 2 tiles; all valid rows of a warp
-          // get there at the same tile because everything is appended until then), later whenever a list is about to saturate
+          // get there at the same tile because everything is appended until then), later whenever a list is about to saturate.
+          // MASK: a row left without a threshold by the first rebuild (lo = +inf, see below) is rebuilt by the full selection
+          // as soon as it holds k entries, so it grows at most a tile and a queue beyond k unfiltered and the saturation
+          // margin below holds for it as for every other row.
           const int first_n = WIDE ? p.k + 2 * BN : INIT_N - BN;
           const bool first = !warp_inited && __any_sync(0xffffffffu, valid && st.cnt >= first_n);
-          unsigned need = __ballot_sync(0xffffffffu, valid && st.cnt <= cap && (first || (warp_inited && st.cnt > cap - 4 * QCAP)));
+          auto unbounded = [&]() { return MASK && warp_inited && st.lo == INFINITY && st.cnt >= p.k; };
+          unsigned need = __ballot_sync(0xffffffffu, valid && st.cnt <= cap &&
+                                                         (first || (warp_inited && st.cnt > cap - 4 * QCAP) || unbounded()));
           if (need) {  // the radix scratch aliases the queues: empty them first (lengths may grow a little)
             const long long tq = now();
-            drain_queues<cap>(st, queue, buf, hrow, p.k, p.clamp);
+            drain_queues<cap, MASK>(st, queue, buf, hrow, p.k, p.clamp, excur, p.ex_idx);
             if (PROF && lane == 0) { atomicAdd(p.prof + 19, (unsigned long long)(now() - tq)); atomicAdd(p.prof + 18, 1ull); }
-            need = __ballot_sync(0xffffffffu, valid && st.cnt <= cap && (first || (warp_inited && st.cnt > cap - 4 * QCAP)));
+            need = __ballot_sync(0xffffffffu, valid && st.cnt <= cap &&
+                                                  (first || (warp_inited && st.cnt > cap - 4 * QCAP) || unbounded()));
           }
           while (need) {
             const int owner = __ffs(need) - 1;
@@ -798,6 +881,20 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
             float2* obuf = p.cand + ((long long)ub * BM + q * 32 + owner) * cap;
             uint32_t* ohist = hist_rows + (q * 32 + owner) * HSTRIDE;
             const float lo_o = __shfl_sync(0xffffffffu, st.lo, owner);
+            // MASK: list lengths differ per row (excluded ids are never listed), so the warp's first rebuild can meet a row
+            // that holds fewer than k entries.  No lower bound of its k-th best unseen score exists yet: the row keeps no
+            // threshold (every entry is listed, so it stays exact) and an idle histogram (lo = +inf) until it holds k
+            // entries; then the trigger above gives it the full selection below.
+            if (MASK && n_o < p.k) {
+              if (lane == owner) {
+                st.thr = st.thr_ext;
+                st.lo = INFINITY;
+                st.bthr = 0;
+                st.A = 0;
+              }
+              __syncwarp();
+              continue;
+            }
             const long long tr = now();
             int which = 0;
             if (!WIDE && first && n_o <= INIT_N) {
@@ -830,7 +927,7 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmapU, const __grid_consta
         }
         w_init += now() - t2;
       }
-      if (!DUMP) drain_queues<cap>(st, queue, buf, hrow, p.k, p.clamp);
+      if (!DUMP) drain_queues<cap, MASK>(st, queue, buf, hrow, p.k, p.clamp, excur, p.ex_idx);
       if (PROF && lane == 0) {
         atomicAdd(p.prof + 4, (unsigned long long)w_tfull); atomicAdd(p.prof + 5, (unsigned long long)w_work);
         atomicAdd(p.prof + 6, (unsigned long long)w_init); atomicAdd(p.prof + 7, 1ull);
@@ -877,6 +974,8 @@ struct RerankParams {
   unsigned long long* prof;
   int* out_idx;
   float* out_score;
+  const int* ex_ptr;  // masked top-k: CSR of the excluded global item ids (exact_rows_kernel only), else NULL
+  const int* ex_idx;
 };
 
 // Streams a row's list of n entries from global memory (DEPTH loads in flight per lane) and gathers those that pass
@@ -1096,11 +1195,13 @@ __global__ void __launch_bounds__((WIDE ? RR_WARPS_W : RR_WARPS) * 32) rerank_ke
 // exact path for rows whose candidate list overflowed (huge tie groups, adversarially ordered scores): all
 // canonical scores of the row go to scratch; a block-wide radix select finds the k-th largest score T; entries > T
 // plus the lowest-indexed entries == T are collected (k in total) and ranked by (score desc, id asc).
+// Masked top-k (p.ex_ptr set, raw scores): excluded items score -inf and only the kk = min(k, unseen items) best are
+// selected; slots [kk, k) are padded with (-inf, INT32_MAX).
 // (At most 32 CTAs run it, so registers matter more than occupancy: minimum 1 block per SM.)
 __global__ void __launch_bounds__(256, 1) exact_rows_kernel(const RerankParams p, const int* __restrict__ ovf_count,
                                                          const int* __restrict__ ovf_rows, float* __restrict__ scratch) {
   __shared__ int hist[256];
-  __shared__ int s_bin, s_krem, s_cnt_gt, s_cnt_eq, s_warp_tot[8];
+  __shared__ int s_bin, s_krem, s_cnt_gt, s_cnt_eq, s_warp_tot[8], s_n_ex;
   __shared__ float sel_s[WIDE_MAX_K];
   __shared__ int sel_i[WIDE_MAX_K];
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
@@ -1111,6 +1212,7 @@ __global__ void __launch_bounds__(256, 1) exact_rows_kernel(const RerankParams p
   for (int o = blockIdx.x; o < n_ovf; o += gridDim.x) {
     const long long row = ovf_rows[o];
     const float* u = p.U + row * p.ld;
+    if (tid == 0) s_n_ex = 0;
     for (int i = tid; i < n; i += 256) {
       const float* v = p.V + (long long)i * p.ld;
       double acc = 0.0;
@@ -1120,9 +1222,27 @@ __global__ void __launch_bounds__(256, 1) exact_rows_kernel(const RerankParams p
       sc[i] = s + 0.0f;
     }
     __syncthreads();
-    // ---- k-th largest key, 8 bits per pass
+    if (p.ex_ptr != nullptr) {
+      int n_ex = 0;
+      for (int e = p.ex_ptr[row] + tid; e < p.ex_ptr[row + 1]; e += 256) {
+        const int i = p.ex_idx[e] - p.item_offset;
+        if (i >= 0 && i < n && atomicExch(&sc[i], -INFINITY) != -INFINITY) ++n_ex;  // a repeated id counts once
+      }
+      atomicAdd(&s_n_ex, n_ex);
+      __syncthreads();
+    }
+    const int kk = min(k, n - s_n_ex);
+    for (int t = kk + tid; t < k; t += 256) {
+      p.out_idx[row * k + t] = 0x7fffffff;
+      p.out_score[row * k + t] = -INFINITY;
+    }
+    if (kk == 0) {  // block-uniform; every thread has read s_n_ex before the next row resets it
+      __syncthreads();
+      continue;
+    }
+    // ---- kk-th largest key, 8 bits per pass
     uint32_t prefix = 0, mask = 0;
-    int krem = k;
+    int krem = kk;
     for (int shift = 24; shift >= 0; shift -= 8) {
       hist[tid] = 0;
       __syncthreads();
@@ -1146,10 +1266,10 @@ __global__ void __launch_bounds__(256, 1) exact_rows_kernel(const RerankParams p
       krem = s_krem;
       __syncthreads();
     }
-    const float T = key2f(prefix);  // exactly the k-th largest score; krem of the entries == T are needed
+    const float T = key2f(prefix);  // exactly the kk-th largest score; krem of the entries == T are needed
     if (tid == 0) { s_cnt_gt = 0; s_cnt_eq = 0; }
     __syncthreads();
-    // ---- collect: every entry > T (k - krem of them), and the krem lowest-indexed entries == T (ordered scan)
+    // ---- collect: every entry > T (kk - krem of them), and the krem lowest-indexed entries == T (ordered scan)
     for (int i0 = 0; i0 < n; i0 += 256) {
       const int i = i0 + tid;
       const float s = i < n ? sc[i] : -INFINITY;
@@ -1166,9 +1286,9 @@ __global__ void __launch_bounds__(256, 1) exact_rows_kernel(const RerankParams p
       int before = s_cnt_eq;
       for (int w2 = 0; w2 < wid; ++w2) before += s_warp_tot[w2];
       const int my = before + __popc(beq & ((1u << lane) - 1u));
-      if (eq && my < krem) {  // slots [k - krem, k) hold the tied entries in index order
-        sel_s[k - krem + my] = s;
-        sel_i[k - krem + my] = i;
+      if (eq && my < krem) {  // slots [kk - krem, kk) hold the tied entries in index order
+        sel_s[kk - krem + my] = s;
+        sel_i[kk - krem + my] = i;
       }
       __syncthreads();
       if (tid == 0) {
@@ -1178,16 +1298,81 @@ __global__ void __launch_bounds__(256, 1) exact_rows_kernel(const RerankParams p
       }
       __syncthreads();
     }
-    // ---- rank the k selected entries
-    for (int t = tid; t < k; t += 256) {
+    // ---- rank the kk selected entries
+    for (int t = tid; t < kk; t += 256) {
       const float s = sel_s[t];
       const int id = sel_i[t];
       int rank = 0;
-      for (int j = 0; j < k; ++j) rank += (sel_s[j] > s) || (sel_s[j] == s && sel_i[j] < id);
+      for (int j = 0; j < kk; ++j) rank += (sel_s[j] > s) || (sel_s[j] == s && sel_i[j] < id);
       p.out_idx[row * k + rank] = id + p.item_offset;
       p.out_score[row * k + rank] = s;
     }
     __syncthreads();
+  }
+}
+
+// Clamp mode of the masked top-k.  The main kernel, the rerank and the exact path rank each row's unseen items by RAW score;
+// the clamped ranking (max(s, 0) desc, id asc) differs only where the k-th raw score is <= 0.  Such a row holds all of its
+// m < k unseen items with a positive score, in order, and the clamped answer continues with zero-score ties: the lowest
+// unseen ids of the slab not among those m (+0.0 each), then padding.  One warp per row.
+constexpr int FILL_WARPS = 4;
+__device__ __forceinline__ bool sorted_contains(const int* v, int lo, int hi, int x) {
+  const int end = hi;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (v[mid] < x) lo = mid + 1; else hi = mid;
+  }
+  return lo < end && v[lo] == x;
+}
+__global__ void __launch_bounds__(FILL_WARPS * 32) clamp_fill_kernel(long long n_users, long long n_items, int k, int item_offset,
+                                                                   const int* __restrict__ ex_ptr, const int* __restrict__ ex_idx,
+                                                                   int* __restrict__ out_idx, float* __restrict__ out_score) {
+  __shared__ int pos_ids[FILL_WARPS][WIDE_MAX_K];
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long row = (long long)blockIdx.x * FILL_WARPS + w;
+  if (row >= n_users) return;
+  int* oi = out_idx + row * k;
+  float* os = out_score + row * k;
+  if (os[k - 1] > 0.f) return;  // k positive scores: already the clamped answer
+  int m = 0;  // the positive entries: a prefix of the sorted row
+  for (int t0 = 0; t0 < k; t0 += 32) {
+    const unsigned b = __ballot_sync(0xffffffffu, t0 + lane < k && os[t0 + lane] > 0.f);
+    m += __popc(b);
+    if (b != 0xffffffffu) break;
+  }
+  // their ids in ascending order (bitonic sort, INT_MAX pads to a power of two)
+  int* ids = pos_ids[w];
+  int np2 = 1;
+  while (np2 < m) np2 <<= 1;
+  for (int t = lane; t < np2; t += 32) ids[t] = t < m ? oi[t] : INT_MAX;
+  __syncwarp();
+  for (int size = 2; size <= np2; size <<= 1) {
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      for (int i = lane; i < np2 / 2; i += 32) {
+        const int a = 2 * i - (i & (stride - 1));
+        const int x = ids[a], y = ids[a + stride];
+        if ((x > y) == ((a & size) == 0)) { ids[a] = y; ids[a + stride] = x; }
+      }
+      __syncwarp();
+    }
+  }
+  // the slab's ids upward, 32 at a time: keep those neither excluded nor positive
+  const int ea = ex_ptr[row], eb = ex_ptr[row + 1];
+  int filled = m;
+  for (long long i0 = 0; i0 < n_items && filled < k; i0 += 32) {
+    const int id = item_offset + (int)(i0 + lane);
+    const bool keep = i0 + lane < n_items && !sorted_contains(ex_idx, ea, eb, id) && !sorted_contains(ids, 0, m, id);
+    const unsigned bal = __ballot_sync(0xffffffffu, keep);
+    const int pos = filled + __popc(bal & ((1u << lane) - 1u));
+    if (keep && pos < k) {
+      oi[pos] = id;
+      os[pos] = 0.0f;
+    }
+    filled += __popc(bal);
+  }
+  for (int t = filled + lane; t < k; t += 32) {
+    oi[t] = 0x7fffffff;
+    os[t] = -INFINITY;
   }
 }
 
@@ -1365,7 +1550,8 @@ extern "C" size_t tmf_score_topk_ws_bytes(int64_t n_users, int64_t n_items, int3
 
 static int score_topk_impl(const float* U, int64_t n_users, const float* V, int64_t n_items, int32_t n_comp, int32_t ld,
                            int32_t k, int32_t clamp, int32_t item_offset, int32_t* out_idx, float* out_score, void* ws,
-                           size_t ws_bytes, tmf_stream_t stream, float* dump, const float* row_bound = nullptr, int force_fmt = -1) {
+                           size_t ws_bytes, tmf_stream_t stream, float* dump, const float* row_bound = nullptr, int force_fmt = -1,
+                           const int32_t* ex_ptr = nullptr, const int32_t* ex_idx = nullptr) {
   TMF_REQUIRE(n_users >= 0 && n_items > 0 && n_comp > 0 && n_comp <= ld, "tmf_score_topk: bad shape");
   TMF_REQUIRE(n_comp <= MAX_KB * BK, "tmf_score_topk: n_components up to %d supported", MAX_KB * BK);
   TMF_REQUIRE(k >= 1 && k <= WIDE_MAX_K && k <= n_items, "tmf_score_topk: need 1 <= k <= min(%d, n_items) (k=%d)", WIDE_MAX_K, k);
@@ -1417,10 +1603,13 @@ static int score_topk_impl(const float* U, int64_t n_users, const float* V, int6
   rc = make_tmap(&tmapV, Vb, L.ni_pad, L.k_pad, BN);
   if (rc) return rc;
 
+  // masked: raw ranking of the unseen items; clamp mode is finished by clamp_fill_kernel
+  const bool mask = ex_ptr != nullptr;
   TopkParams p{};
   p.n_users = n_users; p.n_items = n_items;
   p.n_tiles = (int)(L.ni_pad / BN); p.kb = L.kb;
-  p.k = k; p.clamp = clamp ? 1 : 0; p.item_offset = item_offset;
+  p.k = k; p.clamp = clamp && !mask ? 1 : 0; p.item_offset = item_offset;
+  p.ex_ptr = ex_ptr; p.ex_idx = ex_idx;
   p.erow = erow;
   p.cand = cand; p.cnt = cnt; p.thr_out = thr; p.ovf_count = ovfc; p.ovf_rows = ovfr;
   p.dump = dump; p.dump_ld = n_items;
@@ -1440,12 +1629,14 @@ static int score_topk_impl(const float* U, int64_t n_users, const float* V, int6
   q.n_users = n_users; q.n_items = n_items; q.k = k; q.clamp = p.clamp; q.item_offset = item_offset; q.r = n_comp; q.ld = ld;
   q.U = U; q.V = V; q.erow = erow; q.prof = p.prof; q.cand = cand; q.cnt = cnt; q.thr = thr; q.ovf_count = ovfc; q.ovf_rows = ovfr;
   q.out_idx = out_idx; q.out_score = out_score;
+  q.ex_ptr = ex_ptr; q.ex_idx = ex_idx;
 
-  const size_t smem = 1024 + topk_smem(L.kb).total;  // + room to align the base
-  auto main_kernel = L.wide ? score_topk_kernel<false, false, true>
-                            : dump != nullptr ? score_topk_kernel<true, false, false> : score_topk_kernel<false, false, false>;
+  const size_t smem = 1024 + topk_smem(L.kb).total + (mask ? BM * EXCUR_BYTES : 0);  // + room to align the base
+  auto main_kernel = L.wide ? (mask ? score_topk_kernel<false, false, true, true> : score_topk_kernel<false, false, true>)
+                   : dump != nullptr ? score_topk_kernel<true, false, false>
+                   : mask ? score_topk_kernel<false, false, false, true> : score_topk_kernel<false, false, false>;
 #ifdef TMF_DEVTOOLS
-  if (p.prof && dump == nullptr) main_kernel = L.wide ? score_topk_kernel<false, true, true> : score_topk_kernel<false, true, false>;
+  if (p.prof && dump == nullptr && !mask) main_kernel = L.wide ? score_topk_kernel<false, true, true> : score_topk_kernel<false, true, false>;
 #endif
   TMF_CUDA(cudaFuncSetAttribute(main_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int rr_warps = L.wide ? RR_WARPS_W : RR_WARPS;
@@ -1470,6 +1661,11 @@ static int score_topk_impl(const float* U, int64_t n_users, const float* V, int6
   if (dump != nullptr) return TMF_OK;
   exact_rows_kernel<<<L.scratch_rows, 256, 0, st>>>(q, ovfc, ovfr, scratch);
   TMF_LAUNCH_CHECK();
+  if (mask && clamp) {
+    clamp_fill_kernel<<<(unsigned)cdiv(n_users, FILL_WARPS), FILL_WARPS * 32, 0, st>>>(n_users, n_items, k, item_offset, ex_ptr, ex_idx,
+                                                                                     out_idx, out_score);
+    TMF_LAUNCH_CHECK();
+  }
 #ifdef TMF_DEVTOOLS
   if (p.prof) {  // profiling aid only: synchronises
     unsigned long long h[24]; int novf = 0;
@@ -1498,6 +1694,14 @@ extern "C" int tmf_score_topk_bounded(const float* U, int64_t n_users, const flo
                                       float* out_score, void* ws, size_t ws_bytes, tmf_stream_t stream) {
   return score_topk_impl(U, n_users, V, n_items, n_comp, ld, k, clamp, item_offset, out_idx, out_score, ws, ws_bytes, stream, nullptr,
                          row_bound);
+}
+
+extern "C" int tmf_score_topk_masked(const float* U, int64_t n_users, const float* V, int64_t n_items, int32_t n_comp, int32_t ld,
+                                     int32_t k, int32_t clamp, int32_t item_offset, const int32_t* ex_ptr, const int32_t* ex_idx,
+                                     int32_t* out_idx, float* out_score, void* ws, size_t ws_bytes, tmf_stream_t stream) {
+  TMF_REQUIRE(ex_ptr != nullptr && out_idx != nullptr && out_score != nullptr, "tmf_score_topk_masked: null argument");
+  return score_topk_impl(U, n_users, V, n_items, n_comp, ld, k, clamp, item_offset, out_idx, out_score, ws, ws_bytes, stream, nullptr,
+                         nullptr, -1, ex_ptr, ex_idx);
 }
 
 extern "C" int tmf_score_dense_tc(const float* U, int64_t n_users, const float* V, int64_t n_items, int32_t n_comp, int32_t ld,

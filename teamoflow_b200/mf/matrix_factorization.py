@@ -29,9 +29,6 @@ from .utils import gather_matrix_indices, random_sampler  # noqa: F401  (ref:20)
 # the fused tcgen05 top-k kernel keeps at most this many results per row; larger k (full rankings)
 # go through dense canonical scores + a segmented sort
 TOPK_FUSED_MAX_K = 1024
-# k up to this runs the kernel's narrow configuration (shorter candidate lists); recommend() keeps its
-# over-fetched list within it whenever k does
-TOPK_NARROW_MAX_K = 128
 
 
 def _public(st, r):
@@ -271,32 +268,22 @@ class MatrixFactorization:
         return _rank_rows(P, clamp)[:, :k].contiguous()
 
     def _hits_relevant(self, A, k):
-        a_ptr, a_idx, a_val = _csr_of(A, self.user_embedding.shape[0], self.item_embedding.shape[0])
-        topk = self._topk(k, clamp=True)  # ref:237,245
-        n_u = topk.shape[0]
-        hits = torch.empty(n_u, dtype=torch.float32, device=topk.device)
-        relevant = torch.empty(n_u, dtype=torch.float32, device=topk.device)
-        _abi.call("tmf_metrics_hits", _abi.ptr(topk), n_u, topk.shape[1], _abi.ptr(a_ptr), _abi.ptr(a_idx),
-                  _abi.ptr(a_val), _abi.ptr(hits), _abi.ptr(relevant))
-        return hits, relevant
+        from . import evaluation as ev
+        a_csr = _csr_of(A, self.user_embedding.shape[0], self.item_embedding.shape[0])
+        return ev.hits_relevant(self._topk(k, clamp=True), a_csr)  # ref:237,245
 
     def recall_at_k(self, A, k=10, preserve_rows=False):
-        """ref:218-269 (hits count any non-zero interaction; relevant counts positive ones)."""
+        """ref:218-269 (hits count any non-zero interaction; relevant counts positive ones).  Held-out evaluation with
+        the training items excluded: ``evaluation.recall_at_k``."""
+        from . import evaluation as ev
         hits, relevant = self._hits_relevant(A, k)
-        if not preserve_rows:
-            m = relevant != 0.0
-            return hits[m] / relevant[m]
-        recall = hits / relevant
-        return torch.where(torch.isnan(recall), torch.zeros_like(recall), recall)
+        return ev.recall_from_hits(hits, relevant, preserve_rows)
 
     def precision_at_k(self, A, k=10, preserve_rows=False):
         """ref:271-304."""
+        from . import evaluation as ev
         hits, relevant = self._hits_relevant(A, k)
-        kk = torch.full_like(hits, float(k))  # tensor / tensor is a true IEEE division (tensor / scalar multiplies by 1/k)
-        if not preserve_rows:
-            m = relevant != 0.0
-            return hits[m] / kk[m]
-        return hits / kk
+        return ev.precision_from_hits(hits, relevant, k, preserve_rows)
 
     def f1_at_k(self, A, k=10, beta=1.0):
         """ref:306-318 (formula kept as written)."""
@@ -306,12 +293,9 @@ class MatrixFactorization:
 
     def dcg_at_k(self, dense_interactions, k=10):
         """ref:320-351 -- DCG of the top-k RAW scores with gains ``2^A - 1``."""
-        n_u, n_i = self.user_embedding.shape[0], self.item_embedding.shape[0]
-        a_ptr, a_idx, a_val = _csr_of(dense_interactions, n_u, n_i)
-        topk = self._topk(k, clamp=False)
-        dcg = torch.empty(n_u, dtype=torch.float32, device=topk.device)
-        _abi.call("tmf_dcg", _abi.ptr(topk), n_u, topk.shape[1], _abi.ptr(a_ptr), _abi.ptr(a_idx), _abi.ptr(a_val), _abi.ptr(dcg))
-        return dcg
+        from . import evaluation as ev
+        a_csr = _csr_of(dense_interactions, self.user_embedding.shape[0], self.item_embedding.shape[0])
+        return ev.dcg_of(self._topk(k, clamp=False), a_csr)
 
     def idcg_at_k(self, dense_interactions, k=10):
         """ref:353-384 -- gains sorted descending, first k."""
@@ -327,12 +311,10 @@ class MatrixFactorization:
 
     def ndcg_at_k(self, A, k=10, preserve_rows=False):
         """ref:386-413."""
+        from . import evaluation as ev
         dcg = self.dcg_at_k(A, k)
         idcg, row_nnz = self._idcg(A, k)
-        ndcg = dcg / idcg
-        if not preserve_rows:
-            return ndcg[row_nnz > 0]
-        return torch.where(~torch.isnan(ndcg), ndcg, torch.zeros_like(ndcg))
+        return ev.ndcg_from_dcg(dcg, idcg, row_nnz, preserve_rows)
 
     def retrieve_user_recs(self, user=None, k=None, exclude=None):
         """Item rankings on RAW scores as a numpy int32 array (ref:416-438).
@@ -356,17 +338,17 @@ class MatrixFactorization:
         EXCLUDING the non-zero cells of the interaction table ``seen`` (sparse or dense, never densified).  int32 ``[n, k]``
         on the device; a user with fewer than ``k`` unseen items has its row padded with -1.
 
-        The fused tcgen05 top-k produces each row's top-``kc`` list (``kc = min(k + heaviest row, 128)``, or ``1024`` in
-        place of ``128`` for ``128 < k <= 1024``) and
-        ``tmf_filter_seen`` keeps the first ``k`` unseen entries; the few rows that have more seen items among their
-        top-``kc`` than the list can absorb are ranked exactly (dense canonical scores of those rows, seen cells masked)."""
+        For ``k <= 1024`` the fused tcgen05 top-k drops the seen items itself (``tmf_score_topk_masked``), so the answer costs
+        one ranking pass however many of a user's best items are seen; larger ``k`` ranks dense blocks of canonical scores
+        (``evaluation.masked_topk``)."""
+        from . import evaluation as ev
         n_u, n_i = self.user_embedding.shape[0], self.item_embedding.shape[0]
-        a_ptr, a_idx, _ = _csr_of(seen, n_u, n_i, drop_zeros=True)
+        a_ptr, a_idx = ev.exclusion_csr(seen, n_u, n_i)
         dev = self.user_embedding.device
         k = int(k)
         if k < 1:
             raise ValueError("k must be >= 1")
-        rows = None
+        U = eng.storage_of(self.user_embedding)
         if users is not None:
             rows = torch.as_tensor(users, device=dev, dtype=torch.int64).reshape(-1)
             cnt = (a_ptr[1:] - a_ptr[:-1])[rows]
@@ -375,40 +357,13 @@ class MatrixFactorization:
             take = torch.repeat_interleave(a_ptr[:-1][rows].to(torch.int64) - sub_ptr[:-1].to(torch.int64), cnt.to(torch.int64)) \
                 + torch.arange(int(sub_ptr[-1]), device=dev)
             a_ptr, a_idx = sub_ptr, a_idx[take].contiguous()
-        n = n_u if rows is None else int(rows.numel())
+            U = U[rows].contiguous()
+        n = U.shape[0]
         out = torch.full((n, k), -1, dtype=torch.int32, device=dev)
         if n == 0:
             return out
-        row_nnz = (a_ptr[1:] - a_ptr[:-1])
-        kk = min(k, n_i)
-        kc = min(n_i, TOPK_NARROW_MAX_K if kk <= TOPK_NARROW_MAX_K else TOPK_FUSED_MAX_K, kk + int(row_nnz.max()))
-        short = torch.ones(n, dtype=torch.int32, device=dev)
-        if kc >= kk and kk <= TOPK_FUSED_MAX_K:
-            cand = self._topk(kc, clamp=False, users=rows)
-            got = torch.empty(n, kk, dtype=torch.int32, device=dev)
-            _abi.call("tmf_filter_seen", _abi.ptr(cand), None, n, kc, kk, _abi.ptr(a_ptr), _abi.ptr(a_idx), _abi.ptr(got), None,
-                      _abi.ptr(short))
-            ok = short == 0
-            out[ok, :kk] = got[ok]
-        todo = torch.nonzero(short).reshape(-1)
-        # exact fallback, a bounded block of rows at a time: dense canonical scores, seen cells -> -inf, stable ranking
-        U, V = eng.storage_of(self.user_embedding), eng.storage_of(self.item_embedding)
-        block = max(1, min(4096, (1 << 27) // max(n_i, 1)))
-        for b0 in range(0, int(todo.numel()), block):
-            sel = todo[b0:b0 + block]
-            gu = sel if rows is None else rows[sel]
-            Ub = U[gu].contiguous()
-            P = torch.empty(sel.numel(), n_i, dtype=torch.float32, device=dev)
-            _abi.call("tmf_predict_dense", _abi.ptr(Ub), Ub.shape[0], _abi.ptr(V), n_i, self.n_components, U.shape[1], _abi.ptr(P))
-            c = row_nnz[sel].to(torch.int64)
-            rr = torch.repeat_interleave(torch.arange(sel.numel(), device=dev), c)
-            first = torch.repeat_interleave(a_ptr[:-1][sel].to(torch.int64) - (torch.cumsum(c, 0) - c), c)
-            cols = a_idx[first + torch.arange(int(c.sum()), device=dev)].long()
-            P[rr, cols] = float("-inf")
-            order = _rank_rows(P, clamp=False)[:, :kk]
-            unseen = (n_i - c).clamp(max=kk)
-            order = torch.where(torch.arange(kk, device=dev)[None, :] < unseen[:, None], order, torch.full_like(order, -1))
-            out[sel, :kk] = order
+        got = ev.masked_topk(U, eng.storage_of(self.item_embedding), self.n_components, k, False, a_ptr, a_idx)
+        out[:, :got.shape[1]] = torch.where(got == ev.PAD_ID, torch.full_like(got, -1), got)
         return out
 
     # ------------------------------------------------------------------ save / load (in-memory, ref:440-475)
