@@ -184,7 +184,10 @@ def test_step_parity(loss, kinds, feat):
 
 @pytest.mark.parametrize("r,S", [(3, 5), (10, 40), (32, 336), (64, 128), (128, 32), (200, 17), (64, 700)])
 def test_wmrb_shapes(r, S):
-    """component counts that exercise every row-group width and the register / shared-memory G paths"""
+    """WMRB through the engine at seven (rank, samples) shapes.  They launch seven of the 27 user-pass instantiations,
+    (LPR, VPL, JPL) = (4, 1, 2), (4, 1, 16), (16, 1, 8), (32, 1, 2), (32, 1, 16), (32, 1, -1) (G in shared memory) and
+    (32, 2, 2): no LPR 8 kernel, and two float4 columns per lane only with JPL 2.  (32, 336) and (64, 700) run the narrow
+    sample gather.  tests/test_gpu_train_variants.py compares every instantiation with an fp64 reference."""
     n_u, n_i = 97, max(S + 3, 211)
     for seed in range(20):
         rng, rows, cols, vals, samp = make_problem(n_u, n_i, r, 2500, S, 7 + seed, values=(1.0, 4.0, -1.0))
