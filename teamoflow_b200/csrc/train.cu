@@ -103,6 +103,14 @@ __device__ __forceinline__ float gsum(float v) {
   return v;
 }
 
+// One step of a reduce-scatter over a group of LPR lanes: of the sums lo and hi, the lane keeps lo if its bit o is clear
+// and hi if it is set, and adds the partner lane's partial of that sum.  This adds the same two partial sums, in the same
+// order, as gsum's step of offset o, so a reduce-scatter whose steps run over gsum's offsets gives every sum gsum's bits.
+template <int LPR>
+__device__ __forceinline__ float scatter_step(float lo, float hi, int o, bool up) {
+  return (up ? hi : lo) + __shfl_xor_sync(0xffffffffu, up ? lo : hi, o, LPR);
+}
+
 // One WARP per work item (a CTA is one warp, up to 32 of them resident per SM): the phases of a user are separated by
 // warp-level synchronisation only, and many users per SM are in flight in different phases.  (The first version gave a
 // user to a 256-thread CTA: 4 CTAs per SM, five block barriers per user and shared-memory reductions over 16 row groups --
@@ -119,7 +127,6 @@ user_pass_kernel(const UserPassParams p) {
   constexpr int NG = NT / LPR;
   constexpr int JH = JPL > 0 ? JPL / 2 : 1;
   constexpr int PD = (JPL >= 0 && JPL <= 4 && VPL == 1) ? 4 : 2;   // row buffers of the interaction loop
-  constexpr int SB = (JPL >= 0 && JPL <= 4 && VPL == 1) ? 8 : 4;   // sample rows gathered at once per group
   constexpr unsigned FULL = 0xffffffffu;
   extern __shared__ __align__(16) float smem[];
   const int tid = threadIdx.x;
@@ -130,34 +137,47 @@ user_pass_kernel(const UserPassParams p) {
   const int S = p.n_samples;
   float* sS = smem;                     // [s_pad]  sample scores, later final G_j
   float* sG = sS + p.s_pad;             // [NG][s_pad] per-group partial G (generic path only)
+  // [2][NT] d and c of the interactions of the current batch, at their owner lanes' slots (shared memory rather than two
+  // registers per lane across the interaction loop, which has none to spare)
+  float* sDC = smem + (LOSS == TMF_LOSS_WMRB ? (1 + (JPL < 0 ? NG : 0)) * p.s_pad : 0);
+  // [3] user and slot of the work item, then the next work item: warp-uniform values that wait in shared memory (every
+  // lane stores the same value) while the sample scores and the interaction loop need the registers
+  int* sItem = reinterpret_cast<int*>(sDC + 2 * NT);
 
-  // work items come from an atomic counter; the NEXT item is claimed while the current one is processed
-  int next = 0;
-  if (tid == 0) next = atomicAdd(p.counter, 1);
+  // work items come from an atomic counter; the NEXT item is claimed while the current one is processed, and its id
+  // waits in shared memory
+  if (tid == 0) sItem[2] = atomicAdd(p.counter, 1);
   for (;;) {
     __syncwarp();  // shared-memory reuse across work items
-    const int t_work = __shfl_sync(FULL, next, 0);
+    const int t_work = sItem[2];
     if (t_work >= p.n_work) break;
-    if (tid == 0) next = atomicAdd(p.counter, 1);
     // a work item is a whole user or, for very heavy users, one slice of its interactions (load balance: a user
     // with millions of interactions would otherwise be one CTA's serial tail)
-    const int u = p.work_user ? p.work_user[t_work] : t_work;
+    int u = p.work_user ? p.work_user[t_work] : t_work;
     const int a = p.work_user ? p.work_a[t_work] : p.row_ptr[u];
     const int b = p.work_user ? p.work_b[t_work] : p.row_ptr[u + 1];
-    const int slot = p.work_user ? p.work_slot[t_work] : -1;
+    int slot = p.work_user ? p.work_slot[t_work] : -1;
 
     if (a == b) {  // no interactions: all gradients of this user are zero
+      __syncwarp();  // every lane has read this item's id
+      if (tid == 0) sItem[2] = atomicAdd(p.counter, 1);
       if (LOSS == TMF_LOSS_WMRB)
         for (int j = tid; j < S; j += NT) p.coef_out[coef_slot(p.coef_pos, p.nnz + (long long)u * S + j)] = 0.f;
       for (int c = tid; c < ld; c += NT) p.dEu[(long long)u * ld + c] = 0.f;
       continue;
     }
 
+    sItem[0] = u;
+    sItem[1] = slot;
     float4 eu[VPL];
     load_row<LPR, VPL>(p.Eu, u, ld, nv, lg, eu);  // zero past the row's end
     const char* ei_lane[VPL];
 #pragma unroll
-    for (int v = 0; v < VPL; ++v) ei_lane[v] = reinterpret_cast<const char*>(p.Ei) + 16 * min(lg + LPR * v, nv - 1);
+    for (int v = 0; v < VPL; ++v) {
+      ei_lane[v] = reinterpret_cast<const char*>(p.Ei) + 16 * min(lg + LPR * v, nv - 1);
+      // kept in registers (the 64-register variants would rebuild it from p.Ei, four instructions per row gather)
+      if constexpr (VPL == 1) asm("" : "+l"(ei_lane[v]));
+    }
     const unsigned ld_bytes = 4u * (unsigned)ld;
 
     // When many samples force the hinge layout's LPR above the row width (S > 16 * row lanes), the two phases that only
@@ -197,21 +217,37 @@ user_pass_kernel(const UserPassParams p) {
             if (j0 + q < S && sl == 0) sS[j0 + q] = sc;
           }
         }
-      }
-      const int n_sit = narrow ? 0 : (S + NG * SB - 1) / (NG * SB);
-      for (int it = 0; it < n_sit; ++it) {  // SB independent row gathers in flight per group; warp-uniform trip count
-        const int j0 = (it * NG + g) * SB;
-        int idx[SB];
-        float4 row[SB][VPL];
+      } else {
+        // 32 samples per round: group g scores samples j0 + g LPR + r, r < LPR.  The round's sample ids are one coalesced
+        // load, handed to the group's lanes by shuffle.  The scores are summed by a reduce-scatter over the group (offsets
+        // LPR / 2, ..., 1, gsum's order): afterwards lane lg holds the score of sample j0 + g LPR + lg = j0 + tid, and the
+        // warp stores the round's 32 scores with one instruction.  The steps down to offset P run as the U rows of samples
+        // r, r + P, ... arrive, so P partial sums are live at a time.
+        for (int j0 = 0; j0 < S; j0 += 32) {
+          constexpr int P = LPR / 2 < 8 ? LPR / 2 : 8;
+          constexpr int U = LPR / P;
+          const int my_id = (j0 + tid < S) ? su[j0 + tid] : 0;
+          float part[P];
 #pragma unroll
-        for (int q = 0; q < SB; ++q) idx[q] = (j0 + q < S) ? su[j0 + q] : 0;
+          for (int r = 0; r < P; ++r) {
+            float x[U];
 #pragma unroll
-        for (int q = 0; q < SB; ++q) load_item<VPL>(ei_lane, idx[q], ld_bytes, row[q]);
+            for (int t = 0; t < U; ++t) {
+              float4 row[VPL];
+              load_item<VPL>(ei_lane, __shfl_sync(FULL, my_id, r + t * P, LPR), ld_bytes, row);
+              x[t] = dotv<VPL>(eu, row);
+            }
 #pragma unroll
-        for (int q = 0; q < SB; ++q) {
-          const int j = j0 + q;
-          const float s = gsum<LPR>(dotv<VPL>(eu, row[q]));
-          if (j < S && lg == 0) sS[j] = s;
+            for (int o = LPR / 2, n = U / 2; o >= P; o >>= 1, n >>= 1)
+#pragma unroll
+              for (int t = 0; t < n; ++t) x[t] = scatter_step<LPR>(x[t], x[t + n], o, lg & o);
+            part[r] = x[0];
+          }
+#pragma unroll
+          for (int o = P / 2; o > 0; o >>= 1)
+#pragma unroll
+            for (int r = 0; r < o; ++r) part[r] = scatter_step<LPR>(part[r], part[r + o], o, lg & o);
+          if (j0 + tid < S) sS[j0 + tid] = part[0];
         }
       }
       if constexpr (JPL < 0) {
@@ -236,12 +272,12 @@ user_pass_kernel(const UserPassParams p) {
 
     // ---- interactions of this user, strided over the NG row groups; warp-uniform trip count.  One interaction per
     // row group and iteration: score, S hinge terms (each lane owns JPL of them, evaluated two at a time with packed
-    // fp32x2 instructions), dL/dscore, and acc += c * row while the row is still in registers.  Lane 0 of the group
-    // stores (1 + m, c); the logarithm is applied by a coalesced in-place pass after the loop.
-    auto process = [&](const float4 (&row)[VPL], const float a_k, const int k, const int cpos_k) {
-      const bool active = k < b;
+    // fp32x2 instructions), dL/dscore, and acc += c * row while the row is still in registers.  Returns d (1 + m for
+    // WMRB, the squared error for MSE) and c in every lane of the group.
+    auto process = [&](const float4 (&row)[VPL], const float a_k, const bool active, float& d, float& c) {
       const float pk = gsum<LPR>(dotv<VPL>(eu, row));
-      float c = 0.f, d = 0.f;
+      c = 0.f;
+      d = 0.f;
       if constexpr (LOSS == TMF_LOSS_MSE) {
         const float df = a_k - pk;  // loss_graphs.py:52
         d = df * df;
@@ -301,52 +337,68 @@ user_pass_kernel(const UserPassParams p) {
       }
 #pragma unroll
       for (int v = 0; v < VPL; ++v) fma4(acc[v], c, row[v]);
-      if (lg == 0 && active) {
-        p.loss_out[k] = d;
-        p.coef_out[cpos_k] = c;
-      }
     };
-    // Software pipeline over PD row buffers: (item id, value) of an interaction are fetched PD iterations ahead, its row
-    // PD - 1 iterations ahead, so neither the id -> row dependency nor the row's L2 / HBM latency sits on the critical
-    // path (PD = 4 where the registers allow it: with a 1 GB item table the rows come from HBM and one row in flight per
-    // warp would leave the memory system idle).  Iteration i uses buffer i % PD; the loop is unrolled PD times so the
-    // buffers are addressed statically (no register copies).  Indices past the slice are clamped (a tail iteration
-    // re-reads the last row and is masked by `active`).
-    const int* cpos = p.coef_pos;
-    auto fetch_idx = [&](int& idx, float& a_k, int& pos, const int k) {
-      const int kc = min(k, b - 1);
-      idx = p.col_idx[kc];
-      a_k = p.val[kc];
-      pos = (int)coef_slot(cpos, kc);
-    };
+    // Iteration it of group g is interaction a + it NG + g.  The iterations run in batches of LPR: in the batch that starts
+    // at iteration it0, lane lg of group g owns iteration it0 + lg.  It holds that interaction's value (one coalesced load
+    // for the warp's 32 interactions), the group parks the interaction's d and c at the lane's slots of sDC, and once the
+    // batch is done the lane stores log(d) (one coalesced store for the warp) and c.  Item ids are held the same way PD - 1
+    // iterations ahead (lane lg: iteration it0 + PD - 1 + lg), and the next batch's ids and values are loaded when a batch
+    // starts.
+    // Software pipeline over PD row buffers: a row is gathered PD - 1 iterations before it is used, so the row's L2 / HBM
+    // latency does not sit on the critical path (PD = 4 where the registers allow it: with a 1 GB item table the rows come
+    // from HBM and one row in flight per warp would leave the memory system idle).  Iteration i uses buffer i % PD; the
+    // loop is unrolled PD times so the buffers are addressed statically (no register copies).  Interactions past the
+    // slice are clamped (a tail iteration re-reads the last row and is masked by `active`).
     {
       const int n_it = (b - a + NG - 1) / NG;
-      int k = a + g;
+      const int n_git = (b - a - g + NG - 1) / NG;  // iterations in which this group has an interaction
+      auto clamped = [&](int it) { return min(a + it * NG + g, b - 1); };
       float4 rows[PD][VPL];
-      int ids[PD], ps[PD];
-      float vs[PD];
 #pragma unroll
-      for (int q = 0; q < PD; ++q) fetch_idx(ids[q], vs[q], ps[q], k + q * NG);
+      for (int q = 0; q < PD - 1; ++q) load_item<VPL>(ei_lane, p.col_idx[clamped(q)], ld_bytes, rows[q]);
+      int nxt_id = p.col_idx[clamped(PD - 1 + lg)];
+      float nxt_v = p.val[clamped(lg)];
+      // shared-memory address of the group's d and c slots, held in a register (rebuilding it costs more than the register)
+      unsigned dc_g = (unsigned)__cvta_generic_to_shared(sDC + g * LPR);
+      asm("" : "+r"(dc_g));
+      for (int it0 = 0; it0 < n_it; it0 += LPR) {
+        const int cur_id = nxt_id;
+        const float cur_v = nxt_v;
+        nxt_id = p.col_idx[clamped(it0 + LPR + PD - 1 + lg)];
+        nxt_v = p.val[clamped(it0 + LPR + lg)];
+        const int n_in = min(LPR, n_it - it0);
+        const int n_act = n_git - it0;  // iterations it0 + i of this group with i < n_act are in the slice
+        __syncwarp();  // the previous batch's d and c have been read
+        for (int i = 0; i < n_in; i += PD) {
 #pragma unroll
-      for (int q = 0; q < PD - 1; ++q) load_item<VPL>(ei_lane, ids[q], ld_bytes, rows[q]);
-      for (int it = 0; it < n_it; it += PD, k += PD * NG) {
-#pragma unroll
-        for (int q = 0; q < PD; ++q) {
-          if (q == 0 || it + q < n_it) {  // warp-uniform
-            const int qn = (q + PD - 1) % PD;                       // buffer of iteration it + q + PD - 1
-            load_item<VPL>(ei_lane, ids[qn], ld_bytes, rows[qn]);
-            const float v = vs[q];
-            const int pk = ps[q];
-            fetch_idx(ids[q], vs[q], ps[q], k + (q + PD) * NG);
-            process(rows[q], v, k + q * NG, pk);
+          for (int q = 0; q < PD; ++q) {
+            if (q == 0 || i + q < n_in) {  // warp-uniform
+              load_item<VPL>(ei_lane, __shfl_sync(FULL, cur_id, i + q, LPR), ld_bytes, rows[(q + PD - 1) % PD]);
+              float d, c;
+              process(rows[q], __shfl_sync(FULL, cur_v, i + q, LPR), i + q < n_act, d, c);
+              // every lane of the group holds d and c: all write the same value to the owner's slots
+              asm volatile("st.shared.f32 [%0], %1;" ::"r"(dc_g + 4 * (i + q)), "f"(d) : "memory");
+              asm volatile("st.shared.f32 [%0], %1;" ::"r"(dc_g + 4 * (NT + i + q)), "f"(c) : "memory");
+            }
           }
+        }
+        __syncwarp();  // the group's stores of d and c are visible to their owner lanes
+        if (lg < n_act) {
+          // (coef_pos is read here rather than with the batch's values: the loop above has no register to keep it in)
+          const int k_own = a + (it0 + lg) * NG + g;
+          const float d = sDC[tid];
+          p.loss_out[k_own] = LOSS == TMF_LOSS_WMRB ? logf(d) : d;  // log(1 + m), loss_graphs.py:88
+          p.coef_out[coef_slot(p.coef_pos, k_own)] = sDC[NT + tid];
         }
       }
     }
 
+    u = sItem[0];
+    slot = sItem[1];
+
+    const int* cpos = p.coef_pos;
     if constexpr (LOSS == TMF_LOSS_WMRB) {
-      __syncwarp();  // every lane's (1 + m) stores are visible to the warp; sS (sample scores) is no longer read
-      for (int k = a + tid; k < b; k += NT) p.loss_out[k] = logf(p.loss_out[k]);  // log(1 + m), loss_graphs.py:88
+      __syncwarp();  // sS (sample scores of the generic path) is no longer read
       // A whole user's G_uj is final and goes to its coefficient slot; a slice's is a partial sum, written to its part_G
       // row and added up by the fix-up kernel.  sS keeps G for the sample term below.  (The JPL > 0 store stays split by
       // destination: a single store through a selected pointer costs the 64-register variants extra spill bytes.)
@@ -397,6 +449,8 @@ user_pass_kernel(const UserPassParams p) {
         }
       }
     }
+
+    if (tid == 0) sItem[2] = atomicAdd(p.counter, 1);
 
     // ---- dE_u[u] = sum over the row groups
 #pragma unroll
@@ -466,8 +520,8 @@ template <int LPR, int VPL, int JPL, int LOSS>
 static int launch_user_pass(const UserPassParams& p, cudaStream_t st) {
   constexpr int NG = kUserPassThreads / LPR;
   auto kern = user_pass_kernel<LPR, VPL, JPL, LOSS>;
-  size_t smem = 0;
-  if (LOSS == TMF_LOSS_WMRB) smem = (size_t)(1 + (JPL < 0 ? NG : 0)) * p.s_pad * sizeof(float);
+  size_t smem = (2 * kUserPassThreads + 4) * sizeof(float);  // sDC, sItem
+  if (LOSS == TMF_LOSS_WMRB) smem += (size_t)(1 + (JPL < 0 ? NG : 0)) * p.s_pad * sizeof(float);
   UserPassParams q = p;
   TMF_REQUIRE(smem <= 200 * 1024, "tmf_user_pass: n_samples=%d too large for shared memory (%zu B)", p.n_samples, smem);
   if (smem > 48 * 1024) TMF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
